@@ -3,7 +3,7 @@
 (GeoAc3D, ToyAtmo.met, theta 1-60 deg step 1 x azimuth 0-359.9 deg step 0.1 = 216 000 rays, 2 bounces, CalcAmp on,
 WriteRays=False); one pass over the whole launch-angle grid = one "step".
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Workloads: config1 ... config5 are BASELINE.json's five configurations (SURVEY.md section 8d); config4s / config5s are the
 same range-dependent runs on a coarser node grid with fewer rays (quick checks); smallgrid / midgrid are reduced config-2
@@ -375,6 +375,8 @@ def run_ours(args):
     t_wall = time.perf_counter() - t_wall0
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, n, n_rec, d_rec, d_status, d_nsteps)
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     kern_ms = sum(a.elapsed_time(b) for a, b in kev) / args.steps        # scheduling pass + trace kernel (+4 memsets) per pass
     total_steps, _ = tr.last_stats()                                    # RK4 steps of one pass on this rank
@@ -498,6 +500,29 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, n, n_rec, d_rec, d_status, d_nsteps):
+    """Write the records of the last timed pass as float64 .npy files under out_dir, shaped as Tracer.trace returns them:
+    rec [NFIELDS][rays][n_rec], status and n_steps [rays][n_rec], plus ray_index [rays] (the rays' positions in the traced
+    batch).  When all rays would exceed DUMP_BYTES, a fixed seeded sample of rays is written, every bounce of each, so that
+    runs of two builds with the same arguments can be compared file for file."""
+    import torch
+    nf = d_rec.shape[0]
+    per_ray = 8 * ((nf + 2) * n_rec + 1)
+    k = min(n, (DUMP_BYTES - 4 * 4096) // per_ray)                       # 4096 bytes per file left for the .npy header
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    sel = torch.from_numpy(idx).to(d_rec.device)
+    arrays = {"rec": d_rec.view(nf, n, n_rec).index_select(1, sel),
+              "status": d_status.view(n, n_rec).index_select(0, sel),
+              "n_steps": d_nsteps.view(n, n_rec).index_select(0, sel)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.to(torch.float64).cpu().numpy())
+    np.save(os.path.join(out_dir, "ray_index.npy"), idx.astype(np.float64))
+
+
 def single_process_multi_record(args, world):
     """Rank 0 only, the other ranks idle at a barrier: ONE process drives all `world` devices through the product's own multi-device
     entry point (geoac_create_multi + geoac_trace_multi: host threads, interleaved 4096-ray blocks, pinned staging, merge by ray
@@ -604,7 +629,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="development aid: skip the end-to-end leg")
     ap.add_argument("--no-strong", action="store_true", help="skip the config-5 strong-scaling sub-record")
     ap.add_argument("--ray-limit", type=float, default=0.0, help="profiling aid: override ray_limit (RK4 step limit per segment = 100 x ray_limit)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write rank 0's records of the last timed pass to DIR/*.npy (float64, at most 64 MB: a seeded sample of rays beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's records (--impl ours)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
