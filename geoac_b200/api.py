@@ -360,18 +360,19 @@ class Tracer:
         return steps / (32.0 * t.value) if t.value else 0.0
 
     def last_kernel_launches(self):
-        """Kernels the last trace enqueued (1; 5 or 10 with the longest-ray-first scheduling pass)."""
+        """Kernels the last trace enqueued (1; 6 or 7 for the range-dependent sets and 10 for the stratified ones with the
+        longest-ray-first scheduling pass)."""
         k = C.c_int64(0)
         self._check(lib().geoac_last_trace_counters(self._h, None, C.byref(k)), "geoac_last_trace_counters")
         return k.value
 
     def last_schedule(self):
-        """Scheduling facts of the last trace: packet grouping, long-region packets, exclusive long-region CTAs, kernels."""
+        """Scheduling facts of the last trace: long-region packets, quarter packets, exclusive long-region CTAs, kernels."""
         o = (C.c_int64 * 8)()
         self._check(lib().geoac_last_schedule(self._h, o), "geoac_last_schedule")
         ms = np.zeros(2)
         lib().geoac_last_launch_ms(self._h, _p(ms))
-        return {"rd_group": o[0], "long_packets": o[1], "quarter_packets": o[4], "long_ctas": o[2], "launches": o[3], "main_ms": float(ms[0]), "long_ms": float(ms[1])}
+        return {"long_packets": o[1], "quarter_packets": o[4], "long_ctas": o[2], "launches": o[3], "main_ms": float(ms[0]), "long_ms": float(ms[1])}
 
     def predicted_costs(self, n):
         """RK4 step counts the cost scout predicted for the n rays of the last trace (diagnosis hook)."""

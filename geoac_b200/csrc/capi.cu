@@ -14,13 +14,11 @@
 #include <type_traits>
 #include <thread>
 #include <atomic>
+#include <limits>
 
 #include "core.cuh"
 #include "eq_cartesian.cuh"
-#if __has_include("eq_global.cuh")
 #include "eq_global.cuh"
-#define GEOAC_HAVE_GLOBAL 1
-#endif
 #include "eq_rngdep.cuh"
 #include "trace_kernel.cuh"
 #include "host_tables.hpp"
@@ -33,41 +31,40 @@ static thread_local std::string g_create_error;
 // geoac_create; afterwards only geoac_set_knob changes them -- nothing on the launch path touches the environment.
 struct Knobs {
     int lpt = 1;            // claim order: 0 natural, 1 automatic, 2 always
-    int packet = -1;        // whole-warp refill for the stratified sets: -1 automatic, 0 / 1 forced
     int scout_coarse = 0;   // step-size multiple of the cost scout (0 = default per variant)
-    int stable = 1;         // (cost, inclination, index) order for the stratified sets
     int cost_shift = 2;     // log2 coarsening of the cost key
     int coop = 1;           // cooperative (several lanes per ray) modes of the range-dependent sets
     int sbpoly = 1;         // absorption through per-interval polynomials
-    int block3d = 384;      // lanes per SM of Eq3D<true>
     int host_tables = 0;    // build the node tables on the host
-    int rd_group = 0;       // range-dependent packets: 0 = 32 consecutive rays (inclination neighbours), 1 = equal inclination / neighbouring azimuth, -1 = automatic
     int long_alpha = 100;   // a packet is LONG if its cost exceeds long_alpha % of the average work of a lane
-    int long_width = 32;    // long-region CTAs: 32 = one thread per ray, 8 = cooperative kernel (four lanes per ray, cell cache in shared memory)
     int long_sm_pct = 90;   // at most this share of the SMs is given to the long-region launch (its CTAs help with the main region once theirs is drained)
     int exclusive = 1;      // long-region launch keeps its SMs to itself (0: one launch, long packets first)
-    int rd_ctas = 0;        // range-dependent sets: CTAs per SM of the main launch (0 = as many as fit)
     int dilate = 400;       // range-dependent sets: the ordering cost of a ray is the maximum over its inclination neighbours within this many
                             // millidegrees (0 = off): the edge of a long ray family is scheduled as long
-    int refine = 0;         // range-dependent sets: rays the cost scout finds long are scouted again at a quarter of its step multiple (measured on the
-                            // config-5 share of one of 8 GPUs: +8 s for the second pass, no change of the long launch -- off)
     int quarter = 1;        // the longest long-region packets are claimed as quarter packets while the exclusive SMs have warps to spare
     int quarter_alpha = 210;// ... those whose cost exceeds this % of the average lane work (lone-warp speed is ~2.1x the loaded one)
-    int scout_stride = 0;   // the cost scout traces every N-th ray of the batch (0 = default: every ray; measured on config 2: every 4th ray costs 24 % -- the warps' rays stop ending together)
 };
-static int env_int(const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; }
+// name for geoac_set_knob, suffix of the environment variable, field, and the range a value is clamped to
+struct KnobDef { const char* name; const char* env; int Knobs::* field; int lo, hi; };
+constexpr int kLo = std::numeric_limits<int>::min(), kHi = std::numeric_limits<int>::max();   // no clamp
+static const KnobDef kKnobs[] = {
+    { "lpt", "LPT", &Knobs::lpt, kLo, kHi },
+    { "scout_coarse", "SCOUT_COARSE", &Knobs::scout_coarse, 0, kHi },
+    { "cost_shift", "COSTSHIFT", &Knobs::cost_shift, 0, 7 },
+    { "coop", "COOP", &Knobs::coop, kLo, kHi },
+    { "sbpoly", "SBPOLY", &Knobs::sbpoly, kLo, kHi },
+    { "host_tables", "HOST_TABLES", &Knobs::host_tables, kLo, kHi },
+    { "long_alpha", "LONG_ALPHA", &Knobs::long_alpha, 1, kHi },
+    { "long_sm_pct", "LONG_SM_PCT", &Knobs::long_sm_pct, 1, 90 },
+    { "exclusive", "EXCLUSIVE", &Knobs::exclusive, kLo, kHi },
+    { "dilate", "DILATE", &Knobs::dilate, 0, kHi },
+    { "quarter", "QUARTER", &Knobs::quarter, kLo, kHi },
+    { "quarter_alpha", "QUARTER_ALPHA", &Knobs::quarter_alpha, 1, kHi },
+};
 static Knobs knobs_from_env() {
     Knobs k;
-    k.lpt = env_int("GEOAC_B200_LPT", k.lpt); k.packet = env_int("GEOAC_B200_PACKET", k.packet);
-    k.scout_coarse = std::max(0, env_int("GEOAC_B200_SCOUT_COARSE", 0)); k.stable = env_int("GEOAC_B200_STABLE", k.stable);
-    k.cost_shift = std::min(7, std::max(0, env_int("GEOAC_B200_COSTSHIFT", k.cost_shift))); k.coop = env_int("GEOAC_B200_COOP", k.coop);
-    k.sbpoly = env_int("GEOAC_B200_SBPOLY", k.sbpoly); k.block3d = env_int("GEOAC_B200_BLOCK", k.block3d);
-    k.host_tables = env_int("GEOAC_B200_HOST_TABLES", k.host_tables);
-    k.rd_group = env_int("GEOAC_B200_RD_GROUP", k.rd_group); k.long_alpha = std::max(1, env_int("GEOAC_B200_LONG_ALPHA", k.long_alpha));
-    k.long_width = env_int("GEOAC_B200_LONG_WIDTH", k.long_width) == 8 ? 8 : 32;
-    k.long_sm_pct = std::min(90, std::max(1, env_int("GEOAC_B200_LONG_SM_PCT", k.long_sm_pct))); k.exclusive = env_int("GEOAC_B200_EXCLUSIVE", k.exclusive);
-    k.rd_ctas = std::max(0, env_int("GEOAC_B200_RD_CTAS", k.rd_ctas)); k.quarter = env_int("GEOAC_B200_QUARTER", k.quarter); k.refine = env_int("GEOAC_B200_REFINE", k.refine); k.dilate = std::max(0, env_int("GEOAC_B200_DILATE", k.dilate)); k.quarter_alpha = std::max(1, env_int("GEOAC_B200_QUARTER_ALPHA", k.quarter_alpha));
-    k.scout_stride = std::max(0, env_int("GEOAC_B200_SCOUT_STRIDE", k.scout_stride));
+    for (const KnobDef& d : kKnobs)
+        if (const char* e = std::getenv((std::string("GEOAC_B200_") + d.env).c_str())) k.*d.field = std::clamp(std::atoi(e), d.lo, d.hi);
     return k;
 }
 
@@ -92,18 +89,19 @@ struct geoac_ctx {
     double* d_prev = nullptr; size_t cap_prev = 0; // y_{k-1} scratch of the trace kernel
     double* d_path = nullptr; size_t cap_path = 0; int32_t* d_path_rows = nullptr; size_t cap_path_rows = 0;   // raypath capture staging
     double* d_caus = nullptr; size_t cap_caus = 0; int32_t* d_caus_rows = nullptr; size_t cap_caus_rows = 0;   // caustic event staging
-    uint32_t* d_refine = nullptr; int64_t cap_refine = 0;    // rays scouted a second time
-    uint32_t *d_cost = nullptr, *d_order = nullptr, *d_hist = nullptr, *d_blockhist = nullptr, *d_order2 = nullptr; uint8_t* d_keys = nullptr; int64_t cap_order = 0, cap_keys = 0;   // longest-ray-first scheduling
+    // longest-ray-first scheduling: predicted costs, the costs the order uses (dilated), claim order, sort scratch; capacities in bytes
+    uint32_t *d_cost = nullptr, *d_cost_dilated = nullptr, *d_order = nullptr, *d_order2 = nullptr, *d_hist = nullptr, *d_blockhist = nullptr;
+    uint8_t* d_keys = nullptr;
+    size_t cap_cost = 0, cap_cost_dilated = 0, cap_order = 0, cap_order2 = 0, cap_hist = 0, cap_blockhist = 0, cap_keys = 0;
     int last_launches = 0;
     // staging for the host-buffer entry point
     double *d_theta = nullptr, *d_phi = nullptr, *d_rec = nullptr;
     int32_t *d_status = nullptr, *d_nsteps = nullptr;
-    int64_t cap_rays = 0, cap_slots = 0;
+    size_t cap_theta = 0, cap_phi = 0, cap_rec = 0, cap_status = 0, cap_nsteps = 0;
     cudaStream_t stream = nullptr, stream_long = nullptr;      // stream_long: the concurrent long-region launch of the range-dependent sets
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_fork = nullptr, ev_join = nullptr, ev_m0 = nullptr, ev_m1 = nullptr, ev_l0 = nullptr, ev_l1 = nullptr;
     bool timed_launches = false;
-    double grid_dh = 0.0, grid_dz = 0.0;                       // median node spacing [km] of the range-dependent grid (packet grouping heuristic)
-    int last_long_packets = 0, last_long_ctas = 0, last_rd_group = 0, last_quarter_packets = 0;
+    int last_long_packets = 0, last_long_ctas = 0, last_quarter_packets = 0;
     int64_t last_steps = 0; double last_ms = 0.0;
     bool consts_dirty = true;
     bool src_set = false;
@@ -171,7 +169,7 @@ extern "C" void geoac_destroy(geoac_ctx* ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     cudaFree(ctx->d_table); cudaFree(ctx->d_sbpoly); cudaFree(ctx->d_consts); cudaFree(ctx->d_counters); cudaFree(ctx->d_prev);
-    cudaFree(ctx->d_refine); cudaFree(ctx->d_cost); cudaFree(ctx->d_order); cudaFree(ctx->d_hist); cudaFree(ctx->d_blockhist); cudaFree(ctx->d_order2); cudaFree(ctx->d_keys); cudaFree(ctx->d_path); cudaFree(ctx->d_path_rows); cudaFree(ctx->d_caus); cudaFree(ctx->d_caus_rows);
+    cudaFree(ctx->d_cost_dilated); cudaFree(ctx->d_cost); cudaFree(ctx->d_order); cudaFree(ctx->d_hist); cudaFree(ctx->d_blockhist); cudaFree(ctx->d_order2); cudaFree(ctx->d_keys); cudaFree(ctx->d_path); cudaFree(ctx->d_path_rows); cudaFree(ctx->d_caus); cudaFree(ctx->d_caus_rows);
     cudaFree(ctx->d_tuv); cudaFree(ctx->d_rho); cudaFree(ctx->d_ax);
     cudaFree(ctx->d_theta); cudaFree(ctx->d_phi); cudaFree(ctx->d_rec); cudaFree(ctx->d_status); cudaFree(ctx->d_nsteps);
     cudaFreeHost(ctx->pin_theta.p); cudaFreeHost(ctx->pin_phi.p); cudaFreeHost(ctx->pin_rec.p); cudaFreeHost(ctx->pin_status.p); cudaFreeHost(ctx->pin_nsteps.p);
@@ -199,18 +197,9 @@ extern "C" int geoac_set_params(geoac_ctx* ctx, const geoac_params* p) {
 
 extern "C" int geoac_set_knob(geoac_ctx* ctx, const char* name, int value) {
     if (!ctx || !name) return GEOAC_ERR_BAD_ARG;
-    Knobs& k = ctx->knobs;
-    const std::string n(name);
-    if (n == "lpt") k.lpt = value; else if (n == "packet") k.packet = value; else if (n == "scout_coarse") k.scout_coarse = std::max(0, value);
-    else if (n == "stable") k.stable = value; else if (n == "cost_shift") k.cost_shift = std::min(7, std::max(0, value));
-    else if (n == "coop") k.coop = value; else if (n == "sbpoly") k.sbpoly = value; else if (n == "block3d") k.block3d = value;
-    else if (n == "host_tables") k.host_tables = value;
-    else if (n == "rd_group") k.rd_group = value; else if (n == "long_alpha") k.long_alpha = std::max(1, value);
-    else if (n == "long_width") k.long_width = (value == 8) ? 8 : 32; else if (n == "long_sm_pct") k.long_sm_pct = std::min(90, std::max(1, value));
-    else if (n == "exclusive") k.exclusive = value; else if (n == "rd_ctas") k.rd_ctas = std::max(0, value); else if (n == "quarter") k.quarter = value; else if (n == "refine") k.refine = value; else if (n == "dilate") k.dilate = std::max(0, value); else if (n == "quarter_alpha") k.quarter_alpha = std::max(1, value);
-    else if (n == "scout_stride") k.scout_stride = std::max(0, value);
-    else return fail(ctx, GEOAC_ERR_BAD_ARG, "unknown knob " + n);
-    return GEOAC_OK;
+    for (const KnobDef& d : kKnobs)
+        if (!std::strcmp(name, d.name)) { ctx->knobs.*d.field = std::clamp(value, d.lo, d.hi); return GEOAC_OK; }
+    return fail(ctx, GEOAC_ERR_BAD_ARG, std::string("unknown knob ") + name);
 }
 
 // ---- knot slopes of the natural spline: same tridiagonal recurrences as G2S_Spline1D.cpp:161-196 ----
@@ -422,8 +411,6 @@ extern "C" int geoac_set_atmosphere_3d(geoac_ctx* ctx, int n0, int n1, int nz, c
     g.tuv = ctx->d_tuv; g.rho = ctx->d_rho; g.ax0 = ctx->d_ax; g.ax1 = ctx->d_ax + (size_t)n0 * AX; g.axz = ctx->d_ax + (size_t)(n0 + n1) * AX;
     g.n0 = n0; g.n1 = n1; g.nz = nz; g.scratch = nullptr; g.role = 0; g.nrole = 1; g.glane0 = 0; g.gmask = 0;
     g.amin = ax0[0]; g.amax = ax0[n0 - 1]; g.bmin = ax1[0]; g.bmax = ax1[n1 - 1]; g.zmin = z[0]; g.zmax = z[nz - 1];
-    ctx->grid_dh = 0.5 * ((ax0[n0 - 1] - ax0[0]) / (n0 - 1) + (ax1[n1 - 1] - ax1[0]) / (n1 - 1)) * (glob ? kREarth : 1.0);   // mean node spacing [km]
-    ctx->grid_dz = (z[nz - 1] - z[0]) / (nz - 1);
     // GeoAc_SetPropRegion: G2S_MultiDimSpline3D.cpp:22-33 / G2S_GlobalMultiDimSpline3D.cpp:22-33
     ctx->prm.vert_limit = g.zmax;
     ctx->prm.box_min[0] = g.amin; ctx->prm.box_max[0] = g.amax; ctx->prm.box_min[1] = g.bmin; ctx->prm.box_max[1] = g.bmax;
@@ -500,234 +487,150 @@ static int refresh_consts(geoac_ctx* ctx) {
 }
 
 // ---- kernel launch ----
-template <class EQ, int BLOCK, bool PATHS = false>
-static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
-    constexpr bool kGrid = std::is_same<typename EQ::Atmo, Grid3D>::value;
-    const size_t lane_doubles = ((size_t)LaneLayout<EQ>::STRIDE * BLOCK + 1) & ~(size_t)1;
-    const size_t fixed = ((sizeof(LaunchConsts) + 15) / 16) * 16 + 16 + lane_doubles * sizeof(double);
-    const size_t tab_bytes = kGrid ? 0 : (size_t)TAB_NARR * ctx->n * sizeof(double);
-    int max_optin = 0;
-    CK(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
-    if (fixed > (size_t)max_optin) return fail(ctx, GEOAC_ERR_CUDA, "lane records do not fit in shared memory");
-    const bool in_smem = !kGrid && fixed + tab_bytes <= (size_t)max_optin;
-    const size_t smem = in_smem ? fixed + tab_bytes : fixed;
-    const void* fn;
-    if constexpr (PATHS) {            // raypath / caustic capture; a profile too large for shared memory is read through L1/L2 like in the plain trace
-        if constexpr (kGrid) fn = (const void*)trace_kernel<EQ, BLOCK, false, true>;
-        else fn = in_smem ? (const void*)trace_kernel<EQ, BLOCK, true, true> : (const void*)trace_kernel<EQ, BLOCK, false, true>;
-    }
-    else fn = in_smem ? (const void*)trace_kernel<EQ, BLOCK, true> : (const void*)trace_kernel<EQ, BLOCK, false>;
-    CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 1;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, BLOCK, smem));
-    if (per_sm < 1) return fail(ctx, GEOAC_ERR_CUDA, "trace kernel does not fit on an SM");
-    if (kGrid && ctx->knobs.rd_ctas > 0) per_sm = std::min(per_sm, ctx->knobs.rd_ctas);
-    // persistent grid: every resident CTA slot of every SM, but never more lanes than rays
-    const int64_t warps_needed = (a.n_rays + 31) / 32;
-    const int64_t ctas_needed = std::max<int64_t>(1, (warps_needed + (BLOCK / 32) - 1) / (BLOCK / 32));
-    const int grid = (int)std::min<int64_t>((int64_t)ctx->sm_count * per_sm, ctas_needed);
-    if (NeedsPrev<EQ>::value) {
-        const size_t need = (size_t)EQ::NEQ * grid * BLOCK * sizeof(double);
-        if (need > ctx->cap_prev) {
-            cudaFree(ctx->d_prev); ctx->d_prev = nullptr; ctx->cap_prev = 0;
-            CK(cudaMalloc(&ctx->d_prev, need));
-            ctx->cap_prev = need;
-        }
-    }
-    a.prev = ctx->d_prev;
-    a.order = nullptr; a.n_claims = a.n_rays; a.n_long_packets = 0; a.n_quarter_packets = 0; a.counter_long = ctx->d_counters + 4; a.counter_quarter = ctx->d_counters + 5;
-    a.prefer_long = 0; a.long_width = 32;
-    a.packet_refill = ctx->knobs.packet > 0 ? 1 : 0;
-    ctx->last_launches = 0; ctx->last_long_packets = 0; ctx->last_long_ctas = 0; ctx->last_rd_group = 0; ctx->last_quarter_packets = 0;
-    int grid_long = 0;
-    // longest-predicted-ray-first claim order, when a lane will process more than one ray (see trace_kernel.cuh)
-    // knob lpt: 0 = natural order, 1 = automatic (default), 2 = always (used by the tests on small batches)
-    const int lpt_mode = ctx->knobs.lpt;
-    if ((lpt_mode == 2 || (lpt_mode == 1 && a.n_rays > (int64_t)grid * BLOCK)) && a.n_rays < ((int64_t)1 << 32)) {
-        constexpr int group = PacketMode<EQ>::value ? 32 : 1;
-        const int64_t n_entries = ((a.n_rays + group - 1) / group) * group;
-        if (n_entries > ctx->cap_order) {
-            cudaFree(ctx->d_cost); cudaFree(ctx->d_order); ctx->d_cost = ctx->d_order = nullptr; ctx->cap_order = 0;
-            CK(cudaMalloc(&ctx->d_cost, sizeof(uint32_t) * n_entries)); CK(cudaMalloc(&ctx->d_order, sizeof(uint32_t) * n_entries));
-            ctx->cap_order = n_entries;
-        }
-        // d_hist: [0..255] buckets, [256] largest cost, [257] number of long packets, [258..259] cost sum (64 bit), [260..265] grid shape (3 doubles)
-        if (!ctx->d_hist) CK(cudaMalloc(&ctx->d_hist, sizeof(uint32_t) * (kCostBuckets + 16)));
-        CK(cudaMemsetAsync(ctx->d_hist, 0, sizeof(uint32_t) * (kCostBuckets + 16), st));
-        uint32_t* cmax = ctx->d_hist + kCostBuckets;
-        uint32_t* n_long = ctx->d_hist + kCostBuckets + 1;
-        unsigned long long* cost_sum = reinterpret_cast<unsigned long long*>(ctx->d_hist + kCostBuckets + 2);
-        double* shape = reinterpret_cast<double*>(ctx->d_hist + kCostBuckets + 4);
-        uint32_t* n_quarter = ctx->d_hist + kCostBuckets + 10;
-        {   // cost scout: persistent, the table in shared memory when it fits
-            using SEQ = typename EQ::Scout;
-            constexpr int kScoutBlock = ScoutBlock<SEQ>::value;
-            const size_t s_tab = kGrid ? 0 : 16 + tab_bytes;
-            const bool s_in = !kGrid && s_tab <= (size_t)max_optin;
-            const void* sfn = s_in ? (const void*)scout_kernel<SEQ, true> : (const void*)scout_kernel<SEQ, false>;
-            const size_t s_smem = s_in ? s_tab : 16;
-            CK(cudaFuncSetAttribute(sfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s_smem));
-            int s_per_sm = 1;
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&s_per_sm, sfn, kScoutBlock, s_smem));
-            int stride = ctx->knobs.scout_stride > 0 ? ctx->knobs.scout_stride : 1;
-            const int64_t s_need = ((a.n_rays + stride - 1) / stride + kScoutBlock - 1) / kScoutBlock;
-            const int sblocks = (int)std::min<int64_t>((int64_t)ctx->sm_count * std::max(1, s_per_sm), s_need);
-            unsigned long long* scounter = ctx->d_counters + 3;
-            int coarse = ctx->knobs.scout_coarse > 0 ? ctx->knobs.scout_coarse : (kGrid ? kScoutCoarse : 2 * kScoutCoarse);   // stratified: 32x measured best (404.8 vs 421.0 / 443.3 ms at 16x / 64x)
-            const uint32_t* no_list = nullptr; const unsigned long long* no_count = nullptr;
-            void* sargs[] = { (void*)&a, (void*)&ctx->d_cost, (void*)&cmax, (void*)&cost_sum, (void*)&scounter, (void*)&coarse, (void*)&stride, (void*)&no_list, (void*)&no_count };
-            CK(cudaLaunchKernel(sfn, dim3(sblocks), dim3(kScoutBlock), sargs, s_smem, st));
-            if (kGrid && ctx->knobs.refine && coarse > 1) {
-                // second look at the rays the first pass found long, at a quarter of its step multiple (a few per cent of the rays)
-                if (n_entries > ctx->cap_refine) {
-                    cudaFree(ctx->d_refine); ctx->d_refine = nullptr; ctx->cap_refine = 0;
-                    CK(cudaMalloc(&ctx->d_refine, sizeof(uint32_t) * n_entries));
-                    ctx->cap_refine = n_entries;
-                }
-                unsigned long long* n_list = ctx->d_counters + 6; unsigned long long* rcounter = ctx->d_counters + 7;
-                refine_select_kernel<<<ctx->sm_count, 256, 0, st>>>(ctx->d_cost, a.n_rays, cost_sum, (long long)grid * BLOCK, ctx->knobs.long_alpha, ctx->d_refine, n_list);
-                int coarse2 = std::max(1, coarse / 4), one = 1;
-                const uint32_t* lst = ctx->d_refine; const unsigned long long* cnt = n_list;
-                void* rargs[] = { (void*)&a, (void*)&ctx->d_cost, (void*)&cmax, (void*)&cost_sum, (void*)&rcounter, (void*)&coarse2, (void*)&one, (void*)&lst, (void*)&cnt };
-                CK(cudaLaunchKernel(sfn, dim3(sblocks), dim3(kScoutBlock), rargs, s_smem, st));
-                ctx->last_launches += 2;
-            }
-        }
-        const uint32_t* d_cost_used = ctx->d_cost;
-        if (kGrid && ctx->knobs.dilate > 0) {
+// device buffers that only grow: kept across calls, reallocated when a call needs more (need and cap in bytes)
+template <class T>
+static int grow(geoac_ctx* ctx, T*& buf, size_t& cap, size_t need) {
+    if (need <= cap) return GEOAC_OK;
+    cudaFree(buf); buf = nullptr; cap = 0;
+    CK(cudaMalloc(&buf, need));
+    cap = need;
+    return GEOAC_OK;
+}
+
+// cost scout: predicted RK4 step counts of the rays into ctx->d_cost, their maximum and sum.  Persistent, the table in shared
+// memory when it fits.
+template <class SEQ>
+static int launch_cost_scout(geoac_ctx* ctx, const TraceArgs& a, int max_optin, cudaStream_t st, uint32_t* cmax, unsigned long long* cost_sum) {
+    constexpr bool kGrid = PacketMode<SEQ>::value;
+    constexpr int kScoutBlock = ScoutBlock<SEQ>::value;
+    const size_t s_tab = kGrid ? 0 : 16 + (size_t)TAB_NARR * ctx->n * sizeof(double);
+    const bool s_in = !kGrid && s_tab <= (size_t)max_optin;
+    const void* sfn;
+    if constexpr (kGrid) sfn = (const void*)scout_kernel<SEQ, false>;
+    else sfn = s_in ? (const void*)scout_kernel<SEQ, true> : (const void*)scout_kernel<SEQ, false>;
+    const size_t s_smem = s_in ? s_tab : 16;
+    CK(cudaFuncSetAttribute(sfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s_smem));
+    int s_per_sm = 1;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&s_per_sm, sfn, kScoutBlock, s_smem));
+    const int sblocks = (int)std::min<int64_t>((int64_t)ctx->sm_count * std::max(1, s_per_sm), (a.n_rays + kScoutBlock - 1) / kScoutBlock);
+    unsigned long long* scounter = ctx->d_counters + 3;
+    int coarse = ctx->knobs.scout_coarse > 0 ? ctx->knobs.scout_coarse : (kGrid ? kScoutCoarse : 2 * kScoutCoarse);   // stratified: 32x measured best (404.8 vs 421.0 / 443.3 ms at 16x / 64x)
+    void* sargs[] = { (void*)&a, (void*)&ctx->d_cost, (void*)&cmax, (void*)&cost_sum, (void*)&scounter, (void*)&coarse };
+    CK(cudaLaunchKernel(sfn, dim3(sblocks), dim3(kScoutBlock), sargs, s_smem, st));
+    ctx->last_launches += 1;
+    return GEOAC_OK;
+}
+
+// Step 1: the longest-predicted-ray-first claim order (trace_kernel.cuh): cost scout, (range-dependent sets) cost dilation, sort.
+// Sets a.order, a.n_claims, a.packet_refill and a.n_long_packets; n_quarter = long packets long enough for quarter claims.
+// `lanes` = lanes of the main launch (the average work of a lane is the scout's cost sum over them).
+template <class EQ>
+static int build_claim_order(geoac_ctx* ctx, TraceArgs& a, long long lanes, int max_optin, cudaStream_t st, int64_t& n_quarter) {
+    constexpr bool kGrid = PacketMode<EQ>::value;
+    constexpr int group = kGrid ? 32 : 1;                     // range-dependent sets: packets of 32 consecutive rays
+    const int64_t n = a.n_rays, n_entries = ((n + group - 1) / group) * group;
+    const size_t ids = sizeof(uint32_t) * n_entries;
+    // d_hist: [0..255] buckets, [256] largest cost, [257] long packets, [258] quarter packets, [260..261] cost sum (64 bit)
+    const size_t hist_bytes = sizeof(uint32_t) * (kCostBuckets + 8);
+    int rc;
+    if ((rc = grow(ctx, ctx->d_cost, ctx->cap_cost, ids)) || (rc = grow(ctx, ctx->d_order, ctx->cap_order, ids))
+        || (rc = grow(ctx, ctx->d_hist, ctx->cap_hist, hist_bytes))) return rc;
+    CK(cudaMemsetAsync(ctx->d_hist, 0, hist_bytes, st));
+    uint32_t* cmax = ctx->d_hist + kCostBuckets;
+    uint32_t* n_long = cmax + 1;                              // n_long[1]: quarter packets
+    unsigned long long* cost_sum = reinterpret_cast<unsigned long long*>(cmax + 4);
+    if ((rc = launch_cost_scout<typename EQ::Scout>(ctx, a, max_optin, st, cmax, cost_sum))) return rc;
+    if (kGrid) {
+        const uint32_t* cost = ctx->d_cost;
+        if (ctx->knobs.dilate > 0) {
             // the estimate used for the claim order: maximum over the inclination neighbours (trace_kernel.cuh: cost_dilate_kernel)
-            if (n_entries > ctx->cap_refine) {
-                cudaFree(ctx->d_refine); ctx->d_refine = nullptr; ctx->cap_refine = 0;
-                CK(cudaMalloc(&ctx->d_refine, sizeof(uint32_t) * n_entries));
-                ctx->cap_refine = n_entries;
-            }
-            cost_dilate_kernel<<<ctx->sm_count * 2, 256, 0, st>>>(ctx->d_cost, a.theta, a.n_rays, ctx->knobs.dilate * 1e-3 * kPi / 180.0, 16, ctx->d_refine);
-            d_cost_used = ctx->d_refine;
+            if ((rc = grow(ctx, ctx->d_cost_dilated, ctx->cap_cost_dilated, ids))) return rc;
+            cost_dilate_kernel<<<ctx->sm_count * 2, 256, 0, st>>>(ctx->d_cost, a.theta, n, ctx->knobs.dilate * 1e-3 * kPi / 180.0, 16, ctx->d_cost_dilated);
+            cost = ctx->d_cost_dilated;
             ctx->last_launches += 1;
         }
-        // Range-dependent sets: which 32 rays make a packet (trace_kernel.cuh: grid_shape_kernel).  The choice only schedules.
-        bool by_theta = !PacketMode<EQ>::value;
-        if (PacketMode<EQ>::value) {
-            int mode = ctx->knobs.rd_group;
-            if (mode < 0) {
-                double h_shape[3] = { 0, 0, 0 };
-                grid_shape_kernel<<<1, 1024, 0, st>>>(a.theta, a.phi, a.n_rays, shape);
-                CK(cudaMemcpyAsync(h_shape, shape, sizeof h_shape, cudaMemcpyDeviceToHost, st));
-                CK(cudaStreamSynchronize(st));
-                ctx->last_launches += 1;
-                // spread of a packet per km of path, in cells: 32 dtheta / dz (inclination neighbours) vs 32 dphi / dh (azimuth neighbours)
-                mode = (h_shape[1] > 0.0 && h_shape[0] > 0.0 && ctx->grid_dh > 0.0 && ctx->grid_dz > 0.0
-                        && h_shape[1] / ctx->grid_dh < h_shape[0] / ctx->grid_dz) ? 1 : 0;
-            }
-            by_theta = mode == 1;
-            ctx->last_rd_group = mode;
-        }
+        // packets by cost bucket, longest first; also counts the long and the quarter packets
+        order_hist_kernel<<<ctx->sm_count, 256, 0, st>>>(cost, n, group, cmax, ctx->d_hist, cost_sum, lanes, n_long, ctx->knobs.long_alpha, n_long + 1, ctx->knobs.quarter_alpha);
+        order_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_hist);
+        order_scatter_kernel<<<ctx->sm_count, 256, 0, st>>>(cost, n, group, cmax, ctx->d_hist, ctx->d_order);
+        ctx->last_launches += 3;
+    } else {
         // order by (cost bucket, inclination, batch index) + whole-warp refill: a warp's lanes then read the same few table
-        // records (stratified sets: trace_kernel.cuh) / walk through the same grid cells (range-dependent sets with azimuth
-        // neighbours); knob stable = 0 keeps the plain counting sort for the stratified sets (A/B measurements)
-        if (by_theta && (PacketMode<EQ>::value || ctx->knobs.stable)) {
-            const int nblk = ctx->sm_count;
-            const int64_t n = a.n_rays, chunk = (n + nblk - 1) / nblk;
-            if (!ctx->d_blockhist) CK(cudaMalloc(&ctx->d_blockhist, sizeof(uint32_t) * (size_t)nblk * kCostBuckets + 2 * sizeof(double)));
-            if (n_entries > ctx->cap_keys) {
-                cudaFree(ctx->d_keys); cudaFree(ctx->d_order2); ctx->d_keys = nullptr; ctx->d_order2 = nullptr; ctx->cap_keys = 0;
-                CK(cudaMalloc(&ctx->d_keys, (size_t)3 * n_entries)); CK(cudaMalloc(&ctx->d_order2, sizeof(uint32_t) * n_entries));
-                ctx->cap_keys = n_entries;
-            }
-            double* trange = reinterpret_cast<double*>(ctx->d_blockhist + (size_t)nblk * kCostBuckets);
-            uint8_t *key_t = ctx->d_keys, *key_c = ctx->d_keys + n, *key_t2 = ctx->d_keys + 2 * n;
-            order_theta_range_kernel<<<1, 1024, 0, st>>>(a.theta, n, trange);
-            const int cost_shift = ctx->knobs.cost_shift;
-            auto pass = [&](const uint8_t* key, const uint32_t* src, uint32_t* dst) {
-                stable_hist_kernel<<<nblk, 256, 0, st>>>(key, src, n, chunk, ctx->d_blockhist);
-                stable_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_blockhist, nblk);
-                stable_scatter_kernel<<<nblk, 32, 0, st>>>(key, src, n, chunk, ctx->d_blockhist, dst);
-            };
-            if (PacketMode<EQ>::value) {           // 16-bit inclination key: a packet holds ONE inclination wherever a row of the grid is long enough
-                order_keys16_kernel<<<ctx->sm_count, 256, 0, st>>>(d_cost_used, a.theta, n, cmax, trange, key_t, key_t2, key_c, cost_shift);
-                pass(key_t, nullptr, ctx->d_order);
-                pass(key_t2, ctx->d_order, ctx->d_order2);
-                pass(key_c, ctx->d_order2, ctx->d_order);
-                if (n_entries > n) CK(cudaMemsetAsync(ctx->d_order + n, 0xff, sizeof(uint32_t) * (n_entries - n), st));
-                packet_long_kernel<<<ctx->sm_count, 256, 0, st>>>(ctx->d_order, d_cost_used, n_entries / 32, n, cost_sum, (long long)grid * BLOCK, ctx->knobs.long_alpha, n_long, n_quarter, ctx->knobs.quarter_alpha);
-                ctx->last_launches += 12;
-            } else {
-                order_keys_kernel<<<ctx->sm_count, 256, 0, st>>>(ctx->d_cost, a.theta, n, cmax, trange, key_t, key_c, cost_shift);
-                pass(key_t, nullptr, ctx->d_order2);
-                pass(key_c, ctx->d_order2, ctx->d_order);
-                ctx->last_launches += 8;
-                if (ctx->knobs.packet < 0) a.packet_refill = 1;
-            }
-        } else {
-            order_hist_kernel<<<ctx->sm_count, 256, 0, st>>>(d_cost_used, a.n_rays, group, cmax, ctx->d_hist, cost_sum, (long long)grid * BLOCK, n_long, ctx->knobs.long_alpha, n_quarter, ctx->knobs.quarter_alpha);
-            order_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_hist);
-            order_scatter_kernel<<<ctx->sm_count, 256, 0, st>>>(d_cost_used, a.n_rays, group, cmax, ctx->d_hist, ctx->d_order);
-            ctx->last_launches += 3;
-        }
-        CK(cudaGetLastError());
-        a.n_claims = n_entries;
-        a.order = ctx->d_order;
-        ctx->last_launches += 1;                                        // the cost scout
-        if (PacketMode<EQ>::value && ctx->knobs.coop) {
-            // the long region: packets that would outlast the pass on a fully loaded SM.  Their count sizes the second launch.
-            uint32_t h_long = 0, h_quarter = 0;
-            CK(cudaMemcpyAsync(&h_long, n_long, sizeof h_long, cudaMemcpyDeviceToHost, st));
-            CK(cudaMemcpyAsync(&h_quarter, n_quarter, sizeof h_quarter, cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            a.n_long_packets = std::min<int64_t>(h_long, n_entries / 32);
-            ctx->last_long_packets = (int)a.n_long_packets;
-            if (a.n_long_packets > 0 && ctx->knobs.exclusive && !PATHS) {
-                const int64_t per_cta = (ctx->knobs.long_width == 8) ? kCoopSlots : BLOCK;      // rays a long-region CTA holds at a time
-                const int64_t max_ctas = std::max<int64_t>(1, (int64_t)ctx->sm_count * ctx->knobs.long_sm_pct / 100);
-                grid_long = (int)std::min<int64_t>((a.n_long_packets * 32 + per_cta - 1) / per_cta, max_ctas);
-                grid_long = std::max(grid_long, 1);
-                if (ctx->knobs.long_width == 32 && ctx->knobs.quarter) {
-                    // The very longest packets set the length of the pass: even alone on its scheduler a warp needs ~60 us per step of its
-                    // 32 rays.  Packets whose cost exceeds quarter_alpha % of the average lane work (they would outlast the pass even at
-                    // lone-warp speed) are split over four warps -- quarter claims, four lanes per ray, ~40 us per step -- as far as the
-                    // exclusive SMs have warps to spare.  Measured on one GPU's share of the 8-way config-5 split: 31.4 s -> 22.2 s.
-                    const int64_t warps = max_ctas * (BLOCK / 32);
-                    a.n_quarter_packets = std::min<int64_t>(std::min<int64_t>(a.n_long_packets, h_quarter), std::max<int64_t>(0, (warps - a.n_long_packets) / 3));
-                    grid_long = (int)std::min<int64_t>(max_ctas, (a.n_long_packets + 3 * a.n_quarter_packets + (BLOCK / 32) - 1) / (BLOCK / 32));
-                }
-            }
-        }
+        // records (trace_kernel.cuh).  Two stable counting-sort passes, inclination first.
+        const int nblk = ctx->sm_count;
+        const int64_t chunk = (n + nblk - 1) / nblk;
+        if ((rc = grow(ctx, ctx->d_blockhist, ctx->cap_blockhist, sizeof(uint32_t) * (size_t)nblk * kCostBuckets + 2 * sizeof(double)))
+            || (rc = grow(ctx, ctx->d_keys, ctx->cap_keys, (size_t)2 * n)) || (rc = grow(ctx, ctx->d_order2, ctx->cap_order2, ids))) return rc;
+        double* trange = reinterpret_cast<double*>(ctx->d_blockhist + (size_t)nblk * kCostBuckets);
+        uint8_t *key_t = ctx->d_keys, *key_c = ctx->d_keys + n;
+        order_theta_range_kernel<<<1, 1024, 0, st>>>(a.theta, n, trange);
+        order_keys_kernel<<<ctx->sm_count, 256, 0, st>>>(ctx->d_cost, a.theta, n, cmax, trange, key_t, key_c, ctx->knobs.cost_shift);
+        auto pass = [&](const uint8_t* key, const uint32_t* src, uint32_t* dst) {
+            stable_hist_kernel<<<nblk, 256, 0, st>>>(key, src, n, chunk, ctx->d_blockhist);
+            stable_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_blockhist, nblk);
+            stable_scatter_kernel<<<nblk, 32, 0, st>>>(key, src, n, chunk, ctx->d_blockhist, dst);
+        };
+        pass(key_t, nullptr, ctx->d_order2);
+        pass(key_c, ctx->d_order2, ctx->d_order);
+        ctx->last_launches += 8;
+        a.packet_refill = 1;
     }
-    a.long_width = 32;                                                  // one-thread-per-ray CTAs take whole packets
-    ctx->last_quarter_packets = (int)a.n_quarter_packets;
+    CK(cudaGetLastError());
+    a.n_claims = n_entries;
+    a.order = ctx->d_order;
+    n_quarter = 0;
+    if (kGrid && ctx->knobs.coop) {
+        // the long region: packets that would outlast the pass on a fully loaded SM.  Their count sizes the second launch.
+        uint32_t h[2] = { 0, 0 };
+        CK(cudaMemcpyAsync(h, n_long, sizeof h, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        a.n_long_packets = std::min<int64_t>(h[0], n_entries / 32);
+        n_quarter = h[1];
+    }
+    return GEOAC_OK;
+}
+
+// Step 2: CTAs of the exclusive long-region launch (0 = none: the main launch drains the long region first).  Sets
+// a.n_quarter_packets.  The capture kernels always run as one launch.
+static int size_long_region(const geoac_ctx* ctx, TraceArgs& a, int64_t n_quarter, int block, bool paths) {
+    if (a.n_long_packets == 0 || !ctx->knobs.exclusive || paths) return 0;
+    const int64_t max_ctas = std::max<int64_t>(1, (int64_t)ctx->sm_count * ctx->knobs.long_sm_pct / 100);
+    if (!ctx->knobs.quarter) return (int)std::max<int64_t>(1, std::min<int64_t>((a.n_long_packets * 32 + block - 1) / block, max_ctas));
+    // The very longest packets set the length of the pass: even alone on its scheduler a warp needs ~60 us per step of its
+    // 32 rays.  Packets whose cost exceeds quarter_alpha % of the average lane work (they would outlast the pass even at
+    // lone-warp speed) are split over four warps -- quarter claims, four lanes per ray, ~40 us per step -- as far as the
+    // exclusive SMs have warps to spare.  Measured on one GPU's share of the 8-way config-5 split: 31.4 s -> 22.2 s.
+    const int64_t warps = max_ctas * (block / 32);
+    a.n_quarter_packets = std::min<int64_t>(std::min<int64_t>(a.n_long_packets, n_quarter), std::max<int64_t>(0, (warps - a.n_long_packets) / 3));
+    return (int)std::min<int64_t>(max_ctas, (a.n_long_packets + 3 * a.n_quarter_packets + (block / 32) - 1) / (block / 32));
+}
+
+// Step 3: the trace launch(es).  With a long region of its own, two concurrent launches of the same kernel: the long region
+// -- packets that would outlast the pass on a loaded SM -- goes to CTAs that keep their SM to themselves (their
+// shared-memory request leaves no room for a main CTA), launched first on a high-priority stream; the main launch fills the
+// other SMs, and its surplus CTAs start as SMs free up.  Each side drains its own region first and then helps with the other.
+template <class EQ, int BLOCK>
+static int enqueue_launches(geoac_ctx* ctx, const void* fn, size_t smem, int max_optin, int grid, int grid_long, TraceArgs a, cudaStream_t st) {
     if (grid_long > 0) {
-        // Two concurrent launches.  The long region -- packets that would outlast the pass on a loaded SM -- goes to CTAs that
-        // keep their SM to themselves (their shared-memory request leaves no room for a main CTA), launched first on a
-        // high-priority stream; the main launch fills the other SMs, and its surplus CTAs start as SMs free up.  Each side
-        // drains its own region first and then helps with the other.  knob long_width = 32 (default): the same one-thread-per-ray
-        // kernel; 8: the cooperative kernel (four lanes per ray, the ray's cell in shared memory via TMA: trace_kernel.cuh), which
-        // measured at half the throughput and is kept for A/B runs.
-        const bool coop = ctx->knobs.long_width == 8;
-        const void* fn_long = fn; size_t smem_long = 0; int block_long = BLOCK; size_t lanes_long = (size_t)grid_long * BLOCK;
-        if constexpr (PacketMode<EQ>::value) {
-            if (coop) { fn_long = (const void*)trace_coop_kernel<EQ>; smem_long = CoopLayout<EQ>::bytes(); block_long = kCoopBlock; lanes_long = (size_t)grid_long * kCoopSlots; }
-        }
-        if (!smem_long) smem_long = std::min((size_t)max_optin, std::max(smem, (size_t)max_optin - smem + 4096));   // no room for a main CTA beside it
-        if (smem_long > (size_t)max_optin) return fail(ctx, GEOAC_ERR_CUDA, "cooperative kernel does not fit in shared memory");
-        CK(cudaFuncSetAttribute(fn_long, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_long));
-        if (NeedsPrev<EQ>::value) {
-            const size_t need = (size_t)EQ::NEQ * ((size_t)grid * BLOCK + lanes_long) * sizeof(double);
-            if (need > ctx->cap_prev) {
-                CK(cudaStreamSynchronize(st));
-                cudaFree(ctx->d_prev); ctx->d_prev = nullptr; ctx->cap_prev = 0;
-                CK(cudaMalloc(&ctx->d_prev, need));
-                ctx->cap_prev = need;
-            }
-            a.prev = ctx->d_prev;
-        }
+        const size_t smem_long = std::min((size_t)max_optin, std::max(smem, (size_t)max_optin - smem + 4096));
+        CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_long));
         TraceArgs al = a;
         al.prefer_long = 1;
-        if (NeedsPrev<EQ>::value) al.prev = ctx->d_prev + (size_t)EQ::NEQ * grid * BLOCK;
+        if (NeedsPrev<EQ>::value) {                          // y_{k-1} scratch of both launches, the long one's after the main one's
+            const size_t main_doubles = (size_t)EQ::NEQ * grid * BLOCK;
+            const size_t need = (main_doubles + (size_t)EQ::NEQ * grid_long * BLOCK) * sizeof(double);
+            if (need > ctx->cap_prev) {
+                CK(cudaStreamSynchronize(st));                // a trace still running may use the old scratch
+                if (int rc = grow(ctx, ctx->d_prev, ctx->cap_prev, need)) return rc;
+            }
+            a.prev = ctx->d_prev;
+            al.prev = ctx->d_prev + main_doubles;
+        }
         CK(cudaEventRecord(ctx->ev_fork, st));
         CK(cudaStreamWaitEvent(ctx->stream_long, ctx->ev_fork, 0));
         void* largs[] = { (void*)&al };
         CK(cudaEventRecord(ctx->ev_l0, ctx->stream_long));
-        CK(cudaLaunchKernel(fn_long, dim3(grid_long), dim3(block_long), largs, smem_long, ctx->stream_long));
+        CK(cudaLaunchKernel(fn, dim3(grid_long), dim3(BLOCK), largs, smem_long, ctx->stream_long));
         CK(cudaEventRecord(ctx->ev_l1, ctx->stream_long));
         CK(cudaEventRecord(ctx->ev_join, ctx->stream_long));
         ctx->last_launches += 1; ctx->last_long_ctas = grid_long;
@@ -740,6 +643,68 @@ static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
     if (grid_long > 0) CK(cudaStreamWaitEvent(st, ctx->ev_join, 0));
     ctx->last_launches += 1;
     return GEOAC_OK;
+}
+
+template <class EQ, int BLOCK, bool PATHS>
+static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
+    constexpr bool kGrid = PacketMode<EQ>::value;
+    const size_t lane_doubles = ((size_t)LaneLayout<EQ>::STRIDE * BLOCK + 1) & ~(size_t)1;
+    const size_t fixed = ((sizeof(LaunchConsts) + 15) / 16) * 16 + 16 + lane_doubles * sizeof(double);
+    const size_t tab_bytes = kGrid ? 0 : (size_t)TAB_NARR * ctx->n * sizeof(double);
+    int max_optin = 0;
+    CK(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+    if (fixed > (size_t)max_optin) return fail(ctx, GEOAC_ERR_CUDA, "lane records do not fit in shared memory");
+    const bool in_smem = !kGrid && fixed + tab_bytes <= (size_t)max_optin;
+    const size_t smem = in_smem ? fixed + tab_bytes : fixed;
+    // the range-dependent node tables, and a profile too large for shared memory, are read through L1 / L2
+    const void* fn;
+    if constexpr (kGrid) fn = (const void*)trace_kernel<EQ, BLOCK, false, PATHS>;
+    else fn = in_smem ? (const void*)trace_kernel<EQ, BLOCK, true, PATHS> : (const void*)trace_kernel<EQ, BLOCK, false, PATHS>;
+    CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 1;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, BLOCK, smem));
+    if (per_sm < 1) return fail(ctx, GEOAC_ERR_CUDA, "trace kernel does not fit on an SM");
+    // persistent grid: every resident CTA slot of every SM, but never more lanes than rays
+    const int64_t warps_needed = (a.n_rays + 31) / 32;
+    const int64_t ctas_needed = std::max<int64_t>(1, (warps_needed + (BLOCK / 32) - 1) / (BLOCK / 32));
+    const int grid = (int)std::min<int64_t>((int64_t)ctx->sm_count * per_sm, ctas_needed);
+    if (NeedsPrev<EQ>::value) {
+        if (int rc = grow(ctx, ctx->d_prev, ctx->cap_prev, (size_t)EQ::NEQ * grid * BLOCK * sizeof(double))) return rc;
+    }
+    a.prev = ctx->d_prev;
+    a.order = nullptr; a.n_claims = a.n_rays; a.n_long_packets = 0; a.n_quarter_packets = 0; a.counter_long = ctx->d_counters + 4; a.counter_quarter = ctx->d_counters + 5;
+    a.prefer_long = 0; a.packet_refill = 0;
+    ctx->last_launches = 0; ctx->last_long_packets = 0; ctx->last_long_ctas = 0; ctx->last_quarter_packets = 0;
+    int grid_long = 0;
+    // longest-predicted-ray-first claim order, when a lane will process more than one ray (see trace_kernel.cuh)
+    // knob lpt: 0 = natural order, 1 = automatic (default), 2 = always (used by the tests on small batches)
+    const int lpt_mode = ctx->knobs.lpt;
+    if ((lpt_mode == 2 || (lpt_mode == 1 && a.n_rays > (int64_t)grid * BLOCK)) && a.n_rays < ((int64_t)1 << 32)) {
+        int64_t n_quarter = 0;
+        if (int rc = build_claim_order<EQ>(ctx, a, (long long)grid * BLOCK, max_optin, st, n_quarter)) return rc;
+        grid_long = size_long_region(ctx, a, n_quarter, BLOCK, PATHS);
+    }
+    ctx->last_long_packets = (int)a.n_long_packets;
+    ctx->last_quarter_packets = (int)a.n_quarter_packets;
+    return enqueue_launches<EQ, BLOCK>(ctx, fn, smem, max_optin, grid, grid_long, a, st);
+}
+
+// variant -> (equation set, lanes per CTA); PATHS: the raypath / caustic capture kernels (same lanes per SM as the plain ones)
+template <bool PATHS>
+static int dispatch_trace(geoac_ctx* ctx, const TraceArgs& a, cudaStream_t st) {
+    const bool amp = ctx->prm.calc_amp != 0;
+    switch (ctx->variant) {
+        case GEOAC_2D:     return amp ? launch_trace<Eq2D<true>, 512, PATHS>(ctx, a, st) : launch_trace<Eq2D<false>, 512, PATHS>(ctx, a, st);
+        // Eq3D<true>: 384 lanes = 3 warps per scheduler at <= 168 registers, no spills (420 ms per config-2 pass vs 491 (256) /
+        // 494 (512) in round 1).  Nothing in between exists: the register file is four 16 K-register banks, one per scheduler, so
+        // 13 or 14 warps put 4 on some scheduler and cap every lane at 128 registers -- the 512-lane case, which spills (measured
+        // on B200: 416 / 448 lanes at 152 / 144 registers compile without spills but do not fit on an SM).
+        case GEOAC_3D:     return amp ? launch_trace<Eq3D<true>, 384, PATHS>(ctx, a, st) : launch_trace<Eq3D<false>, 512, PATHS>(ctx, a, st);
+        case GEOAC_GLOBAL: return amp ? launch_trace<EqGlobal<true>, 384, PATHS>(ctx, a, st) : launch_trace<EqGlobal<false>, 512, PATHS>(ctx, a, st);
+        case GEOAC_3D_RNGDEP:     return amp ? launch_trace<Eq3DRD<true>, 128, PATHS>(ctx, a, st)     : launch_trace<Eq3DRD<false>, 128, PATHS>(ctx, a, st);
+        case GEOAC_GLOBAL_RNGDEP: return amp ? launch_trace<EqGlobalRD<true>, 128, PATHS>(ctx, a, st) : launch_trace<EqGlobalRD<false>, 128, PATHS>(ctx, a, st);
+    }
+    return fail(ctx, GEOAC_ERR_BAD_ARG, "variant not implemented");
 }
 
 struct PathArgs { double* path = nullptr; int32_t* rows = nullptr; int stride = 0; int64_t cap = 0;
@@ -769,37 +734,7 @@ static int enqueue_trace(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, 
     a.counter = ctx->d_counters; a.total_steps = ctx->d_counters + 1; a.warp_trips = ctx->d_counters + 2;
     a.path = pa.path; a.path_rows = pa.rows; a.path_stride = pa.stride; a.path_cap = pa.cap;
     a.caus = pa.caus; a.caus_rows = pa.caus_rows; a.caus_cap = pa.caus_cap;
-    const bool amp = ctx->prm.calc_amp != 0;
-    if (pa.stride > 0 || pa.caus_cap > 0) {          // raypath / caustic capture: the PATHS instantiations (same lanes per SM as the plain ones)
-        switch (ctx->variant) {
-            case GEOAC_2D:     return amp ? launch_trace<Eq2D<true>, 512, true>(ctx, a, st)     : launch_trace<Eq2D<false>, 512, true>(ctx, a, st);
-            case GEOAC_3D:     return amp ? launch_trace<Eq3D<true>, 384, true>(ctx, a, st)     : launch_trace<Eq3D<false>, 512, true>(ctx, a, st);
-            case GEOAC_GLOBAL: return amp ? launch_trace<EqGlobal<true>, 384, true>(ctx, a, st) : launch_trace<EqGlobal<false>, 512, true>(ctx, a, st);
-            case GEOAC_3D_RNGDEP:     return amp ? launch_trace<Eq3DRD<true>, 128, true>(ctx, a, st)     : launch_trace<Eq3DRD<false>, 128, true>(ctx, a, st);
-            case GEOAC_GLOBAL_RNGDEP: return amp ? launch_trace<EqGlobalRD<true>, 128, true>(ctx, a, st) : launch_trace<EqGlobalRD<false>, 128, true>(ctx, a, st);
-        }
-    }
-    switch (ctx->variant) {
-        case GEOAC_2D:     return amp ? launch_trace<Eq2D<true>, 512>(ctx, a, st)     : launch_trace<Eq2D<false>, 512>(ctx, a, st);
-        case GEOAC_3D: {
-            if (!amp) return launch_trace<Eq3D<false>, 512>(ctx, a, st);
-            // tuning knob for experiments (lanes per SM vs registers per lane); the default is the measured best
-            const int blk = ctx->knobs.block3d;
-            if (blk == 256) return launch_trace<Eq3D<true>, 256>(ctx, a, st);
-            if (blk == 512) return launch_trace<Eq3D<true>, 512>(ctx, a, st);
-            // 384 lanes = 3 warps per scheduler at <= 168 registers, no spills (420 ms per config-2 pass vs 491 (256) / 494 (512) in round 1).
-            // Nothing in between exists: the register file is four 16 K-register banks, one per scheduler, so 13 or 14 warps put 4
-            // on some scheduler and cap every lane at 128 registers -- the 512-lane case, which spills (measured on B200: 416 / 448
-            // lanes at 152 / 144 registers compile without spills but do not fit on an SM).
-            return launch_trace<Eq3D<true>, 384>(ctx, a, st);
-        }
-#ifdef GEOAC_HAVE_GLOBAL
-        case GEOAC_GLOBAL: return amp ? launch_trace<EqGlobal<true>, 384>(ctx, a, st) : launch_trace<EqGlobal<false>, 512>(ctx, a, st);
-#endif
-        case GEOAC_3D_RNGDEP:     return amp ? launch_trace<Eq3DRD<true>, 128>(ctx, a, st)     : launch_trace<Eq3DRD<false>, 128>(ctx, a, st);
-        case GEOAC_GLOBAL_RNGDEP: return amp ? launch_trace<EqGlobalRD<true>, 128>(ctx, a, st) : launch_trace<EqGlobalRD<false>, 128>(ctx, a, st);
-    }
-    return fail(ctx, GEOAC_ERR_BAD_ARG, "variant not implemented");
+    return (pa.stride > 0 || pa.caus_cap > 0) ? dispatch_trace<true>(ctx, a, st) : dispatch_trace<false>(ctx, a, st);
 }
 
 extern "C" int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, const double* d_phi,
@@ -812,19 +747,11 @@ extern "C" int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* 
 
 // device staging of the host-buffer entry point (angles in, records out), grown on demand and kept across calls
 static int reserve_staging(geoac_ctx* ctx, int64_t n_rays) {
-    const int64_t n_slots = n_rays * (ctx->prm.bounces + 1);
-    if (n_rays > ctx->cap_rays) {
-        cudaFree(ctx->d_theta); cudaFree(ctx->d_phi); ctx->d_theta = ctx->d_phi = nullptr; ctx->cap_rays = 0;
-        CK(cudaMalloc(&ctx->d_theta, sizeof(double) * n_rays)); CK(cudaMalloc(&ctx->d_phi, sizeof(double) * n_rays));
-        ctx->cap_rays = n_rays;
-    }
-    if (n_slots > ctx->cap_slots) {
-        cudaFree(ctx->d_rec); cudaFree(ctx->d_status); cudaFree(ctx->d_nsteps);
-        ctx->d_rec = nullptr; ctx->d_status = ctx->d_nsteps = nullptr; ctx->cap_slots = 0;
-        CK(cudaMalloc(&ctx->d_rec, sizeof(double) * GEOAC_NFIELDS * n_slots));
-        CK(cudaMalloc(&ctx->d_status, sizeof(int32_t) * n_slots)); CK(cudaMalloc(&ctx->d_nsteps, sizeof(int32_t) * n_slots));
-        ctx->cap_slots = n_slots;
-    }
+    const size_t n_slots = (size_t)n_rays * (ctx->prm.bounces + 1);
+    int rc;
+    if ((rc = grow(ctx, ctx->d_theta, ctx->cap_theta, sizeof(double) * n_rays)) || (rc = grow(ctx, ctx->d_phi, ctx->cap_phi, sizeof(double) * n_rays))
+        || (rc = grow(ctx, ctx->d_rec, ctx->cap_rec, sizeof(double) * GEOAC_NFIELDS * n_slots))
+        || (rc = grow(ctx, ctx->d_status, ctx->cap_status, sizeof(int32_t) * n_slots)) || (rc = grow(ctx, ctx->d_nsteps, ctx->cap_nsteps, sizeof(int32_t) * n_slots))) return rc;
     return GEOAC_OK;
 }
 
@@ -839,14 +766,6 @@ extern "C" int geoac_reserve(geoac_ctx* ctx, int64_t n_rays) {
     if (!ctx || n_rays < 0) return GEOAC_ERR_BAD_ARG;
     cudaSetDevice(ctx->device);
     return reserve_staging(ctx, n_rays);
-}
-
-static int grow(geoac_ctx* ctx, void** buf, size_t* cap, size_t need) {
-    if (need <= *cap) return GEOAC_OK;
-    cudaFree(*buf); *buf = nullptr; *cap = 0;
-    CK(cudaMalloc(buf, need));
-    *cap = need;
-    return GEOAC_OK;
 }
 
 static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
@@ -869,16 +788,16 @@ static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const
     cudaStream_t st = ctx->stream;
     if (path_stride > 0) {
         const size_t need = (size_t)n_rays * path_cap * GEOAC_PATH_NF * sizeof(double);
-        int g1 = grow(ctx, (void**)&ctx->d_path, &ctx->cap_path, need); if (g1) return g1;
-        int g2 = grow(ctx, (void**)&ctx->d_path_rows, &ctx->cap_path_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
+        int g1 = grow(ctx, ctx->d_path, ctx->cap_path, need); if (g1) return g1;
+        int g2 = grow(ctx, ctx->d_path_rows, ctx->cap_path_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
         CK(cudaMemsetAsync(ctx->d_path, 0, need, st));
         CK(cudaMemsetAsync(ctx->d_path_rows, 0, sizeof(int32_t) * n_rays, st));
         pa.path = ctx->d_path; pa.rows = ctx->d_path_rows; pa.stride = path_stride; pa.cap = path_cap;
     }
     if (caus_cap > 0) {
         const size_t need = (size_t)n_rays * caus_cap * GEOAC_CAUSTIC_NF * sizeof(double);
-        int g1 = grow(ctx, (void**)&ctx->d_caus, &ctx->cap_caus, need); if (g1) return g1;
-        int g2 = grow(ctx, (void**)&ctx->d_caus_rows, &ctx->cap_caus_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
+        int g1 = grow(ctx, ctx->d_caus, ctx->cap_caus, need); if (g1) return g1;
+        int g2 = grow(ctx, ctx->d_caus_rows, ctx->cap_caus_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
         CK(cudaMemsetAsync(ctx->d_caus, 0, need, st));
         CK(cudaMemsetAsync(ctx->d_caus_rows, 0, sizeof(int32_t) * n_rays, st));
         pa.caus = ctx->d_caus; pa.caus_rows = ctx->d_caus_rows; pa.caus_cap = caus_cap;
@@ -962,15 +881,15 @@ extern "C" int geoac_trace_paths_compact(geoac_ctx* ctx, int64_t n_rays, const d
     cudaStream_t st = ctx->stream;
     if (path_stride > 0) {
         const size_t need = (size_t)n_rays * path_cap * GEOAC_PATH_NF * sizeof(double);
-        int g1 = grow(ctx, (void**)&ctx->d_path, &ctx->cap_path, need); if (g1) return g1;
-        int g2 = grow(ctx, (void**)&ctx->d_path_rows, &ctx->cap_path_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
+        int g1 = grow(ctx, ctx->d_path, ctx->cap_path, need); if (g1) return g1;
+        int g2 = grow(ctx, ctx->d_path_rows, ctx->cap_path_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
         CK(cudaMemsetAsync(ctx->d_path_rows, 0, sizeof(int32_t) * n_rays, st));
         pa.path = ctx->d_path; pa.rows = ctx->d_path_rows; pa.stride = path_stride; pa.cap = path_cap;
     }
     if (caustic_cap > 0) {
         const size_t need = (size_t)n_rays * caustic_cap * GEOAC_CAUSTIC_NF * sizeof(double);
-        int g1 = grow(ctx, (void**)&ctx->d_caus, &ctx->cap_caus, need); if (g1) return g1;
-        int g2 = grow(ctx, (void**)&ctx->d_caus_rows, &ctx->cap_caus_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
+        int g1 = grow(ctx, ctx->d_caus, ctx->cap_caus, need); if (g1) return g1;
+        int g2 = grow(ctx, ctx->d_caus_rows, ctx->cap_caus_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
         CK(cudaMemsetAsync(ctx->d_caus_rows, 0, sizeof(int32_t) * n_rays, st));
         pa.caus = ctx->d_caus; pa.caus_rows = ctx->d_caus_rows; pa.caus_cap = caustic_cap;
     }
@@ -1018,13 +937,12 @@ extern "C" int geoac_trace_paths_compact(geoac_ctx* ctx, int64_t n_rays, const d
     return GEOAC_OK;
 }
 
-// Scheduling facts of the last trace (range-dependent sets): out[0] packet grouping used (0 = consecutive rays, 1 = equal
-// inclination / neighbouring azimuth), out[1] packets in the long region, out[2] CTAs of the exclusive long-region launch,
-// out[3] kernels enqueued.
+// Scheduling facts of the last trace (range-dependent sets): out[0] reserved (0), out[1] packets in the long region, out[2] CTAs
+// of the exclusive long-region launch, out[3] kernels enqueued, out[4] long packets claimed as quarter packets.
 extern "C" int geoac_last_schedule(geoac_ctx* ctx, int64_t* out8) {
     if (!ctx || !out8) return GEOAC_ERR_BAD_ARG;
     for (int i = 0; i < 8; i++) out8[i] = 0;
-    out8[0] = ctx->last_rd_group; out8[1] = ctx->last_long_packets; out8[2] = ctx->last_long_ctas; out8[3] = ctx->last_launches;
+    out8[1] = ctx->last_long_packets; out8[2] = ctx->last_long_ctas; out8[3] = ctx->last_launches;
     out8[4] = ctx->last_quarter_packets;
     return GEOAC_OK;
 }
@@ -1032,7 +950,7 @@ extern "C" int geoac_last_schedule(geoac_ctx* ctx, int64_t* out8) {
 // claim order was built.
 extern "C" int geoac_get_costs(geoac_ctx* ctx, int64_t n, uint32_t* cost) {
     if (!ctx || !cost || n < 0) return GEOAC_ERR_BAD_ARG;
-    if (!ctx->d_cost || n > ctx->cap_order) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_get_costs: no claim order of that size was built");
+    if (!ctx->d_cost || (size_t)n * sizeof(uint32_t) > ctx->cap_cost) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_get_costs: no claim order of that size was built");
     cudaSetDevice(ctx->device);
     CK(cudaMemcpy(cost, ctx->d_cost, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost));
     return GEOAC_OK;

@@ -365,7 +365,7 @@ struct EqGlobalRD {
         const double cn = c * g_rsqrt(n0 * n0 + n1 * n1 + n2 * n2);
         const double c0 = cn * n0, c1 = cn * n1 + w[2], c2 = cn * n2 + w[1];
         dtt = ds_tt * g_rsqrt(c0 * c0 + c1 * c1 + c2 * c2);
-        {   // reference state at the lowest levels under the query point; the ray's own cursor carries the cache tags
+        {   // reference state at the lowest levels under the query point: the vertical search starts from the bottom cell
             const int kz_ray = cur.kz;
             cur.kz = 0;
             ms_wrappers<true, true, false, true>(G, tm, pm, L.z_grnd, cur, wr, dzs);

@@ -38,22 +38,11 @@ struct Grid3D {
     // cooperative mode (trace_kernel.cuh, straggler acceleration): `nrole` = 4 lanes advance ONE ray together, lane `role`
     // evaluates row `role` of the 4x4 node block; lanes glane0 .. glane0+3 (mask gmask) form the group.  nrole = 1: serial.
     int role, nrole, glane0; unsigned gmask;
-    // per-ray CELL CACHE in shared memory (cooperative kernel, trace_kernel.cuh): the 4 x 4 x 2 node block of the cell the ray
-    // is in -- 16 columns x { 2 levels x 18 doubles of tuv | 2 levels x 2 doubles of rho } = 5 120 bytes -- pulled from global
-    // memory by TMA bulk copies when the ray enters a new cell and read from shared memory by every sample until it leaves
-    // (a ray takes >= 10 steps = 50 samples per vertical cell, thousands per horizontal one).  cache_tuv == nullptr: no cache.
-    double* cache_tuv = nullptr; double* cache_rho = nullptr;
-    double* cache_gnd = nullptr;      // Global.RngDep: T and rho of the two lowest levels of the same 16 columns (absorption reference state)
-    uint64_t* cache_bar = nullptr;    // two mbarriers: [0] cell block, [1] ground block
 };
 constexpr int MS_SCRATCH = 30;
-constexpr int MS_CACHE_COL = 36;                 // doubles per column in the tuv cache (2 levels x 18)
-constexpr int MS_CACHE_TUV = 16 * MS_CACHE_COL;  // 576 doubles
-constexpr int MS_CACHE_RHO = 16 * 4;             // 64 doubles
-constexpr int MS_CACHE_GND = 2 * 16 * 4;         // T then rho: [16 columns][2 levels][f, slope]
 
-// cursor of a ray: cell of the last look-up, and the cells its caches hold (cooperative kernel)
-struct Cur3 { int ka, kb, kz; int ca = -1, cb = -1, cz = -1, ga = -1, gb = -1, gz = -1; unsigned phase = 0; };
+// cursor of a ray: cell of the last look-up
+struct Cur3 { int ka, kb, kz; };
 
 // Axis tables: one 32-byte record per node index k,
 //   { x[k], 1/(x[k+1]-x[k]), 1/(x[k+1]-x[max(k-1,0)]), 1/(x[min(k+2,n-1)]-x[k]) }
@@ -260,70 +249,6 @@ GEOAC_HD void ms_group_take(double (&acc)[N], const Grid3D& g, int row) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Cell cache (cooperative kernel).  ms_cache_cell makes sure the ray's cache holds cell (ka, kb, kz): on a miss the lanes of the
-// group issue one 288-byte (tuv, both levels of a column are contiguous) and one 32-byte (rho) cp.async.bulk per column of their
-// row, completion is counted on the ray's mbarrier, and every lane of the group waits for the phase to flip.
-// ---------------------------------------------------------------------------------------------------------------
-#if defined(__CUDA_ARCH__)
-__device__ __forceinline__ uint32_t ms_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void ms_bulk_g2s(void* dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(ms_smem_u32(dst)), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void ms_bar_wait(uint32_t bar, unsigned parity) {
-    unsigned done = 0;
-    while (!done)
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void ms_cache_cell(const Grid3D& g, Cur3& cur, const unsigned (&aoff)[4], const unsigned (&boff)[4]) {
-    if (cur.ca == cur.ka && cur.cb == cur.kb && cur.cz == cur.kz) return;
-    const uint32_t bar = ms_smem_u32(g.cache_bar);
-    __syncwarp(g.gmask);                                                   // nobody of the group still reads the old block
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");           // generic-proxy reads before async-proxy writes
-    if (g.role == 0) asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)(16 * 320)) : "memory");
-    __syncwarp(g.gmask);
-    for (int jb = g.role; jb < 4; jb += g.nrole) {
-#pragma unroll
-        for (int ia = 0; ia < 4; ia++) {
-            const unsigned node = aoff[ia] + boff[jb];                     // element offset of the column in tuv (18 doubles per level)
-            const unsigned kofs = (unsigned)cur.kz * MS_STRIDE;
-            ms_bulk_g2s(g.cache_tuv + (jb * 4 + ia) * MS_CACHE_COL, g.tuv + node + kofs, 2 * MS_STRIDE * 8, bar);
-            ms_bulk_g2s(g.cache_rho + (jb * 4 + ia) * 4, g.rho + (node + kofs) / (MS_STRIDE / 2), 32, bar);
-        }
-    }
-    ms_bar_wait(bar, cur.phase & 1u);
-    cur.phase ^= 1u;
-    cur.ca = cur.ka; cur.cb = cur.kb; cur.cz = cur.kz;
-}
-// ground block: T (f, slope) and rho (f, slope) of levels 0 and 1 of the same 16 columns (Global.RngDep absorption reference)
-__device__ __forceinline__ void ms_cache_ground(const Grid3D& g, Cur3& cur, const unsigned (&aoff)[4], const unsigned (&boff)[4]) {
-    if (cur.ga == cur.ka && cur.gb == cur.kb && cur.gz == cur.kz) return;
-    const uint32_t bar = ms_smem_u32(g.cache_bar + 1);
-    __syncwarp(g.gmask);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    if (g.role == 0) asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)(16 * 64)) : "memory");
-    __syncwarp(g.gmask);
-    for (int jb = g.role; jb < 4; jb += g.nrole) {
-#pragma unroll
-        for (int ia = 0; ia < 4; ia++) {
-            const unsigned node = aoff[ia] + boff[jb] + (unsigned)cur.kz * MS_STRIDE;
-            const int c = jb * 4 + ia;
-            ms_bulk_g2s(g.cache_gnd + c * 4, g.tuv + node, 16, bar);                                   // T: f, slope at the lower level
-            ms_bulk_g2s(g.cache_gnd + c * 4 + 2, g.tuv + node + MS_STRIDE, 16, bar);                   // ... at the upper level
-            ms_bulk_g2s(g.cache_gnd + 64 + c * 4, g.rho + node / (MS_STRIDE / 2), 32, bar);            // rho: both levels
-        }
-    }
-    ms_bar_wait(bar, (cur.phase >> 1) & 1u);
-    cur.phase ^= 2u;
-    cur.ga = cur.ka; cur.gb = cur.kb; cur.gz = cur.kz;
-}
-#else
-inline void ms_cache_cell(const Grid3D&, Cur3&, const unsigned (&)[4], const unsigned (&)[4]) {}
-inline void ms_cache_ground(const Grid3D&, Cur3&, const unsigned (&)[4], const unsigned (&)[4]) {}
-#endif
-
-// ---------------------------------------------------------------------------------------------------------------
 // Eval_Spline_AllOrder1 / AllOrder2 for T, u and v in one pass.  out[field][..] in GRID-axis order:
 //   0 f, 1 d/da, 2 d/db, 3 d/dz, 4 d2/da2, 5 d2/db2, 6 d2/dz2, 7 d2/dadb, 8 d2/dadz, 9 d2/dbdz   (a = ax0, b = ax1, z = vertical)
 // ---------------------------------------------------------------------------------------------------------------
@@ -342,14 +267,7 @@ GEOAC_HD void ms_sample_tuv(const Grid3D& g, double a_in, double b_in, double z_
     ms_weights(wb, B, B.d);
     // d2f/dz2 block: the Cartesian file scales the ax1 slope data by dx (App. A-8); Global uses dp
     const double qs = GLOBAL ? 1.0 : A.d * B.inv_d;
-    unsigned kofs = (unsigned)cur.kz * MS_STRIDE;
-    const double* tuv = g.tuv;
-    if (g.cache_tuv) {                                  // cooperative kernel: read the cell's node block from the ray's shared-memory cache
-        ms_cache_cell(g, cur, A.off, B.off);
-#pragma unroll
-        for (int i = 0; i < 4; i++) { A.off[i] = (unsigned)(i * MS_CACHE_COL); B.off[i] = (unsigned)(i * 4 * MS_CACHE_COL); }
-        kofs = 0; tuv = g.cache_tuv;
-    }
+    const unsigned kofs = (unsigned)cur.kz * MS_STRIDE;
 
     const double ida = A.inv_d, idb = B.inv_d;
 #pragma unroll 1
@@ -357,7 +275,7 @@ GEOAC_HD void ms_sample_tuv(const Grid3D& g, double a_in, double b_in, double z_
         double acc[10];
 #pragma unroll
         for (int i = 0; i < 10; i++) acc[i] = 0.0;
-        const double* base = tuv + kofs + MS_FIELD * F;
+        const double* base = g.tuv + kofs + MS_FIELD * F;
         if (g.nrole == 1) {
 #pragma unroll
             for (int jb = 0; jb < 4; jb++) {
@@ -390,8 +308,7 @@ GEOAC_HD void ms_sample_tuv(const Grid3D& g, double a_in, double b_in, double z_
 // vertical derivative wrappers c_diff / u_diff / v_diff (Eval_Spline_df with the same scaling) -- used by travel time,
 // absorption, amplitude, reflection and the per-launch invariants.  vals: T, u, v, rho;  dz: dT/dz, du/dz, dv/dz.
 // ---------------------------------------------------------------------------------------------------------------
-// GROUND (Global.RngDep absorption reference, sampled at the lowest levels every step): only T and rho are evaluated, from
-// the ray's ground block when it has a cache.
+// GROUND (Global.RngDep absorption reference, sampled at the lowest levels every step): only T and rho are evaluated.
 template <bool GLOBAL, bool WITH_RHO, bool WITH_DZ, bool GROUND = false>
 GEOAC_HD void ms_wrappers(const Grid3D& g, double a_in, double b_in, double z_in, Cur3& cur, double (&vals)[4], double (&dz)[3]) {
     const double a = clampd(a_in, g.amin, g.amax), b = clampd(b_in, g.bmin, g.bmax), z = clampd(z_in, g.zmin, g.zmax);
@@ -405,24 +322,14 @@ GEOAC_HD void ms_wrappers(const Grid3D& g, double a_in, double b_in, double z_in
     MsW wa, wb;
     ms_weights(wa, A, A.d);
     ms_weights(wb, B, GLOBAL ? B.d : A.d);              // the quirk: ax1 slope data times dx
-    unsigned kofs = (unsigned)cur.kz * MS_STRIDE;
-    const double* tuv = g.tuv; const double* rhop = g.rho;
-    bool gnd_cached = false;
-    if (g.cache_tuv) {
-        if (GROUND) ms_cache_ground(g, cur, A.off, B.off); else ms_cache_cell(g, cur, A.off, B.off);
-#pragma unroll
-        for (int i = 0; i < 4; i++) { A.off[i] = (unsigned)(i * MS_CACHE_COL); B.off[i] = (unsigned)(i * 4 * MS_CACHE_COL); }
-        kofs = 0; tuv = g.cache_tuv; rhop = g.cache_rho; gnd_cached = GROUND;
-    }
     vals[1] = vals[2] = 0.0;
 #pragma unroll 1
     for (int F = 0; F < (WITH_RHO ? 4 : 3); F += (GROUND ? 3 : 1)) {
         const bool is_rho = (F == 3);
-        const bool two = is_rho || gnd_cached;          // 2-double records: rho, and both fields of the ground block
-        const double* base = gnd_cached ? g.cache_gnd + (is_rho ? 64 : 0) : (is_rho ? rhop : tuv + MS_FIELD * F);
-        const int lvl = two ? 2 : MS_STRIDE;             // doubles between vertical levels
-        const unsigned ko = gnd_cached ? 0u : (is_rho ? (g.cache_tuv ? 0u : (unsigned)cur.kz * 2u) : kofs);
-        const unsigned shr = two ? (unsigned)(MS_STRIDE / 2) : 1u;   // node offsets were built for the tuv layout: /9 for the 2-double one
+        const double* base = is_rho ? g.rho : g.tuv + MS_FIELD * F;
+        const int lvl = is_rho ? 2 : MS_STRIDE;          // doubles between vertical levels
+        const unsigned ko = (unsigned)cur.kz * (is_rho ? 2u : (unsigned)MS_STRIDE);
+        const unsigned shr = is_rho ? (unsigned)(MS_STRIDE / 2) : 1u;   // node offsets were built for the tuv layout: /9 for rho's 2 doubles
         double av[2] = { 0.0, 0.0 };               // value, d/dz
         const double bscale = GLOBAL ? 1.0 : B.d * A.inv_d;
         auto row = [&](int jb, unsigned boff) {

@@ -44,16 +44,15 @@ struct TraceArgs {
     int64_t n_claims;                 // entries of `order` (a multiple of 32 in packet mode), or n_rays
     // packet mode (range-dependent sets): the first n_long_packets packets of `order` are the LONG region -- packets whose
     // predicted cost exceeds the average work of a lane, i.e. which would outlast the pass on a fully loaded SM.  They are
-    // claimed by the CTAs of a second, concurrent launch that keeps its SMs to itself (one warp per scheduler: see capi.cu),
-    // `long_width` rays at a time (32 = whole packets, 8 = quarter packets traced four lanes per ray from the start).
+    // claimed by the CTAs of a second, concurrent launch that keeps its SMs to itself (one warp per scheduler: see capi.cu).
     int64_t n_long_packets;
     int64_t n_quarter_packets;        // the first of them -- the very longest -- are claimed eight rays at a time and traced four lanes per
                                       // ray from the start: a warp with 8 rays keeps their cells in L1 and needs ~0.6x the instructions per step
     unsigned long long* counter_quarter;
     unsigned long long* counter_long; // next unclaimed entry of the long region
     int prefer_long;                  // this launch claims the long region first (1) or the main region first (0)
-    int long_width;
-    int packet_refill;                // experiment knob: refill a warp only when all of its lanes are idle (always on for PacketMode sets)
+    int packet_refill;                // stratified sets: refill a warp only when all of its lanes are idle (set with the sorted claim order;
+                                      // the PacketMode sets always refill this way)
     double* path; int32_t* path_rows; int path_stride; int64_t path_cap;   // raypath capture (PATHS kernels), else unused
     double* caus; int32_t* caus_rows; int64_t caus_cap;                    // caustic events (PATHS kernels), else unused
     double* prev;                     // y_{k-1} scratch: [NEQ][grid * block] doubles (variants with a quadratic intercept)
@@ -395,8 +394,8 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
                             }
                         } else if (region == 1) {
                             if (nl > nq && !(region_done & 1u)) {
-                                const unsigned long long q = atomicAdd(a.counter_long, (unsigned long long)a.long_width);
-                                if (nq + q < nl) { base = nq + q; width = a.long_width; } else region_done |= 1u;
+                                const unsigned long long q = atomicAdd(a.counter_long, 32ull);
+                                if (nq + q < nl) { base = nq + q; width = 32; } else region_done |= 1u;
                             }
                         } else if (nm && !(region_done & 2u)) {
                             const unsigned long long q = atomicAdd(a.counter, 32ull);
@@ -487,130 +486,6 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Cooperative kernel of the range-dependent sets: FOUR LANES PER RAY, eight rays per warp, the ray's cell in shared memory.
-//
-// Why: in the one-thread-per-ray kernel a warp whose 32 rays sit in 32 different grid cells streams 32 x 4.6 KB of node data
-// through L1 for every sample, five samples per step; long rays decorrelate (config 5: 2.5 % of the rays travel 20 000 km and
-// take 25 % of the steps), L1 thrashes, every dependent load round waits for L2, and a step costs ~100 us however empty the SM
-// is -- so the pass cannot be shorter than (longest ray) x 100 us, which is what capped the 8-GPU scaling of config 5.
-// Here a ray's 4 x 4 x 2 node block (5 KB) is staged into shared memory by TMA bulk copies when the ray enters a cell and every
-// sample of the >= 50 that follow reads it from there (mspline.cuh: ms_cache_cell); 32 rays per SM is what shared memory holds,
-// so four lanes share a ray: lane r evaluates row r of the node block, the row contributions are accumulated lane after lane in
-// the serial order, everything else is executed redundantly -- the arithmetic, hence every record bit, is that of the
-// one-thread-per-ray kernel.  Slots refill one by one (a cell cache makes packets pointless), so no lane waits for a straggler.
-// Used for the LONG region of the claim order (capi.cu), on SMs of its own.
-// ---------------------------------------------------------------------------------------------------------------
-constexpr int kCoopBlock = 128;                       // 4 warps x 8 rays
-constexpr int kCoopSlots = kCoopBlock / 4;
-template <class EQ> struct CoopLayout {
-    static constexpr int REC = LaneLayout<EQ>::STRIDE;                                     // doubles per ray record (incl. work + sampler scratch)
-    static constexpr size_t bytes() {
-        return ((sizeof(LaunchConsts) + 15) / 16) * 16 + sizeof(double) * (size_t)kCoopSlots * (REC + 1 + MS_CACHE_TUV + MS_CACHE_RHO + MS_CACHE_GND)
-               + sizeof(uint64_t) * 2 * kCoopSlots + 64;
-    }
-};
-
-template <class EQ>
-__global__ void __launch_bounds__(kCoopBlock, 1) trace_coop_kernel(const __grid_constant__ TraceArgs a) {
-    constexpr int NEQ = EQ::NEQ;
-    static_assert(PacketMode<EQ>::value, "cooperative kernel: range-dependent sets only");
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    LaunchConsts* Ls = reinterpret_cast<LaunchConsts*>(smem_raw);
-    double* base = reinterpret_cast<double*>(smem_raw + ((sizeof(LaunchConsts) + 15) / 16) * 16);
-    double* c_tuv = base;                                                    // 16-byte aligned blocks first (TMA destinations)
-    double* c_rho = c_tuv + (size_t)kCoopSlots * MS_CACHE_TUV;
-    double* c_gnd = c_rho + (size_t)kCoopSlots * MS_CACHE_RHO;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(c_gnd + (size_t)kCoopSlots * MS_CACHE_GND);
-    double* recs = reinterpret_cast<double*>(bars + 2 * kCoopSlots);
-    for (int i = threadIdx.x; i < (int)(sizeof(LaunchConsts) / 8); i += kCoopBlock)
-        reinterpret_cast<double*>(Ls)[i] = reinterpret_cast<const double*>(a.consts)[i];
-    const unsigned lane = threadIdx.x & 31;
-    const int slot = (int)(threadIdx.x >> 2), role = (int)lane & 3;
-    if (role == 0) {
-        const uint32_t b0 = smem_u32(bars + 2 * slot);
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(b0));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(b0 + 8));
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncthreads();
-    const LaunchConsts& L = *Ls;
-    double* const rec = recs + (size_t)slot * (CoopLayout<EQ>::REC | 1);
-    double* const work = rec + LaneLayout<EQ>::WORK;
-    typename EQ::Atmo T = a.grid;
-    T.scratch = work + 2 * NEQ;
-    T.role = role; T.nrole = 4; T.glane0 = (int)lane & ~3; T.gmask = 0xFu << ((int)lane & ~3);
-    T.cache_tuv = c_tuv + (size_t)slot * MS_CACHE_TUV; T.cache_rho = c_rho + (size_t)slot * MS_CACHE_RHO;
-    T.cache_gnd = c_gnd + (size_t)slot * MS_CACHE_GND; T.cache_bar = bars + 2 * slot;
-    RecOut o; o.rec = a.rec; o.status = a.status; o.n_steps = a.n_steps; o.n_rec = a.n_rec; o.n_slots = a.n_rays * a.n_rec;
-    o.path = nullptr; o.path_rows = nullptr; o.path_stride = 0; o.path_cap = 0; o.caus = nullptr; o.caus_rows = nullptr; o.caus_cap = 0;
-    LaneD<EQ>& ld = *reinterpret_cast<LaneD<EQ>*>(rec);
-    LaneI<EQ> li;                                                            // replicated in the four lanes of the group
-    unsigned cache_phase = 0;                                                // mbarrier phases outlive the rays of a slot
-    const int64_t pstride = (int64_t)gridDim.x * kCoopSlots;
-    double* prev = a.prev + ((int64_t)blockIdx.x * kCoopSlots + slot);
-    bool have_ray = false, exhausted = false;
-    unsigned region_done = 0;
-    unsigned long long my_steps = 0;
-    unsigned my_trips = 0;
-    const unsigned long long nl = (unsigned long long)a.n_long_packets * 32ull;
-    const unsigned long long nm = (unsigned long long)a.n_claims - nl;
-
-    while (true) {
-        // ---------------- refill idle slots one by one (warp-aggregated claim, long region first) ----------------
-        const unsigned wmask = __ballot_sync(0xffffffffu, role == 0 && !have_ray && !exhausted);
-        if (wmask) {
-            const int want_n = __popc(wmask);
-            unsigned long long b1 = 0, b2 = 0; int n1 = 0, n2 = 0;             // up to two runs of entries: one per region
-            if (lane == (unsigned)(__ffs(wmask) - 1)) {
-                int need = want_n;
-                for (int attempt = 0; attempt < 2 && need > 0; attempt++) {
-                    const bool from_long = (attempt == 0) == (a.prefer_long != 0);
-                    unsigned long long q = 0, lim = 0, off = 0;
-                    if (from_long) { if (!nl || (region_done & 1u)) continue; q = atomicAdd(a.counter_long, (unsigned long long)need); lim = nl; }
-                    else           { if (!nm || (region_done & 2u)) continue; q = atomicAdd(a.counter, (unsigned long long)need); lim = nm; off = nl; }
-                    const int got = (q < lim) ? (int)((lim - q < (unsigned long long)need) ? (lim - q) : (unsigned long long)need) : 0;
-                    if (got < need) region_done |= from_long ? 1u : 2u;
-                    if (got > 0) { if (n1 == 0) { b1 = off + q; n1 = got; } else { b2 = off + q; n2 = got; } need -= got; }
-                }
-            }
-            const int leader = __ffs(wmask) - 1;
-            b1 = __shfl_sync(0xffffffffu, b1, leader); b2 = __shfl_sync(0xffffffffu, b2, leader);
-            n1 = __shfl_sync(0xffffffffu, n1, leader); n2 = __shfl_sync(0xffffffffu, n2, leader);
-            const unsigned my_bit = 1u << (lane & ~3u);                         // bit of this group's role-0 lane
-            const bool wants = (wmask & my_bit) != 0;
-            if (wants) {
-                const int rank = __popc(wmask & (my_bit - 1u));
-                long long idx = -1;
-                if (rank < n1) idx = (long long)b1 + rank; else if (rank < n1 + n2) idx = (long long)b2 + (rank - n1);
-                if (idx < 0) exhausted = true;
-                else {
-                    const int64_t r = a.order ? (int64_t)a.order[idx] : idx;
-                    if (r < a.n_rays) {
-                        lane_start<EQ>(ld, li, L, T, r, a.theta[r], a.phi[r]);
-                        li.cur.phase = cache_phase;                             // the slot's mbarriers keep their phase across rays
-                        have_ray = true;
-                    }
-                }
-            }
-        }
-        if (!__any_sync(0xffffffffu, have_ray)) {
-            if (__all_sync(0xffffffffu, exhausted)) break;
-            continue;
-        }
-        my_trips++;
-        if (have_ray) {
-            __syncwarp(T.gmask);
-            have_ray = lane_advance<EQ, false>(ld, li, L, T, prev, pstride, o, work);
-            cache_phase = li.cur.phase;
-            if (role == 0) my_steps++;
-        }
-    }
-    for (int off = 16; off > 0; off >>= 1) my_steps += __shfl_xor_sync(0xffffffffu, my_steps, off);
-    // lane occupancy is reported in units of 32-lane trips: a cooperative trip advances 8 rays with 32 lanes
-    if (lane == 0 && my_steps) { atomicAdd(a.total_steps, my_steps); atomicAdd(a.warp_trips, (unsigned long long)my_trips / 4ull); }
-}
-
-// ---------------------------------------------------------------------------------------------------------------
 // Longest-ray-first scheduling.  Ray lifetimes differ by an order of magnitude and a lane processes only a few rays,
 // so with the natural claim order ~30 % of the lane-steps of a 2e5-ray batch idle in the tail while the last long
 // rays finish.  A SCOUT pass predicts each ray's RK4 step count by tracing it with the amplitude-free equation set
@@ -629,8 +504,7 @@ template <class EQ> struct ScoutBlock { static constexpr int value = std::is_sam
 // in registers.
 template <class EQ, bool TABLE_IN_SMEM>
 __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const __grid_constant__ TraceArgs a, uint32_t* cost, uint32_t* cost_max,
-                                                               unsigned long long* cost_sum, unsigned long long* counter, int coarse, int stride,
-                                                               const uint32_t* list, const unsigned long long* n_list) {
+                                                               unsigned long long* cost_sum, unsigned long long* counter, int coarse) {
     constexpr int NEQ = EQ::NEQ;
     constexpr bool kGrid = std::is_same<typename EQ::Atmo, Grid3D>::value;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -662,11 +536,7 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
             if ((int)lane == leader) base = atomicAdd(counter, (unsigned long long)__popc(wmask));
             base = __shfl_sync(0xffffffffu, base, leader);
             if (want) {
-                // every `stride`-th ray is scouted; its neighbours in the batch (neighbouring launch angles) inherit the estimate --
-                // the cost only orders the claims, and it varies smoothly along the launch grid
-                // (refinement pass: the rays named in `list` -- the ones the first pass found long -- are scouted again at a finer step)
-                const int64_t item = (int64_t)(base + __popc(wmask & ((1u << lane) - 1u)));
-                ray = list ? ((unsigned long long)item < *n_list ? (int64_t)list[item] : a.n_rays) : item * stride;
+                ray = (int64_t)(base + __popc(wmask & ((1u << lane) - 1u)));
                 if (ray < a.n_rays) {
                     cur = typename EQ::Cursor{};
                     EQ::init(L, T, a.theta[ray], a.phi[ray], rc, y, cur);
@@ -702,8 +572,7 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
             }
         }
         if (done) {
-            if (list) { total += (unsigned long long)est - (unsigned long long)cost[ray]; cost[ray] = est; }      // replaces the first estimate (the sum wraps correctly)
-            else for (int j = 0; j < stride && ray + j < a.n_rays; j++) { cost[ray + j] = est; total += est; }
+            cost[ray] = est; total += est;
             worst = max(worst, est); have_ray = false;
         }
         else {
@@ -731,16 +600,6 @@ __global__ void cost_dilate_kernel(const uint32_t* cost, const double* theta, in
         }
         out[i] = c;
     }
-}
-
-// rays whose first estimate exceeds alpha % of the average lane work: candidates for the long region, scouted again at a finer step
-// (they are a few per cent of the rays; a long packet that the coarse scout underestimates is traced as a whole packet instead of
-// four quarters and then sets the length of the pass -- measured: one rank in eight, 27 s instead of 22.5 s)
-__global__ void refine_select_kernel(const uint32_t* cost, int64_t n, const unsigned long long* cost_sum, long long lanes, int alpha_pct,
-                                     uint32_t* list, unsigned long long* n_list) {
-    const unsigned long long thr = (*cost_sum / (unsigned long long)lanes) * (unsigned long long)alpha_pct / 100ull;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        if ((unsigned long long)cost[i] > thr) list[atomicAdd(n_list, 1ull)] = (uint32_t)i;
 }
 
 // counting sort by predicted cost, descending: hist[b] of bucket(cost) -> start offsets -> scatter.  The sorted items are
@@ -883,61 +742,6 @@ __global__ void stable_scatter_kernel(const uint8_t* key, const uint32_t* src, i
         }
         __syncwarp();
     }
-}
-
-// ---- range-dependent sets: which rays share a packet ----
-// A warp's 32 rays should walk through the same grid cells (their node data then come out of L1 as a few shared lines instead
-// of 32 private blocks).  The mains enumerate the launch grid azimuth by azimuth, inclination fastest, so 32 consecutive rays
-// are neighbours in INCLINATION: they stay in one vertical plane and spread over altitude ~ s * 32 dtheta.  32 rays of EQUAL
-// inclination and neighbouring AZIMUTH share their altitude history and spread sideways ~ s * 32 dphi.  Measured in cells
-// (vertical spacing dz, horizontal spacing dh) the second grouping is the tighter one iff dphi / dh < dtheta / dz -- config 5
-// (0.36 deg steps on a 1 deg = 111 km grid), not config 4 (3.6 deg steps on a 5 km grid).  grid_shape_kernel reads the two steps
-// off the batch: shape[0] = dtheta between the first two rays, shape[1] = dphi between the first two azimuth rows (0 if the batch
-// is not such a grid), shape[2] = rays per azimuth row.
-__global__ void grid_shape_kernel(const double* theta, const double* phi, int64_t n, double* shape) {
-    __shared__ int first_wrap;
-    if (threadIdx.x == 0) first_wrap = 0x7fffffff;
-    __syncthreads();
-    const int64_t lim = n < 65536 ? n : 65536;
-    for (int64_t i = 1 + threadIdx.x; i < lim; i += blockDim.x)
-        if (theta[i] < theta[i - 1]) atomicMin(&first_wrap, (int)i);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const int w = first_wrap;
-        shape[0] = (n > 1) ? fabs(theta[1] - theta[0]) : 0.0;
-        shape[1] = (w != 0x7fffffff && w < n) ? fabs(phi[w] - phi[0]) : 0.0;
-        shape[2] = (w != 0x7fffffff) ? (double)w : (double)n;
-    }
-}
-// 16-bit inclination key (two stable 8-bit passes) + cost bucket: order = (cost bucket descending, inclination, batch index)
-__global__ void order_keys16_kernel(const uint32_t* cost, const double* theta, int64_t n, const uint32_t* cost_max, const double* range,
-                                    uint8_t* key_lo, uint8_t* key_hi, uint8_t* key_cost, int cost_shift) {
-    const uint32_t cmax = *cost_max;
-    const double t0 = range[0], span = range[1] - range[0];
-    const double sc = span > 0.0 ? 65535.0 / span : 0.0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        int kt = (int)((theta[i] - t0) * sc + 0.5);
-        kt = kt < 0 ? 0 : (kt > 65535 ? 65535 : kt);
-        key_lo[i] = (uint8_t)(kt & 255); key_hi[i] = (uint8_t)(kt >> 8);
-        key_cost[i] = (uint8_t)(cost_bucket(cost[i], cmax) >> cost_shift);
-    }
-}
-// packets of the final order whose longest ray exceeds the average work of a lane (times alpha_pct / 100): the long region.
-// The order is sorted by cost bucket, so they sit at its head; the count is all the launch needs.
-__global__ void packet_long_kernel(const uint32_t* order, const uint32_t* cost, int64_t n_packets, int64_t n_rays,
-                                   const unsigned long long* cost_sum, long long lanes, int alpha_pct, uint32_t* n_long, uint32_t* n_quarter, int alpha2_pct) {
-    const unsigned long long avg = *cost_sum / (unsigned long long)lanes;
-    const unsigned long long thr = avg * (unsigned long long)alpha_pct / 100ull, thr2 = avg * (unsigned long long)alpha2_pct / 100ull;
-    uint32_t cnt = 0, cnt2 = 0;
-    for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n_packets; g += (int64_t)gridDim.x * blockDim.x) {
-        uint32_t c = 0;
-        for (int l = 0; l < 32; l++) { const uint32_t r = order[g * 32 + l]; if (r < n_rays) c = max(c, cost[r]); }
-        if ((unsigned long long)c > thr) cnt++;
-        if ((unsigned long long)c > thr2) cnt2++;
-    }
-    cnt = __reduce_add_sync(0xffffffffu, cnt); cnt2 = __reduce_add_sync(0xffffffffu, cnt2);
-    if ((threadIdx.x & 31) == 0 && cnt) atomicAdd(n_long, cnt);
-    if ((threadIdx.x & 31) == 0 && cnt2) atomicAdd(n_quarter, cnt2);
 }
 
 #endif  // __CUDACC__

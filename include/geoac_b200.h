@@ -289,13 +289,13 @@ int geoac_eq_count(int variant, int calc_amp);
 /* Scheduling counters of the last trace.  warp_trips: trips round the kernel's step loop summed over warps -- lane
  * occupancy = total_steps / (32 * warp_trips), i.e. how full the warps were on average (ray lifetimes differ; finished
  * lanes are refilled until the batch is exhausted).  kernel_launches: kernels the call enqueued (1 trace kernel; plus, when the
- * longest-ray-first claim order was built, the cost scout and the counting sort: 3 kernels for the range-dependent sets,
- * 8 for the stratified ones, whose order is (cost, inclination, batch index) in two stable passes).  Either pointer may be NULL. */
+ * longest-ray-first claim order was built, the cost scout and the sort: for the range-dependent sets the cost dilation (unless
+ * knob "dilate" is 0), 3 counting-sort kernels and, with a long region of its own, a second trace launch; for the stratified sets
+ * 8 kernels, whose order is (cost, inclination, batch index) in two stable passes).  Either pointer may be NULL. */
 int geoac_last_trace_counters(geoac_ctx* ctx, int64_t* warp_trips, int64_t* kernel_launches);
 
-/* Scheduling facts of the last trace on ctx (8 values): [0] packet grouping of the range-dependent sets (0 = 32 consecutive rays,
- * 1 = equal inclination / neighbouring azimuth), [1] packets in the long region (predicted to outlast the pass on a loaded SM),
- * [2] CTAs of the concurrent launch that traced them on SMs of their own, [3] kernels enqueued, [4] the longest of the long packets
+/* Scheduling facts of the last trace on ctx (8 values): [0] reserved (0), [1] packets of the range-dependent sets in the long
+ * region (predicted to outlast the pass on a loaded SM), [2] CTAs of the concurrent launch that traced them on SMs of their own, [3] kernels enqueued, [4] the longest of the long packets
  * that were split over four warps (quarter claims, four lanes per ray), [5..7] reserved (0). */
 int geoac_last_schedule(geoac_ctx* ctx, int64_t* out8);
 /* Test / diagnosis hook: the RK4 step counts the cost scout PREDICTED for the rays of the last trace (n entries, batch order). */
@@ -317,8 +317,8 @@ int geoac_get_grid_tables(geoac_ctx* ctx, int64_t cap_tuv, double* tuv, int64_t 
 
 /* Tuning / experiment knobs of a context (DESIGN.md section 6).  Their defaults are read from the GEOAC_B200_* environment
  * variables ONCE, in geoac_create; nothing on the launch path reads the environment.  Names: "lpt" (claim order: 0 natural,
- * 1 automatic, 2 always), "packet", "scout_coarse", "stable", "cost_shift", "coop", "sbpoly", "block3d", "host_tables",
- * "rd_group", "long_alpha", "long_width", "long_sm_pct", "exclusive", "rd_ctas", "scout_stride", "quarter", "quarter_alpha", "refine", "dilate".
+ * 1 automatic, 2 always), "scout_coarse", "cost_shift", "coop", "sbpoly", "host_tables", "long_alpha", "long_sm_pct", "exclusive",
+ * "quarter", "quarter_alpha", "dilate"; any other name is GEOAC_ERR_BAD_ARG.
  * No knob changes a record bit except "sbpoly" (absorption sum to 1e-11) -- that is what the tests use them to prove. */
 int geoac_set_knob(geoac_ctx* ctx, const char* name, int value);
 

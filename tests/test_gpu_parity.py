@@ -147,7 +147,7 @@ def test_longest_ray_first_schedule_is_result_neutral(monkeypatch):
             tr = _tracer_for(variant, kv, d)
             tr.set_knob("lpt", int(mode))
             outs.append(tr.trace(th, ph))
-            n_k = tr.last_kernel_launches()          # scout + sort kernels (+ grid-shape probe, + long-region launch) + trace kernel
+            n_k = tr.last_kernel_launches()          # scout (+ cost dilation) + sort kernels (+ long-region launch) + trace kernel
             assert n_k == 1 if mode == "0" else (n_k >= 5 if util.is_rngdep(variant) else n_k == 10)
         assert np.array_equal(outs[0]["status"], outs[1]["status"]) and np.array_equal(outs[0]["n_steps"], outs[1]["n_steps"])
         assert np.array_equal(outs[0]["rec"], outs[1]["rec"])
