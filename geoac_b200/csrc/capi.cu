@@ -15,6 +15,7 @@
 #include <thread>
 #include <atomic>
 #include <limits>
+#include <utility>
 
 #include "core.cuh"
 #include "eq_cartesian.cuh"
@@ -68,6 +69,30 @@ static Knobs knobs_from_env() {
     return k;
 }
 
+// One device allocation (PINNED: page-locked host memory) and its capacity in bytes, freed with its owner.  grow() keeps the
+// allocation when it holds `need` bytes and otherwise frees it and allocates anew: the contents are not kept.
+template <class T, bool PINNED = false>
+struct Buf {
+    T* p = nullptr;
+    size_t cap = 0;
+    Buf() = default;
+    Buf(Buf&& o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    Buf& operator=(Buf&& o) noexcept { if (this != &o) { release(); p = std::exchange(o.p, nullptr); cap = std::exchange(o.cap, 0); } return *this; }
+    ~Buf() { release(); }
+    void release() {
+        if (PINNED) cudaFreeHost(p); else cudaFree(p);
+        p = nullptr; cap = 0;
+    }
+    cudaError_t grow(size_t need) {
+        if (need <= cap) return cudaSuccess;
+        release();
+        void* q = nullptr;
+        const cudaError_t e = PINNED ? cudaHostAlloc(&q, need, cudaHostAllocDefault) : cudaMalloc(&q, need);
+        if (e == cudaSuccess) { p = static_cast<T*>(q); cap = need; }
+        return e;
+    }
+};
+
 struct geoac_ctx {
     int variant = 0, device = 0, sm_count = 0;
     Knobs knobs;
@@ -78,26 +103,24 @@ struct geoac_ctx {
     int n = 0;
     double xmin = 0, xmax = 0;
     std::vector<double> h_table;
-    double* d_table = nullptr;
-    double* d_sbpoly = nullptr;      // per-interval absorption polynomials of the 1-D table (core.cuh), rebuilt with the invariants
+    Buf<double> d_table;
+    Buf<double> d_sbpoly;            // per-interval absorption polynomials of the 1-D table (core.cuh), rebuilt with the invariants
     // range-dependent grid
     bool is_grid = false;
     Grid3D grid{};
-    double *d_tuv = nullptr, *d_rho = nullptr, *d_ax = nullptr;
-    LaunchConsts* d_consts = nullptr;
-    unsigned long long* d_counters = nullptr;     // [0] ray counter, [1] total steps
-    double* d_prev = nullptr; size_t cap_prev = 0; // y_{k-1} scratch of the trace kernel
-    double* d_path = nullptr; size_t cap_path = 0; int32_t* d_path_rows = nullptr; size_t cap_path_rows = 0;   // raypath capture staging
-    double* d_caus = nullptr; size_t cap_caus = 0; int32_t* d_caus_rows = nullptr; size_t cap_caus_rows = 0;   // caustic event staging
-    // longest-ray-first scheduling: predicted costs, the costs the order uses (dilated), claim order, sort scratch; capacities in bytes
-    uint32_t *d_cost = nullptr, *d_cost_dilated = nullptr, *d_order = nullptr, *d_order2 = nullptr, *d_hist = nullptr, *d_blockhist = nullptr;
-    uint8_t* d_keys = nullptr;
-    size_t cap_cost = 0, cap_cost_dilated = 0, cap_order = 0, cap_order2 = 0, cap_hist = 0, cap_blockhist = 0, cap_keys = 0;
+    Buf<double> d_tuv, d_rho, d_ax;
+    Buf<LaunchConsts> d_consts;
+    Buf<unsigned long long> d_counters;           // [0] ray counter, [1] total steps
+    Buf<double> d_prev;                           // y_{k-1} scratch of the trace kernel
+    Buf<double> d_path; Buf<int32_t> d_path_rows; // raypath capture staging
+    Buf<double> d_caus; Buf<int32_t> d_caus_rows; // caustic event staging
+    // longest-ray-first scheduling: predicted costs, the costs the order uses (dilated), claim order, sort scratch
+    Buf<uint32_t> d_cost, d_cost_dilated, d_order, d_order2, d_hist, d_blockhist;
+    Buf<uint8_t> d_keys;
     int last_launches = 0;
     // staging for the host-buffer entry point
-    double *d_theta = nullptr, *d_phi = nullptr, *d_rec = nullptr;
-    int32_t *d_status = nullptr, *d_nsteps = nullptr;
-    size_t cap_theta = 0, cap_phi = 0, cap_rec = 0, cap_status = 0, cap_nsteps = 0;
+    Buf<double> d_theta, d_phi, d_rec;
+    Buf<int32_t> d_status, d_nsteps;
     cudaStream_t stream = nullptr, stream_long = nullptr;      // stream_long: the concurrent long-region launch of the range-dependent sets
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_fork = nullptr, ev_join = nullptr, ev_m0 = nullptr, ev_m1 = nullptr, ev_l0 = nullptr, ev_l1 = nullptr;
     bool timed_launches = false;
@@ -106,7 +129,8 @@ struct geoac_ctx {
     bool consts_dirty = true;
     bool src_set = false;
     // pinned host staging of geoac_trace_multi (this context's share of the batch: angles in, records out)
-    struct Pin { void* p = nullptr; size_t cap = 0; } pin_theta, pin_phi, pin_rec, pin_status, pin_nsteps;
+    Buf<double, true> pin_theta, pin_phi, pin_rec;
+    Buf<int32_t, true> pin_status, pin_nsteps;
 };
 
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
@@ -158,8 +182,8 @@ extern "C" geoac_ctx* geoac_create(int variant, int device, int* status) {
            && cudaEventCreate(&ctx->ev0) == cudaSuccess && cudaEventCreate(&ctx->ev1) == cudaSuccess
            && cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming) == cudaSuccess
            && cudaEventCreate(&ctx->ev_m0) == cudaSuccess && cudaEventCreate(&ctx->ev_m1) == cudaSuccess && cudaEventCreate(&ctx->ev_l0) == cudaSuccess && cudaEventCreate(&ctx->ev_l1) == cudaSuccess
-           && cudaMalloc(&ctx->d_consts, sizeof(LaunchConsts)) == cudaSuccess
-           && cudaMalloc(&ctx->d_counters, 8 * sizeof(unsigned long long)) == cudaSuccess;
+           && ctx->d_consts.grow(sizeof(LaunchConsts)) == cudaSuccess
+           && ctx->d_counters.grow(8 * sizeof(unsigned long long)) == cudaSuccess;
     if (!ok) { std::string m = cudaGetErrorString(cudaGetLastError()); delete ctx; return bail(GEOAC_ERR_CUDA, "context allocation failed: " + m); }
     if (status) *status = GEOAC_OK;
     return ctx;
@@ -167,12 +191,7 @@ extern "C" geoac_ctx* geoac_create(int variant, int device, int* status) {
 
 extern "C" void geoac_destroy(geoac_ctx* ctx) {
     if (!ctx) return;
-    cudaSetDevice(ctx->device);
-    cudaFree(ctx->d_table); cudaFree(ctx->d_sbpoly); cudaFree(ctx->d_consts); cudaFree(ctx->d_counters); cudaFree(ctx->d_prev);
-    cudaFree(ctx->d_cost_dilated); cudaFree(ctx->d_cost); cudaFree(ctx->d_order); cudaFree(ctx->d_hist); cudaFree(ctx->d_blockhist); cudaFree(ctx->d_order2); cudaFree(ctx->d_keys); cudaFree(ctx->d_path); cudaFree(ctx->d_path_rows); cudaFree(ctx->d_caus); cudaFree(ctx->d_caus_rows);
-    cudaFree(ctx->d_tuv); cudaFree(ctx->d_rho); cudaFree(ctx->d_ax);
-    cudaFree(ctx->d_theta); cudaFree(ctx->d_phi); cudaFree(ctx->d_rec); cudaFree(ctx->d_status); cudaFree(ctx->d_nsteps);
-    cudaFreeHost(ctx->pin_theta.p); cudaFreeHost(ctx->pin_phi.p); cudaFreeHost(ctx->pin_rec.p); cudaFreeHost(ctx->pin_status.p); cudaFreeHost(ctx->pin_nsteps.p);
+    cudaSetDevice(ctx->device);                       // the buffers are freed with the context, on its device
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->ev_m0) cudaEventDestroy(ctx->ev_m0);
@@ -251,17 +270,13 @@ extern "C" int geoac_set_atmosphere_1d(geoac_ctx* ctx, int n, const double* z, c
     }
     // build into fresh buffers and swap them in only after every step succeeded: a failed call leaves the previous
     // atmosphere (or "none") fully intact instead of dangling pointers
-    double *nt = nullptr, *ns = nullptr;
-    if (cudaMalloc(&ns, (size_t)(n - 1) * SBP_STRIDE * sizeof(double)) != cudaSuccess
-        || cudaMalloc(&nt, ctx->h_table.size() * sizeof(double)) != cudaSuccess
-        || cudaMemcpy(nt, tb, ctx->h_table.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) {
-        const std::string m = cudaGetErrorString(cudaGetLastError());
-        cudaFree(nt); cudaFree(ns);
-        return fail(ctx, GEOAC_ERR_CUDA, "geoac_set_atmosphere_1d: " + m);
-    }
+    Buf<double> nt, ns;
+    if (ns.grow((size_t)(n - 1) * SBP_STRIDE * sizeof(double)) != cudaSuccess
+        || nt.grow(ctx->h_table.size() * sizeof(double)) != cudaSuccess
+        || cudaMemcpy(nt.p, tb, ctx->h_table.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess)
+        return fail(ctx, GEOAC_ERR_CUDA, std::string("geoac_set_atmosphere_1d: ") + cudaGetErrorString(cudaGetLastError()));
     cudaStreamSynchronize(ctx->stream);                                          // no launch may still read the old tables
-    cudaFree(ctx->d_table); cudaFree(ctx->d_sbpoly);
-    ctx->d_table = nt; ctx->d_sbpoly = ns;
+    ctx->d_table = std::move(nt); ctx->d_sbpoly = std::move(ns);
     ctx->n = n; ctx->xmin = x[0]; ctx->xmax = x[n - 1];
     // GeoAc_SetPropRegion: G2S_Spline1D.cpp:22-28 / G2S_GlobalSpline1D.cpp:22-30
     ctx->prm.vert_limit = ctx->xmax;
@@ -363,27 +378,27 @@ extern "C" int geoac_set_atmosphere_3d(geoac_ctx* ctx, int n0, int n1, int nz, c
     for (int k = 0; k < nz; k++) z[k] = axz[k] + (glob ? kREarth : 0.0);                     // r_vals[nr] += r_earth
     // build into fresh buffers and swap them in only after every step succeeded (a failed call -- e.g. out of memory on a
     // config-5-size grid -- leaves the previous atmosphere, or "none", fully intact)
-    double *n_tuv = nullptr, *n_rho = nullptr, *n_ax = nullptr, *d_f = nullptr, *d_aux = nullptr;
+    Buf<double> n_tuv, n_rho, n_ax;
     auto bail = [&](const std::string& what) {
-        const std::string m = cudaGetErrorString(cudaGetLastError());
-        cudaFree(n_tuv); cudaFree(n_rho); cudaFree(n_ax); cudaFree(d_f); cudaFree(d_aux);
-        return fail(ctx, GEOAC_ERR_CUDA, "geoac_set_atmosphere_3d: " + what + ": " + m);
+        return fail(ctx, GEOAC_ERR_CUDA, "geoac_set_atmosphere_3d: " + what + ": " + cudaGetErrorString(cudaGetLastError()));
     };
-    if (cudaMalloc(&n_tuv, nodes * MS_STRIDE * sizeof(double)) != cudaSuccess) return bail("node tables");
-    if (cudaMalloc(&n_rho, nodes * 2 * sizeof(double)) != cudaSuccess) return bail("density table");
+    if (n_tuv.grow(nodes * MS_STRIDE * sizeof(double)) != cudaSuccess) return bail("node tables");
+    if (n_rho.grow(nodes * 2 * sizeof(double)) != cudaSuccess) return bail("density table");
     std::vector<double> r0, r1, rz;
     build_axis_records(ax0, n0, r0); build_axis_records(ax1, n1, r1); build_axis_records(z.data(), nz, rz);
-    if (cudaMalloc(&n_ax, (size_t)(n0 + n1 + nz) * AX * sizeof(double)) != cudaSuccess) return bail("axis records");
+    if (n_ax.grow((size_t)(n0 + n1 + nz) * AX * sizeof(double)) != cudaSuccess) return bail("axis records");
     if (ctx->knobs.host_tables) {                                          // tests: build the tables on the host instead
         std::vector<double> zz, tuv, rh;
         build_grid_tables(glob, n0, n1, nz, ax0, ax1, axz, T, u, v, rho, zz, tuv, rh);
-        if (cudaMemcpy(n_tuv, tuv.data(), tuv.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess
-            || cudaMemcpy(n_rho, rh.data(), rh.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) return bail("table upload");
+        if (cudaMemcpy(n_tuv.p, tuv.data(), tuv.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess
+            || cudaMemcpy(n_rho.p, rh.data(), rh.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) return bail("table upload");
     } else {
         // raw fields + axis-only coefficients up, slopes and node differences built in HBM
         std::vector<double> aux; build_zaux(z, aux);
-        if (cudaMalloc(&d_f, nodes * 4 * sizeof(double)) != cudaSuccess) return bail("raw fields");
-        if (cudaMalloc(&d_aux, (aux.size() + n0 + n1) * sizeof(double)) != cudaSuccess) return bail("axis coefficients");
+        Buf<double> f_buf, aux_buf;                                        // freed once the tables are built
+        if (f_buf.grow(nodes * 4 * sizeof(double)) != cudaSuccess) return bail("raw fields");
+        if (aux_buf.grow((aux.size() + n0 + n1) * sizeof(double)) != cudaSuccess) return bail("axis coefficients");
+        double *d_f = f_buf.p, *d_aux = aux_buf.p;
         const double* src[4] = { T, u, v, rho };
         cudaError_t e = cudaSuccess;
         for (int F = 0; F < 4 && e == cudaSuccess; F++) e = cudaMemcpy(d_f + (size_t)F * nodes, src[F], nodes * sizeof(double), cudaMemcpyHostToDevice);
@@ -394,21 +409,19 @@ extern "C" int geoac_set_atmosphere_3d(geoac_ctx* ctx, int n0, int n1, int nz, c
             ZAux za; za.A = d_aux; za.DEN = d_aux + nz; za.NC = d_aux + 2 * (size_t)nz; za.P2LO = d_aux + 3 * (size_t)nz; za.P2HI = d_aux + 4 * (size_t)nz;
             const long long nthreads = (long long)n0 * n1 * 10;
             grid_tables_kernel<<<(unsigned)((nthreads + 127) / 128), 128, 0, ctx->stream>>>(glob ? 1 : 0, n0, n1, nz, d_aux + aux.size(), d_aux + aux.size() + n0, za,
-                                                                                           d_f, d_f + nodes, d_f + 2 * nodes, d_f + 3 * nodes, n_tuv, n_rho);
+                                                                                           d_f, d_f + nodes, d_f + 2 * nodes, d_f + 3 * nodes, n_tuv.p, n_rho.p);
             e = cudaGetLastError();
             if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
         }
         if (e != cudaSuccess) return bail("table build");
-        cudaFree(d_f); cudaFree(d_aux); d_f = d_aux = nullptr;
     }
-    if (cudaMemcpy(n_ax, r0.data(), r0.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess
-        || cudaMemcpy(n_ax + (size_t)n0 * AX, r1.data(), r1.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess
-        || cudaMemcpy(n_ax + (size_t)(n0 + n1) * AX, rz.data(), rz.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) return bail("axis upload");
+    if (cudaMemcpy(n_ax.p, r0.data(), r0.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess
+        || cudaMemcpy(n_ax.p + (size_t)n0 * AX, r1.data(), r1.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess
+        || cudaMemcpy(n_ax.p + (size_t)(n0 + n1) * AX, rz.data(), rz.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) return bail("axis upload");
     cudaStreamSynchronize(ctx->stream);                                          // no launch may still read the old tables
-    cudaFree(ctx->d_tuv); cudaFree(ctx->d_rho); cudaFree(ctx->d_ax);
-    ctx->d_tuv = n_tuv; ctx->d_rho = n_rho; ctx->d_ax = n_ax;
+    ctx->d_tuv = std::move(n_tuv); ctx->d_rho = std::move(n_rho); ctx->d_ax = std::move(n_ax);
     Grid3D& g = ctx->grid;
-    g.tuv = ctx->d_tuv; g.rho = ctx->d_rho; g.ax0 = ctx->d_ax; g.ax1 = ctx->d_ax + (size_t)n0 * AX; g.axz = ctx->d_ax + (size_t)(n0 + n1) * AX;
+    g.tuv = ctx->d_tuv.p; g.rho = ctx->d_rho.p; g.ax0 = ctx->d_ax.p; g.ax1 = ctx->d_ax.p + (size_t)n0 * AX; g.axz = ctx->d_ax.p + (size_t)(n0 + n1) * AX;
     g.n0 = n0; g.n1 = n1; g.nz = nz; g.scratch = nullptr; g.role = 0; g.nrole = 1; g.glane0 = 0; g.gmask = 0;
     g.amin = ax0[0]; g.amax = ax0[n0 - 1]; g.bmin = ax1[0]; g.bmax = ax1[n1 - 1]; g.zmin = z[0]; g.zmax = z[nz - 1];
     // GeoAc_SetPropRegion: G2S_MultiDimSpline3D.cpp:22-33 / G2S_GlobalMultiDimSpline3D.cpp:22-33
@@ -424,12 +437,12 @@ extern "C" int geoac_set_atmosphere_3d(geoac_ctx* ctx, int n0, int n1, int nz, c
 // Test hook: the node tables as the kernels read them (tuv[n0][n1][nz][18], rho[n0][n1][nz][2]; mspline.cuh).
 extern "C" int geoac_get_grid_tables(geoac_ctx* ctx, int64_t cap_tuv, double* tuv, int64_t cap_rho, double* rho) {
     if (!ctx) return GEOAC_ERR_BAD_ARG;
-    if (!ctx->is_grid || !ctx->d_tuv) return fail(ctx, GEOAC_ERR_NO_ATMO, "no range-dependent atmosphere set");
+    if (!ctx->is_grid || !ctx->d_tuv.p) return fail(ctx, GEOAC_ERR_NO_ATMO, "no range-dependent atmosphere set");
     const size_t nodes = (size_t)ctx->grid.n0 * ctx->grid.n1 * ctx->grid.nz;
     if (!tuv || !rho || (size_t)cap_tuv < nodes * MS_STRIDE || (size_t)cap_rho < nodes * 2) return fail(ctx, GEOAC_ERR_BAD_ARG, "get_grid_tables: buffers too small");
     cudaSetDevice(ctx->device);
-    CK(cudaMemcpy(tuv, ctx->d_tuv, nodes * MS_STRIDE * sizeof(double), cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(rho, ctx->d_rho, nodes * 2 * sizeof(double), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(tuv, ctx->d_tuv.p, nodes * MS_STRIDE * sizeof(double), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(rho, ctx->d_rho.p, nodes * 2 * sizeof(double), cudaMemcpyDeviceToHost));
     return GEOAC_OK;
 }
 
@@ -475,11 +488,11 @@ static int refresh_consts(geoac_ctx* ctx) {
     L.seg_mode = (ctx->variant == GEOAC_2D) ? 1 : (p.accum_per_segment ? 1 : 0);                          // App. A-2
     L.step_limit = (int)(p.ray_limit * (int)(1.0 / (p.ds_min * 10)));                                     // Solver.cpp:14
     L.per_bounce_zmax = (ctx->variant == GEOAC_3D_RNGDEP || ctx->variant == GEOAC_GLOBAL_RNGDEP);         // App. A-3
-    if (ctx->is_grid) setup_consts_grid_kernel<<<1, 32, 0, ctx->stream>>>(ctx->d_consts, L, ctx->grid, ctx->variant);
+    if (ctx->is_grid) setup_consts_grid_kernel<<<1, 32, 0, ctx->stream>>>(ctx->d_consts.p, L, ctx->grid, ctx->variant);
     else {
-        setup_consts_kernel<<<1, 32, 0, ctx->stream>>>(ctx->d_consts, L, ctx->d_table, ctx->n, ctx->xmin, ctx->xmax, ctx->variant);
-        build_sbpoly_kernel<<<(ctx->n - 1 + 63) / 64, 64, 0, ctx->stream>>>(ctx->d_consts, ctx->d_table, ctx->n, ctx->xmin, ctx->xmax,
-                                                                            ctx->variant == GEOAC_GLOBAL, ctx->d_sbpoly);
+        setup_consts_kernel<<<1, 32, 0, ctx->stream>>>(ctx->d_consts.p, L, ctx->d_table.p, ctx->n, ctx->xmin, ctx->xmax, ctx->variant);
+        build_sbpoly_kernel<<<(ctx->n - 1 + 63) / 64, 64, 0, ctx->stream>>>(ctx->d_consts.p, ctx->d_table.p, ctx->n, ctx->xmin, ctx->xmax,
+                                                                            ctx->variant == GEOAC_GLOBAL, ctx->d_sbpoly.p);
     }
     CK(cudaGetLastError());
     ctx->consts_dirty = false;
@@ -487,16 +500,6 @@ static int refresh_consts(geoac_ctx* ctx) {
 }
 
 // ---- kernel launch ----
-// device buffers that only grow: kept across calls, reallocated when a call needs more (need and cap in bytes)
-template <class T>
-static int grow(geoac_ctx* ctx, T*& buf, size_t& cap, size_t need) {
-    if (need <= cap) return GEOAC_OK;
-    cudaFree(buf); buf = nullptr; cap = 0;
-    CK(cudaMalloc(&buf, need));
-    cap = need;
-    return GEOAC_OK;
-}
-
 // cost scout: predicted RK4 step counts of the rays into ctx->d_cost, their maximum and sum.  Persistent, the table in shared
 // memory when it fits.
 template <class SEQ>
@@ -513,9 +516,9 @@ static int launch_cost_scout(geoac_ctx* ctx, const TraceArgs& a, int max_optin, 
     int s_per_sm = 1;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&s_per_sm, sfn, kScoutBlock, s_smem));
     const int sblocks = (int)std::min<int64_t>((int64_t)ctx->sm_count * std::max(1, s_per_sm), (a.n_rays + kScoutBlock - 1) / kScoutBlock);
-    unsigned long long* scounter = ctx->d_counters + 3;
+    unsigned long long* scounter = ctx->d_counters.p + 3;
     int coarse = ctx->knobs.scout_coarse > 0 ? ctx->knobs.scout_coarse : (kGrid ? kScoutCoarse : 2 * kScoutCoarse);   // stratified: 32x measured best (404.8 vs 421.0 / 443.3 ms at 16x / 64x)
-    void* sargs[] = { (void*)&a, (void*)&ctx->d_cost, (void*)&cmax, (void*)&cost_sum, (void*)&scounter, (void*)&coarse };
+    void* sargs[] = { (void*)&a, (void*)&ctx->d_cost.p, (void*)&cmax, (void*)&cost_sum, (void*)&scounter, (void*)&coarse };
     CK(cudaLaunchKernel(sfn, dim3(sblocks), dim3(kScoutBlock), sargs, s_smem, st));
     ctx->last_launches += 1;
     return GEOAC_OK;
@@ -532,52 +535,50 @@ static int build_claim_order(geoac_ctx* ctx, TraceArgs& a, long long lanes, int 
     const size_t ids = sizeof(uint32_t) * n_entries;
     // d_hist: [0..255] buckets, [256] largest cost, [257] long packets, [258] quarter packets, [260..261] cost sum (64 bit)
     const size_t hist_bytes = sizeof(uint32_t) * (kCostBuckets + 8);
-    int rc;
-    if ((rc = grow(ctx, ctx->d_cost, ctx->cap_cost, ids)) || (rc = grow(ctx, ctx->d_order, ctx->cap_order, ids))
-        || (rc = grow(ctx, ctx->d_hist, ctx->cap_hist, hist_bytes))) return rc;
-    CK(cudaMemsetAsync(ctx->d_hist, 0, hist_bytes, st));
-    uint32_t* cmax = ctx->d_hist + kCostBuckets;
+    CK(ctx->d_cost.grow(ids)); CK(ctx->d_order.grow(ids)); CK(ctx->d_hist.grow(hist_bytes));
+    CK(cudaMemsetAsync(ctx->d_hist.p, 0, hist_bytes, st));
+    uint32_t* cmax = ctx->d_hist.p + kCostBuckets;
     uint32_t* n_long = cmax + 1;                              // n_long[1]: quarter packets
     unsigned long long* cost_sum = reinterpret_cast<unsigned long long*>(cmax + 4);
-    if ((rc = launch_cost_scout<typename EQ::Scout>(ctx, a, max_optin, st, cmax, cost_sum))) return rc;
+    if (int rc = launch_cost_scout<typename EQ::Scout>(ctx, a, max_optin, st, cmax, cost_sum)) return rc;
     if (kGrid) {
-        const uint32_t* cost = ctx->d_cost;
+        const uint32_t* cost = ctx->d_cost.p;
         if (ctx->knobs.dilate > 0) {
             // the estimate used for the claim order: maximum over the inclination neighbours (trace_kernel.cuh: cost_dilate_kernel)
-            if ((rc = grow(ctx, ctx->d_cost_dilated, ctx->cap_cost_dilated, ids))) return rc;
-            cost_dilate_kernel<<<ctx->sm_count * 2, 256, 0, st>>>(ctx->d_cost, a.theta, n, ctx->knobs.dilate * 1e-3 * kPi / 180.0, 16, ctx->d_cost_dilated);
-            cost = ctx->d_cost_dilated;
+            CK(ctx->d_cost_dilated.grow(ids));
+            cost_dilate_kernel<<<ctx->sm_count * 2, 256, 0, st>>>(ctx->d_cost.p, a.theta, n, ctx->knobs.dilate * 1e-3 * kPi / 180.0, 16, ctx->d_cost_dilated.p);
+            cost = ctx->d_cost_dilated.p;
             ctx->last_launches += 1;
         }
         // packets by cost bucket, longest first; also counts the long and the quarter packets
-        order_hist_kernel<<<ctx->sm_count, 256, 0, st>>>(cost, n, group, cmax, ctx->d_hist, cost_sum, lanes, n_long, ctx->knobs.long_alpha, n_long + 1, ctx->knobs.quarter_alpha);
-        order_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_hist);
-        order_scatter_kernel<<<ctx->sm_count, 256, 0, st>>>(cost, n, group, cmax, ctx->d_hist, ctx->d_order);
+        order_hist_kernel<<<ctx->sm_count, 256, 0, st>>>(cost, n, group, cmax, ctx->d_hist.p, cost_sum, lanes, n_long, ctx->knobs.long_alpha, n_long + 1, ctx->knobs.quarter_alpha);
+        order_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_hist.p);
+        order_scatter_kernel<<<ctx->sm_count, 256, 0, st>>>(cost, n, group, cmax, ctx->d_hist.p, ctx->d_order.p);
         ctx->last_launches += 3;
     } else {
         // order by (cost bucket, inclination, batch index) + whole-warp refill: a warp's lanes then read the same few table
         // records (trace_kernel.cuh).  Two stable counting-sort passes, inclination first.
         const int nblk = ctx->sm_count;
         const int64_t chunk = (n + nblk - 1) / nblk;
-        if ((rc = grow(ctx, ctx->d_blockhist, ctx->cap_blockhist, sizeof(uint32_t) * (size_t)nblk * kCostBuckets + 2 * sizeof(double)))
-            || (rc = grow(ctx, ctx->d_keys, ctx->cap_keys, (size_t)2 * n)) || (rc = grow(ctx, ctx->d_order2, ctx->cap_order2, ids))) return rc;
-        double* trange = reinterpret_cast<double*>(ctx->d_blockhist + (size_t)nblk * kCostBuckets);
-        uint8_t *key_t = ctx->d_keys, *key_c = ctx->d_keys + n;
+        CK(ctx->d_blockhist.grow(sizeof(uint32_t) * (size_t)nblk * kCostBuckets + 2 * sizeof(double)));
+        CK(ctx->d_keys.grow((size_t)2 * n)); CK(ctx->d_order2.grow(ids));
+        double* trange = reinterpret_cast<double*>(ctx->d_blockhist.p + (size_t)nblk * kCostBuckets);
+        uint8_t *key_t = ctx->d_keys.p, *key_c = ctx->d_keys.p + n;
         order_theta_range_kernel<<<1, 1024, 0, st>>>(a.theta, n, trange);
-        order_keys_kernel<<<ctx->sm_count, 256, 0, st>>>(ctx->d_cost, a.theta, n, cmax, trange, key_t, key_c, ctx->knobs.cost_shift);
+        order_keys_kernel<<<ctx->sm_count, 256, 0, st>>>(ctx->d_cost.p, a.theta, n, cmax, trange, key_t, key_c, ctx->knobs.cost_shift);
         auto pass = [&](const uint8_t* key, const uint32_t* src, uint32_t* dst) {
-            stable_hist_kernel<<<nblk, 256, 0, st>>>(key, src, n, chunk, ctx->d_blockhist);
-            stable_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_blockhist, nblk);
-            stable_scatter_kernel<<<nblk, 32, 0, st>>>(key, src, n, chunk, ctx->d_blockhist, dst);
+            stable_hist_kernel<<<nblk, 256, 0, st>>>(key, src, n, chunk, ctx->d_blockhist.p);
+            stable_scan_kernel<<<1, kCostBuckets, 0, st>>>(ctx->d_blockhist.p, nblk);
+            stable_scatter_kernel<<<nblk, 32, 0, st>>>(key, src, n, chunk, ctx->d_blockhist.p, dst);
         };
-        pass(key_t, nullptr, ctx->d_order2);
-        pass(key_c, ctx->d_order2, ctx->d_order);
+        pass(key_t, nullptr, ctx->d_order2.p);
+        pass(key_c, ctx->d_order2.p, ctx->d_order.p);
         ctx->last_launches += 8;
         a.packet_refill = 1;
     }
     CK(cudaGetLastError());
     a.n_claims = n_entries;
-    a.order = ctx->d_order;
+    a.order = ctx->d_order.p;
     n_quarter = 0;
     if (kGrid && ctx->knobs.coop) {
         // the long region: packets that would outlast the pass on a fully loaded SM.  Their count sizes the second launch.
@@ -619,12 +620,12 @@ static int enqueue_launches(geoac_ctx* ctx, const void* fn, size_t smem, int max
         if (NeedsPrev<EQ>::value) {                          // y_{k-1} scratch of both launches, the long one's after the main one's
             const size_t main_doubles = (size_t)EQ::NEQ * grid * BLOCK;
             const size_t need = (main_doubles + (size_t)EQ::NEQ * grid_long * BLOCK) * sizeof(double);
-            if (need > ctx->cap_prev) {
+            if (need > ctx->d_prev.cap) {
                 CK(cudaStreamSynchronize(st));                // a trace still running may use the old scratch
-                if (int rc = grow(ctx, ctx->d_prev, ctx->cap_prev, need)) return rc;
+                CK(ctx->d_prev.grow(need));
             }
-            a.prev = ctx->d_prev;
-            al.prev = ctx->d_prev + main_doubles;
+            a.prev = ctx->d_prev.p;
+            al.prev = ctx->d_prev.p + main_doubles;
         }
         CK(cudaEventRecord(ctx->ev_fork, st));
         CK(cudaStreamWaitEvent(ctx->stream_long, ctx->ev_fork, 0));
@@ -668,11 +669,9 @@ static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
     const int64_t warps_needed = (a.n_rays + 31) / 32;
     const int64_t ctas_needed = std::max<int64_t>(1, (warps_needed + (BLOCK / 32) - 1) / (BLOCK / 32));
     const int grid = (int)std::min<int64_t>((int64_t)ctx->sm_count * per_sm, ctas_needed);
-    if (NeedsPrev<EQ>::value) {
-        if (int rc = grow(ctx, ctx->d_prev, ctx->cap_prev, (size_t)EQ::NEQ * grid * BLOCK * sizeof(double))) return rc;
-    }
-    a.prev = ctx->d_prev;
-    a.order = nullptr; a.n_claims = a.n_rays; a.n_long_packets = 0; a.n_quarter_packets = 0; a.counter_long = ctx->d_counters + 4; a.counter_quarter = ctx->d_counters + 5;
+    if (NeedsPrev<EQ>::value) CK(ctx->d_prev.grow((size_t)EQ::NEQ * grid * BLOCK * sizeof(double)));
+    a.prev = ctx->d_prev.p;
+    a.order = nullptr; a.n_claims = a.n_rays; a.n_long_packets = 0; a.n_quarter_packets = 0; a.counter_long = ctx->d_counters.p + 4; a.counter_quarter = ctx->d_counters.p + 5;
     a.prefer_long = 0; a.packet_refill = 0;
     ctx->last_launches = 0; ctx->last_long_packets = 0; ctx->last_long_ctas = 0; ctx->last_quarter_packets = 0;
     int grid_long = 0;
@@ -707,34 +706,22 @@ static int dispatch_trace(geoac_ctx* ctx, const TraceArgs& a, cudaStream_t st) {
     return fail(ctx, GEOAC_ERR_BAD_ARG, "variant not implemented");
 }
 
-struct PathArgs { double* path = nullptr; int32_t* rows = nullptr; int stride = 0; int64_t cap = 0;
-                  double* caus = nullptr; int32_t* caus_rows = nullptr; int64_t caus_cap = 0; };
-
-static int enqueue_trace(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, const double* d_phi,
-                         double* d_rec, int32_t* d_status, int32_t* d_n_steps, cudaStream_t st, const PathArgs& pa = PathArgs()) {
-    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");
-    int rc = refresh_consts(ctx);
-    if (rc) return rc;
-    if (st != ctx->stream) {       // consts were written on ctx->stream: order the caller's stream after it
-        CK(cudaEventRecord(ctx->ev0, ctx->stream));
-        CK(cudaStreamWaitEvent(st, ctx->ev0, 0));
-    }
+// One trace on `st`: zeroes the records and counters, fills in the context's part of `a` and launches.  The caller sets the
+// rays (theta, phi, n_rays) and their outputs (rec, status, n_steps), and the capture fields (zero: no capture).  The launch
+// invariants must be current (refresh_consts) and ordered before `st`.
+static int enqueue_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
     const int n_rec = ctx->prm.bounces + 1;
-    const int64_t n_slots = n_rays * n_rec;
-    CK(cudaMemsetAsync(ctx->d_counters, 0, 8 * sizeof(unsigned long long), st));
-    CK(cudaMemsetAsync(d_rec, 0, sizeof(double) * GEOAC_NFIELDS * n_slots, st));
-    CK(cudaMemsetAsync(d_status, 0, sizeof(int32_t) * n_slots, st));
-    CK(cudaMemsetAsync(d_n_steps, 0, sizeof(int32_t) * n_slots, st));
-    TraceArgs a;
+    const int64_t n_slots = a.n_rays * n_rec;
+    CK(cudaMemsetAsync(ctx->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(a.rec, 0, sizeof(double) * GEOAC_NFIELDS * n_slots, st));
+    CK(cudaMemsetAsync(a.status, 0, sizeof(int32_t) * n_slots, st));
+    CK(cudaMemsetAsync(a.n_steps, 0, sizeof(int32_t) * n_slots, st));
     a.grid = ctx->grid;
-    a.table = ctx->d_table; a.table_n = ctx->n; a.table_xmin = ctx->xmin; a.table_xmax = ctx->xmax;
-    a.sbpoly = (ctx->is_grid || !ctx->knobs.sbpoly) ? nullptr : ctx->d_sbpoly;   // knob sbpoly = 0: the full absorption model at every step (A/B measurements, tests)
-    a.consts = ctx->d_consts; a.theta = d_theta; a.phi = d_phi; a.n_rays = n_rays; a.n_rec = n_rec;
-    a.rec = d_rec; a.status = d_status; a.n_steps = d_n_steps;
-    a.counter = ctx->d_counters; a.total_steps = ctx->d_counters + 1; a.warp_trips = ctx->d_counters + 2;
-    a.path = pa.path; a.path_rows = pa.rows; a.path_stride = pa.stride; a.path_cap = pa.cap;
-    a.caus = pa.caus; a.caus_rows = pa.caus_rows; a.caus_cap = pa.caus_cap;
-    return (pa.stride > 0 || pa.caus_cap > 0) ? dispatch_trace<true>(ctx, a, st) : dispatch_trace<false>(ctx, a, st);
+    a.table = ctx->d_table.p; a.table_n = ctx->n; a.table_xmin = ctx->xmin; a.table_xmax = ctx->xmax;
+    a.sbpoly = (ctx->is_grid || !ctx->knobs.sbpoly) ? nullptr : ctx->d_sbpoly.p;   // knob sbpoly = 0: the full absorption model at every step (A/B measurements, tests)
+    a.consts = ctx->d_consts.p; a.n_rec = n_rec;
+    a.counter = ctx->d_counters.p; a.total_steps = ctx->d_counters.p + 1; a.warp_trips = ctx->d_counters.p + 2;
+    return (a.path_stride > 0 || a.caus_cap > 0) ? dispatch_trace<true>(ctx, a, st) : dispatch_trace<false>(ctx, a, st);
 }
 
 extern "C" int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, const double* d_phi,
@@ -742,16 +729,23 @@ extern "C" int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* 
     if (!ctx || n_rays < 0) return GEOAC_ERR_BAD_ARG;
     if (n_rays == 0) return GEOAC_OK;
     cudaSetDevice(ctx->device);
-    return enqueue_trace(ctx, n_rays, d_theta, d_phi, d_rec, d_status, d_n_steps, (cudaStream_t)cuda_stream);
+    if (int rc = refresh_consts(ctx)) return rc;
+    const cudaStream_t st = (cudaStream_t)cuda_stream;
+    if (st != ctx->stream) {       // consts were written on ctx->stream: order the caller's stream after it
+        CK(cudaEventRecord(ctx->ev0, ctx->stream));
+        CK(cudaStreamWaitEvent(st, ctx->ev0, 0));
+    }
+    TraceArgs a{};
+    a.theta = d_theta; a.phi = d_phi; a.n_rays = n_rays; a.rec = d_rec; a.status = d_status; a.n_steps = d_n_steps;
+    return enqueue_trace(ctx, a, st);
 }
 
 // device staging of the host-buffer entry point (angles in, records out), grown on demand and kept across calls
 static int reserve_staging(geoac_ctx* ctx, int64_t n_rays) {
     const size_t n_slots = (size_t)n_rays * (ctx->prm.bounces + 1);
-    int rc;
-    if ((rc = grow(ctx, ctx->d_theta, ctx->cap_theta, sizeof(double) * n_rays)) || (rc = grow(ctx, ctx->d_phi, ctx->cap_phi, sizeof(double) * n_rays))
-        || (rc = grow(ctx, ctx->d_rec, ctx->cap_rec, sizeof(double) * GEOAC_NFIELDS * n_slots))
-        || (rc = grow(ctx, ctx->d_status, ctx->cap_status, sizeof(int32_t) * n_slots)) || (rc = grow(ctx, ctx->d_nsteps, ctx->cap_nsteps, sizeof(int32_t) * n_slots))) return rc;
+    CK(ctx->d_theta.grow(sizeof(double) * n_rays)); CK(ctx->d_phi.grow(sizeof(double) * n_rays));
+    CK(ctx->d_rec.grow(sizeof(double) * GEOAC_NFIELDS * n_slots));
+    CK(ctx->d_status.grow(sizeof(int32_t) * n_slots)); CK(ctx->d_nsteps.grow(sizeof(int32_t) * n_slots));
     return GEOAC_OK;
 }
 
@@ -768,81 +762,6 @@ extern "C" int geoac_reserve(geoac_ctx* ctx, int64_t n_rays) {
     return reserve_staging(ctx, n_rays);
 }
 
-static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
-                      double* rec, int32_t* status, int32_t* n_steps, int path_stride, int64_t path_cap, double* path, int32_t* path_rows,
-                      int64_t caus_cap, double* caus, int32_t* caus_rows) {
-    if (!ctx || n_rays < 0 || (n_rays > 0 && (!theta || !phi || !rec || !status || !n_steps))) return GEOAC_ERR_BAD_ARG;
-    if (path_stride > 0 && (path_cap <= 0 || !path || !path_rows)) return fail(ctx, GEOAC_ERR_BAD_ARG, "raypath capture needs path buffers and a positive row capacity");
-    if (caus_cap > 0 && (!caus || !caus_rows)) return fail(ctx, GEOAC_ERR_BAD_ARG, "caustic capture needs its buffers");
-    if (caus_cap > 0 && !ctx->prm.calc_amp) return fail(ctx, GEOAC_ERR_BAD_ARG, "caustic capture needs calc_amp = 1 (the Jacobian uses the auxiliary equations)");
-    if ((path_stride > 0 || caus_cap > 0) && ctx->variant != GEOAC_2D && !ctx->prm.accum_per_segment)
-        return fail(ctx, GEOAC_ERR_BAD_ARG, "raypath / caustic rows need accum_per_segment = 1 (the mains' WriteRays accumulation, SURVEY App. A-2)");
-    if (n_rays == 0) return GEOAC_OK;
-    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");
-    cudaSetDevice(ctx->device);
-    const int n_rec = ctx->prm.bounces + 1;
-    const int64_t n_slots = n_rays * n_rec;
-    int rsv = reserve_staging(ctx, n_rays);
-    if (rsv) return rsv;
-    PathArgs pa;
-    cudaStream_t st = ctx->stream;
-    if (path_stride > 0) {
-        const size_t need = (size_t)n_rays * path_cap * GEOAC_PATH_NF * sizeof(double);
-        int g1 = grow(ctx, ctx->d_path, ctx->cap_path, need); if (g1) return g1;
-        int g2 = grow(ctx, ctx->d_path_rows, ctx->cap_path_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
-        CK(cudaMemsetAsync(ctx->d_path, 0, need, st));
-        CK(cudaMemsetAsync(ctx->d_path_rows, 0, sizeof(int32_t) * n_rays, st));
-        pa.path = ctx->d_path; pa.rows = ctx->d_path_rows; pa.stride = path_stride; pa.cap = path_cap;
-    }
-    if (caus_cap > 0) {
-        const size_t need = (size_t)n_rays * caus_cap * GEOAC_CAUSTIC_NF * sizeof(double);
-        int g1 = grow(ctx, ctx->d_caus, ctx->cap_caus, need); if (g1) return g1;
-        int g2 = grow(ctx, ctx->d_caus_rows, ctx->cap_caus_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
-        CK(cudaMemsetAsync(ctx->d_caus, 0, need, st));
-        CK(cudaMemsetAsync(ctx->d_caus_rows, 0, sizeof(int32_t) * n_rays, st));
-        pa.caus = ctx->d_caus; pa.caus_rows = ctx->d_caus_rows; pa.caus_cap = caus_cap;
-    }
-    CK(cudaMemcpyAsync(ctx->d_theta, theta, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->d_phi, phi, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
-    int rc = refresh_consts(ctx);
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev0, st));
-    rc = enqueue_trace(ctx, n_rays, ctx->d_theta, ctx->d_phi, ctx->d_rec, ctx->d_status, ctx->d_nsteps, st, pa);
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev1, st));
-    CK(cudaMemcpyAsync(rec, ctx->d_rec, sizeof(double) * GEOAC_NFIELDS * n_slots, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(status, ctx->d_status, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(n_steps, ctx->d_nsteps, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
-    if (path_stride > 0) {
-        CK(cudaMemcpyAsync(path, ctx->d_path, (size_t)n_rays * path_cap * GEOAC_PATH_NF * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(path_rows, ctx->d_path_rows, sizeof(int32_t) * n_rays, cudaMemcpyDeviceToHost, st));
-    }
-    if (caus_cap > 0) {
-        CK(cudaMemcpyAsync(caus, ctx->d_caus, (size_t)n_rays * caus_cap * GEOAC_CAUSTIC_NF * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(caus_rows, ctx->d_caus_rows, sizeof(int32_t) * n_rays, cudaMemcpyDeviceToHost, st));
-    }
-    unsigned long long cnt[2] = { 0, 0 };
-    CK(cudaMemcpyAsync(cnt, ctx->d_counters, sizeof cnt, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    float ms = 0.f; cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    ctx->last_ms = ms; ctx->last_steps = (int64_t)cnt[1];
-    return GEOAC_OK;
-}
-
-extern "C" int geoac_trace(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
-                           double* rec, int32_t* status, int32_t* n_steps) {
-    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, 0, 0, nullptr, nullptr, 0, nullptr, nullptr);
-}
-
-extern "C" int geoac_trace_paths(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
-                                 double* rec, int32_t* status, int32_t* n_steps,
-                                 int path_stride, int64_t path_cap, double* path, int32_t* path_rows,
-                                 int64_t caustic_cap, double* caustic, int32_t* caustic_rows) {
-    if (path_stride < 0 || caustic_cap < 0 || (path_stride == 0 && caustic_cap == 0))
-        return ctx ? fail(ctx, GEOAC_ERR_BAD_ARG, "ask for raypath rows (path_stride > 0) and / or caustic events (caustic_cap > 0)") : GEOAC_ERR_BAD_ARG;
-    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, path_stride, path_cap, path, path_rows, caustic_cap, caustic, caustic_rows);
-}
-
 // ---- compacted raypath / caustic rows: only the rows produced cross PCIe ----
 __global__ void compact_rows_kernel(const double* dense, const int32_t* rows, const int64_t* offs, int64_t n, int64_t cap, int nf, double* out) {
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -855,86 +774,112 @@ __global__ void compact_rows_kernel(const double* dense, const int32_t* rows, co
     }
 }
 
+// What a host trace captures besides the records (none for geoac_trace).  Dense: data[ray][cap][nf] and the rows produced per
+// ray in `rows` (rows past cap are counted, not kept).  Compact: the kept rows ray after ray in `data`, which has room for
+// total_cap of them; ray i's run from offs[i] to offs[i + 1].
+enum class Capture { none, dense, compact };
+struct CaptureOut { int64_t cap = 0; double* data = nullptr; int32_t* rows = nullptr; int64_t* offs = nullptr; int64_t total_cap = 0; };
+
+// The host-buffer trace (geoac_trace, geoac_trace_paths, geoac_trace_paths_compact, each context of geoac_trace_multi):
+// angles in, one trace on ctx->stream, records out, plus the raypath rows (every path_stride steps) and caustic events asked for.
+static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps,
+                      Capture mode = Capture::none, int path_stride = 0, CaptureOut path = {}, CaptureOut caus = {}) {
+    if (!ctx || n_rays < 0 || (n_rays > 0 && (!theta || !phi || !rec || !status || !n_steps))) return GEOAC_ERR_BAD_ARG;
+    const bool compact = mode == Capture::compact;
+    auto has_rows = [&](const CaptureOut& c) { return compact ? c.offs != nullptr : c.rows != nullptr; };
+    if (mode != Capture::none && (path_stride < 0 || caus.cap < 0 || (path_stride == 0 && caus.cap == 0)))
+        return fail(ctx, GEOAC_ERR_BAD_ARG, "ask for raypath rows (path_stride > 0) and / or caustic events (caustic_cap > 0)");
+    if (path_stride > 0 && (path.cap <= 0 || !path.data || !has_rows(path)))
+        return fail(ctx, GEOAC_ERR_BAD_ARG, compact ? "raypath capture needs its buffers and a positive per-ray capacity"
+                                                    : "raypath capture needs path buffers and a positive row capacity");
+    if (caus.cap > 0 && (!caus.data || !has_rows(caus))) return fail(ctx, GEOAC_ERR_BAD_ARG, "caustic capture needs its buffers");
+    if (caus.cap > 0 && !ctx->prm.calc_amp) return fail(ctx, GEOAC_ERR_BAD_ARG, "caustic capture needs calc_amp = 1 (the Jacobian uses the auxiliary equations)");
+    if ((path_stride > 0 || caus.cap > 0) && ctx->variant != GEOAC_2D && !ctx->prm.accum_per_segment)
+        return fail(ctx, GEOAC_ERR_BAD_ARG, "raypath / caustic rows need accum_per_segment = 1 (the mains' WriteRays accumulation, SURVEY App. A-2)");
+    if (compact && path_stride > 0) path.offs[0] = 0;
+    if (compact && caus.cap > 0) caus.offs[0] = 0;
+    if (n_rays == 0) return GEOAC_OK;
+    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");
+    cudaSetDevice(ctx->device);
+    const int64_t n_slots = n_rays * (ctx->prm.bounces + 1);
+    if (int rc = reserve_staging(ctx, n_rays)) return rc;
+    const cudaStream_t st = ctx->stream;
+    // the captures asked for, staged dense in the context: [ray][cap][nf] and the row count of each ray
+    struct Staged { const CaptureOut& out; Buf<double>& data; Buf<int32_t>& rows; int nf; const char* what; };
+    std::vector<Staged> staged;
+    if (path_stride > 0) staged.push_back({ path, ctx->d_path, ctx->d_path_rows, GEOAC_PATH_NF, "raypath rows" });
+    if (caus.cap > 0) staged.push_back({ caus, ctx->d_caus, ctx->d_caus_rows, GEOAC_CAUSTIC_NF, "caustic rows" });
+    for (const Staged& s : staged) {
+        const size_t bytes = (size_t)n_rays * s.out.cap * s.nf * sizeof(double);
+        CK(s.data.grow(bytes)); CK(s.rows.grow(sizeof(int32_t) * n_rays));
+        if (!compact) CK(cudaMemsetAsync(s.data.p, 0, bytes, st));       // the caller receives every slot; compaction copies only rows produced
+        CK(cudaMemsetAsync(s.rows.p, 0, sizeof(int32_t) * n_rays, st));
+    }
+    TraceArgs a{};
+    a.theta = ctx->d_theta.p; a.phi = ctx->d_phi.p; a.n_rays = n_rays; a.rec = ctx->d_rec.p; a.status = ctx->d_status.p; a.n_steps = ctx->d_nsteps.p;
+    if (path_stride > 0) { a.path = ctx->d_path.p; a.path_rows = ctx->d_path_rows.p; a.path_stride = path_stride; a.path_cap = path.cap; }
+    if (caus.cap > 0) { a.caus = ctx->d_caus.p; a.caus_rows = ctx->d_caus_rows.p; a.caus_cap = caus.cap; }
+    CK(cudaMemcpyAsync(ctx->d_theta.p, theta, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->d_phi.p, phi, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
+    if (int rc = refresh_consts(ctx)) return rc;                         // before ev0: the timed window holds the trace alone
+    CK(cudaEventRecord(ctx->ev0, st));
+    if (int rc = enqueue_trace(ctx, a, st)) return rc;
+    CK(cudaEventRecord(ctx->ev1, st));
+    CK(cudaMemcpyAsync(rec, ctx->d_rec.p, sizeof(double) * GEOAC_NFIELDS * n_slots, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, ctx->d_status.p, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(n_steps, ctx->d_nsteps.p, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
+    std::vector<int32_t> h_rows;
+    for (const Staged& s : staged) {
+        const int64_t cap = s.out.cap;
+        if (!compact) {
+            CK(cudaMemcpyAsync(s.out.data, s.data.p, (size_t)n_rays * cap * s.nf * sizeof(double), cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(s.out.rows, s.rows.p, sizeof(int32_t) * n_rays, cudaMemcpyDeviceToHost, st));
+            continue;
+        }
+        // per-ray row counts -> offsets on the host (n_rays integers), rows gathered on the device, only those copied out
+        h_rows.resize((size_t)n_rays);
+        CK(cudaMemcpyAsync(h_rows.data(), s.rows.p, sizeof(int32_t) * n_rays, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        int64_t* offs = s.out.offs;
+        for (int64_t i = 0; i < n_rays; i++) offs[i + 1] = offs[i] + std::min<int64_t>(h_rows[(size_t)i], cap);
+        const int64_t total = offs[n_rays];
+        if (total > s.out.total_cap) return fail(ctx, GEOAC_ERR_TOO_LARGE, std::string(s.what) + ": " + std::to_string(total) + " rows produced, buffer holds "
+                                                 + std::to_string(s.out.total_cap) + " (the offsets are filled in: the last one is the size to allocate)");
+        if (total == 0) continue;
+        Buf<int64_t> d_offs; Buf<double> d_out;                        // scratch of this call: nothing of it stays allocated
+        CK(d_offs.grow(sizeof(int64_t) * (n_rays + 1))); CK(d_out.grow(sizeof(double) * total * s.nf));
+        CK(cudaMemcpyAsync(d_offs.p, offs, sizeof(int64_t) * (n_rays + 1), cudaMemcpyHostToDevice, st));
+        compact_rows_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(s.data.p, s.rows.p, d_offs.p, n_rays, cap, s.nf, d_out.p);
+        CK(cudaMemcpyAsync(s.out.data, d_out.p, sizeof(double) * total * s.nf, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
+    unsigned long long cnt[2] = { 0, 0 };
+    CK(cudaMemcpyAsync(cnt, ctx->d_counters.p, sizeof cnt, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0.f; cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
+    ctx->last_ms = ms; ctx->last_steps = (int64_t)cnt[1];
+    return GEOAC_OK;
+}
+
+extern "C" int geoac_trace(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
+                           double* rec, int32_t* status, int32_t* n_steps) {
+    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps);
+}
+
+extern "C" int geoac_trace_paths(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
+                                 double* rec, int32_t* status, int32_t* n_steps,
+                                 int path_stride, int64_t path_cap, double* path, int32_t* path_rows,
+                                 int64_t caustic_cap, double* caustic, int32_t* caustic_rows) {
+    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, Capture::dense, path_stride,
+                      { path_cap, path, path_rows }, { caustic_cap, caustic, caustic_rows });
+}
+
 extern "C" int geoac_trace_paths_compact(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
                                          double* rec, int32_t* status, int32_t* n_steps,
                                          int path_stride, int64_t path_cap, int64_t path_total_cap, double* path, int64_t* path_offset,
                                          int64_t caustic_cap, int64_t caustic_total_cap, double* caustic, int64_t* caustic_offset) {
-    if (!ctx || n_rays < 0) return GEOAC_ERR_BAD_ARG;
-    if (path_stride < 0 || caustic_cap < 0 || (path_stride == 0 && caustic_cap == 0))
-        return fail(ctx, GEOAC_ERR_BAD_ARG, "ask for raypath rows (path_stride > 0) and / or caustic events (caustic_cap > 0)");
-    if (path_stride > 0 && (path_cap <= 0 || !path || !path_offset)) return fail(ctx, GEOAC_ERR_BAD_ARG, "raypath capture needs its buffers and a positive per-ray capacity");
-    if (caustic_cap > 0 && (!caustic || !caustic_offset)) return fail(ctx, GEOAC_ERR_BAD_ARG, "caustic capture needs its buffers");
-    if (n_rays > 0 && (!theta || !phi || !rec || !status || !n_steps)) return GEOAC_ERR_BAD_ARG;
-    if (caustic_cap > 0 && !ctx->prm.calc_amp) return fail(ctx, GEOAC_ERR_BAD_ARG, "caustic capture needs calc_amp = 1 (the Jacobian uses the auxiliary equations)");
-    if (ctx->variant != GEOAC_2D && !ctx->prm.accum_per_segment)
-        return fail(ctx, GEOAC_ERR_BAD_ARG, "raypath / caustic rows need accum_per_segment = 1 (the mains' WriteRays accumulation, SURVEY App. A-2)");
-    if (path_stride > 0) path_offset[0] = 0;
-    if (caustic_cap > 0) caustic_offset[0] = 0;
-    if (n_rays == 0) return GEOAC_OK;
-    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");
-    cudaSetDevice(ctx->device);
-    const int n_rec = ctx->prm.bounces + 1;
-    const int64_t n_slots = n_rays * n_rec;
-    int rsv = reserve_staging(ctx, n_rays);
-    if (rsv) return rsv;
-    PathArgs pa;
-    cudaStream_t st = ctx->stream;
-    if (path_stride > 0) {
-        const size_t need = (size_t)n_rays * path_cap * GEOAC_PATH_NF * sizeof(double);
-        int g1 = grow(ctx, ctx->d_path, ctx->cap_path, need); if (g1) return g1;
-        int g2 = grow(ctx, ctx->d_path_rows, ctx->cap_path_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
-        CK(cudaMemsetAsync(ctx->d_path_rows, 0, sizeof(int32_t) * n_rays, st));
-        pa.path = ctx->d_path; pa.rows = ctx->d_path_rows; pa.stride = path_stride; pa.cap = path_cap;
-    }
-    if (caustic_cap > 0) {
-        const size_t need = (size_t)n_rays * caustic_cap * GEOAC_CAUSTIC_NF * sizeof(double);
-        int g1 = grow(ctx, ctx->d_caus, ctx->cap_caus, need); if (g1) return g1;
-        int g2 = grow(ctx, ctx->d_caus_rows, ctx->cap_caus_rows, sizeof(int32_t) * n_rays); if (g2) return g2;
-        CK(cudaMemsetAsync(ctx->d_caus_rows, 0, sizeof(int32_t) * n_rays, st));
-        pa.caus = ctx->d_caus; pa.caus_rows = ctx->d_caus_rows; pa.caus_cap = caustic_cap;
-    }
-    CK(cudaMemcpyAsync(ctx->d_theta, theta, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->d_phi, phi, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
-    int rc = refresh_consts(ctx);
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev0, st));
-    rc = enqueue_trace(ctx, n_rays, ctx->d_theta, ctx->d_phi, ctx->d_rec, ctx->d_status, ctx->d_nsteps, st, pa);
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev1, st));
-    CK(cudaMemcpyAsync(rec, ctx->d_rec, sizeof(double) * GEOAC_NFIELDS * n_slots, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(status, ctx->d_status, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(n_steps, ctx->d_nsteps, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
-    // per-ray row counts -> offsets on the host (n_rays integers), rows gathered on the device, only those copied out
-    std::vector<int32_t> h_rows((size_t)n_rays);
-    int64_t* d_offs = nullptr; double* d_out = nullptr;
-    auto cleanup = [&]() { cudaFree(d_offs); cudaFree(d_out); };
-    auto compact = [&](const int32_t* d_rows, const double* d_dense, int64_t cap, int nf, int64_t total_cap, double* out, int64_t* offs, const char* what) -> int {
-        if (cudaMemcpyAsync(h_rows.data(), d_rows, sizeof(int32_t) * n_rays, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
-            return fail(ctx, GEOAC_ERR_CUDA, std::string(what) + ": row counts: " + cudaGetErrorString(cudaGetLastError()));
-        offs[0] = 0;
-        for (int64_t i = 0; i < n_rays; i++) offs[i + 1] = offs[i] + std::min<int64_t>(h_rows[(size_t)i], cap);
-        const int64_t total = offs[n_rays];
-        if (total > total_cap) return fail(ctx, GEOAC_ERR_TOO_LARGE, std::string(what) + ": " + std::to_string(total) + " rows produced, buffer holds " + std::to_string(total_cap)
-                                                                     + " (the offsets are filled in: the last one is the size to allocate)");
-        if (total == 0) return GEOAC_OK;
-        cudaFree(d_offs); cudaFree(d_out); d_offs = nullptr; d_out = nullptr;
-        if (cudaMalloc(&d_offs, sizeof(int64_t) * (n_rays + 1)) != cudaSuccess || cudaMalloc(&d_out, sizeof(double) * total * nf) != cudaSuccess)
-            return fail(ctx, GEOAC_ERR_CUDA, std::string(what) + ": out of device memory");
-        if (cudaMemcpyAsync(d_offs, offs, sizeof(int64_t) * (n_rays + 1), cudaMemcpyHostToDevice, st) != cudaSuccess) return fail(ctx, GEOAC_ERR_CUDA, "offset upload");
-        compact_rows_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(d_dense, d_rows, d_offs, n_rays, cap, nf, d_out);
-        if (cudaMemcpyAsync(out, d_out, sizeof(double) * total * nf, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
-            return fail(ctx, GEOAC_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(cudaGetLastError()));
-        return GEOAC_OK;
-    };
-    if (path_stride > 0) { rc = compact(ctx->d_path_rows, ctx->d_path, path_cap, GEOAC_PATH_NF, path_total_cap, path, path_offset, "raypath rows"); if (rc) { cleanup(); return rc; } }
-    if (caustic_cap > 0) { rc = compact(ctx->d_caus_rows, ctx->d_caus, caustic_cap, GEOAC_CAUSTIC_NF, caustic_total_cap, caustic, caustic_offset, "caustic rows"); if (rc) { cleanup(); return rc; } }
-    unsigned long long cnt[2] = { 0, 0 };
-    cudaMemcpyAsync(cnt, ctx->d_counters, sizeof cnt, cudaMemcpyDeviceToHost, st);
-    cudaStreamSynchronize(st);
-    cleanup();
-    float ms = 0.f; cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    ctx->last_ms = ms; ctx->last_steps = (int64_t)cnt[1];
-    return GEOAC_OK;
+    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, Capture::compact, path_stride,
+                      { path_cap, path, nullptr, path_offset, path_total_cap }, { caustic_cap, caustic, nullptr, caustic_offset, caustic_total_cap });
 }
 
 // Scheduling facts of the last trace (range-dependent sets): out[0] reserved (0), out[1] packets in the long region, out[2] CTAs
@@ -950,9 +895,9 @@ extern "C" int geoac_last_schedule(geoac_ctx* ctx, int64_t* out8) {
 // claim order was built.
 extern "C" int geoac_get_costs(geoac_ctx* ctx, int64_t n, uint32_t* cost) {
     if (!ctx || !cost || n < 0) return GEOAC_ERR_BAD_ARG;
-    if (!ctx->d_cost || (size_t)n * sizeof(uint32_t) > ctx->cap_cost) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_get_costs: no claim order of that size was built");
+    if (!ctx->d_cost.p || (size_t)n * sizeof(uint32_t) > ctx->d_cost.cap) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_get_costs: no claim order of that size was built");
     cudaSetDevice(ctx->device);
-    CK(cudaMemcpy(cost, ctx->d_cost, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(cost, ctx->d_cost.p, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost));
     return GEOAC_OK;
 }
 
@@ -978,14 +923,6 @@ extern "C" int geoac_last_launch_ms(geoac_ctx* ctx, double* ms2) {
 // records back at the rays' places in the caller's arrays.  No collective, no exchange between devices; the merged result
 // is bitwise what one context yields (tests/test_gpu_parity.py).
 // ---------------------------------------------------------------------------------------------------------------
-static int pin_grow(geoac_ctx* ctx, geoac_ctx::Pin& b, size_t need) {
-    if (need <= b.cap) return GEOAC_OK;
-    cudaFreeHost(b.p); b.p = nullptr; b.cap = 0;
-    CK(cudaHostAlloc(&b.p, need, cudaHostAllocDefault));
-    b.cap = need;
-    return GEOAC_OK;
-}
-
 extern "C" int geoac_create_multi(int variant, const int* device_ids, int n_devices, geoac_ctx** ctxs, int* status) {
     if (!device_ids || !ctxs || n_devices < 1) { if (status) *status = GEOAC_ERR_BAD_ARG; g_create_error = "geoac_create_multi: need device ordinals and room for the contexts"; return GEOAC_ERR_BAD_ARG; }
     for (int i = 0; i < n_devices; i++) {
@@ -1026,10 +963,6 @@ extern "C" int geoac_multi_set_params(geoac_ctx* const* ctxs, int n_ctx, const g
     return for_each_ctx(ctxs, n_ctx, [&](geoac_ctx* c, int) { return geoac_set_params(c, p); });
 }
 
-static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
-                      double* rec, int32_t* status, int32_t* n_steps, int path_stride, int64_t path_cap, double* path, int32_t* path_rows,
-                      int64_t caus_cap, double* caus, int32_t* caus_rows);
-
 extern "C" int geoac_trace_multi(geoac_ctx* const* ctxs, int n_ctx, int64_t n_rays, const double* theta, const double* phi,
                                  double* rec, int32_t* status, int32_t* n_steps) {
     if (!ctxs || n_ctx < 1 || n_rays < 0) return GEOAC_ERR_BAD_ARG;
@@ -1041,26 +974,24 @@ extern "C" int geoac_trace_multi(geoac_ctx* const* ctxs, int n_ctx, int64_t n_ra
     if (n_rays == 0) return GEOAC_OK;
     const int n_rec = ctxs[0]->prm.bounces + 1;
     const int64_t B = GEOAC_SHARD_BLOCK, n_blocks = (n_rays + B - 1) / B, n_slots = n_rays * n_rec;
-    return for_each_ctx(ctxs, n_ctx, [&](geoac_ctx* c, int r) -> int {
-        cudaSetDevice(c->device);
+    return for_each_ctx(ctxs, n_ctx, [&](geoac_ctx* ctx, int r) -> int {
+        cudaSetDevice(ctx->device);
         int64_t mine = 0;                                                       // rays of the blocks b = r, r + n_ctx, r + 2 n_ctx, ...
         for (int64_t b = r; b < n_blocks; b += n_ctx) mine += std::min(B, n_rays - b * B);
         if (mine == 0) return GEOAC_OK;
         const int64_t my_slots = mine * n_rec;
-        int g = pin_grow(c, c->pin_theta, sizeof(double) * mine); if (g) return g;
-        g = pin_grow(c, c->pin_phi, sizeof(double) * mine); if (g) return g;
-        g = pin_grow(c, c->pin_rec, sizeof(double) * GEOAC_NFIELDS * my_slots); if (g) return g;
-        g = pin_grow(c, c->pin_status, sizeof(int32_t) * my_slots); if (g) return g;
-        g = pin_grow(c, c->pin_nsteps, sizeof(int32_t) * my_slots); if (g) return g;
-        double *h_th = (double*)c->pin_theta.p, *h_ph = (double*)c->pin_phi.p, *h_rec = (double*)c->pin_rec.p;
-        int32_t *h_st = (int32_t*)c->pin_status.p, *h_ns = (int32_t*)c->pin_nsteps.p;
+        CK(ctx->pin_theta.grow(sizeof(double) * mine)); CK(ctx->pin_phi.grow(sizeof(double) * mine));
+        CK(ctx->pin_rec.grow(sizeof(double) * GEOAC_NFIELDS * my_slots));
+        CK(ctx->pin_status.grow(sizeof(int32_t) * my_slots)); CK(ctx->pin_nsteps.grow(sizeof(int32_t) * my_slots));
+        double *h_th = ctx->pin_theta.p, *h_ph = ctx->pin_phi.p, *h_rec = ctx->pin_rec.p;
+        int32_t *h_st = ctx->pin_status.p, *h_ns = ctx->pin_nsteps.p;
         int64_t at = 0;
         for (int64_t b = r; b < n_blocks; b += n_ctx) {
             const int64_t s0 = b * B, len = std::min(B, n_rays - s0);
             std::memcpy(h_th + at, theta + s0, sizeof(double) * len); std::memcpy(h_ph + at, phi + s0, sizeof(double) * len);
             at += len;
         }
-        const int rc = trace_host(c, mine, h_th, h_ph, h_rec, h_st, h_ns, 0, 0, nullptr, nullptr, 0, nullptr, nullptr);
+        const int rc = trace_host(ctx, mine, h_th, h_ph, h_rec, h_st, h_ns);
         if (rc != GEOAC_OK) return rc;
         at = 0;
         for (int64_t b = r; b < n_blocks; b += n_ctx) {                          // merge by ray index
@@ -1083,7 +1014,7 @@ extern "C" int geoac_source_state(geoac_ctx* ctx, double* out4) {
     cudaSetDevice(ctx->device);
     int rc = refresh_consts(ctx); if (rc != GEOAC_OK) return rc;
     LaunchConsts L;
-    CK(cudaMemcpyAsync(&L, ctx->d_consts, sizeof L, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&L, ctx->d_consts.p, sizeof L, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     out4[0] = L.c_src; out4[1] = L.u_src; out4[2] = L.v_src; out4[3] = L.rho_src;
     return GEOAC_OK;
@@ -1093,7 +1024,7 @@ extern "C" int geoac_last_trace_stats(geoac_ctx* ctx, int64_t* total_steps, doub
     if (!ctx) return GEOAC_ERR_BAD_ARG;
     cudaSetDevice(ctx->device);
     unsigned long long cnt[2] = { 0, 0 };
-    CK(cudaMemcpy(cnt, ctx->d_counters, sizeof cnt, cudaMemcpyDeviceToHost));   // also valid after geoac_trace_device + sync
+    CK(cudaMemcpy(cnt, ctx->d_counters.p, sizeof cnt, cudaMemcpyDeviceToHost));   // also valid after geoac_trace_device + sync
     ctx->last_steps = (int64_t)cnt[1];
     if (total_steps) *total_steps = ctx->last_steps;
     if (kernel_ms) *kernel_ms = ctx->last_ms;
@@ -1104,7 +1035,7 @@ extern "C" int geoac_last_trace_counters(geoac_ctx* ctx, int64_t* warp_trips, in
     if (!ctx) return GEOAC_ERR_BAD_ARG;
     cudaSetDevice(ctx->device);
     unsigned long long t = 0;
-    CK(cudaMemcpy(&t, ctx->d_counters + 2, sizeof t, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&t, ctx->d_counters.p + 2, sizeof t, cudaMemcpyDeviceToHost));
     if (warp_trips) *warp_trips = (int64_t)t;
     if (kernel_launches) *kernel_launches = ctx->last_launches;
     return GEOAC_OK;
@@ -1238,14 +1169,13 @@ __global__ void selftest_math_kernel(int n, unsigned long long* worst) {        
 extern "C" int geoac_selftest_math(geoac_ctx* ctx, int n_per_thread, double* max_rel_err) {
     if (!ctx || !max_rel_err || n_per_thread <= 0) return GEOAC_ERR_BAD_ARG;
     cudaSetDevice(ctx->device);
-    unsigned long long* d = nullptr;
-    CK(cudaMalloc(&d, 7 * sizeof(unsigned long long)));
-    CK(cudaMemset(d, 0, 7 * sizeof(unsigned long long)));
-    selftest_math_kernel<<<ctx->sm_count, 256, 0, ctx->stream>>>(n_per_thread, d);
+    Buf<unsigned long long> d;
+    CK(d.grow(7 * sizeof(unsigned long long)));
+    CK(cudaMemset(d.p, 0, 7 * sizeof(unsigned long long)));
+    selftest_math_kernel<<<ctx->sm_count, 256, 0, ctx->stream>>>(n_per_thread, d.p);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(ctx->stream));
-    CK(cudaMemcpy(max_rel_err, d, 7 * sizeof(double), cudaMemcpyDeviceToHost));
-    cudaFree(d);
+    CK(cudaMemcpy(max_rel_err, d.p, 7 * sizeof(double), cudaMemcpyDeviceToHost));
     return GEOAC_OK;
 }
 
@@ -1267,18 +1197,17 @@ extern "C" double geoac_measure_fp64_peak(geoac_ctx* ctx, double* out_ms) {
     if (!ctx) return -1.0;
     cudaSetDevice(ctx->device);
     const int block = 512, grid = ctx->sm_count * 4, iters = 4096;
-    double* d = nullptr;
-    if (cudaMalloc(&d, sizeof(double) * block * grid) != cudaSuccess) return -1.0;
+    Buf<double> d;
+    if (d.grow(sizeof(double) * block * grid) != cudaSuccess) return -1.0;
     float best = 1e30f;
     for (int rep = 0; rep < 5; rep++) {
         cudaEventRecord(ctx->ev0, ctx->stream);
-        dfma_peak_kernel<<<grid, block, 0, ctx->stream>>>(d, iters, 0.999999, 1e-7);
+        dfma_peak_kernel<<<grid, block, 0, ctx->stream>>>(d.p, iters, 0.999999, 1e-7);
         cudaEventRecord(ctx->ev1, ctx->stream);
         cudaStreamSynchronize(ctx->stream);
         float ms = 0; cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
         if (rep > 0 && ms < best) best = ms;
     }
-    cudaFree(d);
     if (out_ms) *out_ms = best;
     const double flops = 2.0 * 64.0 * (double)iters * (double)block * (double)grid;
     return flops / (best * 1e-3) / 1e12;

@@ -116,6 +116,20 @@ def test_synthetic_grids_match_their_node_files(built_lib, tmp_path):
                 assert np.allclose(a, b, rtol=0.0, atol=atol[nm]), (nm, float(np.abs(a - b).max()))
 
 
+def test_trace_entry_points_refuse_a_null_context(built_lib):
+    """geoac_trace, geoac_trace_paths(_compact), geoac_reserve and geoac_trace_multi return GEOAC_ERR_BAD_ARG for a NULL
+    context (or a NULL entry of the context list) before any device call."""
+    L, bad = api.lib(), abi.GEOAC_ERR_BAD_ARG
+    x, s, o = np.zeros(64), np.zeros(64, np.int32), np.zeros(2, np.int64)
+    d, i, l = (a.ctypes.data_as(C.POINTER(t)) for a, t in ((x, C.c_double), (s, C.c_int32), (o, C.c_int64)))
+    assert L.geoac_trace(None, 1, d, d, d, i, i) == bad
+    assert L.geoac_trace_paths(None, 1, d, d, d, i, i, 25, 4, d, i, 2, d, i) == bad
+    assert L.geoac_trace_paths_compact(None, 1, d, d, d, i, i, 25, 4, 4, d, l, 2, 2, d, l) == bad
+    assert L.geoac_reserve(None, 1) == bad
+    assert L.geoac_trace_multi(None, 1, 1, d, d, d, i, i) == bad
+    assert L.geoac_trace_multi((C.c_void_p * 2)(), 2, 1, d, d, d, i, i) == bad
+
+
 def test_pinned_host_allocation_binding(built_lib):
     """geoac_host_alloc / geoac_host_free: NULL (and a GeoAcError from the wrapper) without a device, a usable buffer with one."""
     p = api.lib().geoac_host_alloc(4096)
