@@ -14,6 +14,12 @@ CAUSTIC_NF = 6         # doubles per caustic event row: state[0..2], travel time
 PATH_NF = 8            # doubles per raypath row (geoac_trace_paths): state[0..2], amplitude, absorption, travel time, bounce, step
 ST_NONE, ST_ARRIVAL, ST_BREAK, ST_LIMIT = range(4)
 
+# geoac_sample_atmosphere: rows of out[field][point]
+ATM_C, ATM_U, ATM_V, ATM_RHO, ATM_DC, ATM_DU, ATM_DV, ATM_ALPHA = range(8)
+ATM_T, ATM_UF, ATM_VF = 8, 18, 28     # each 10 rows: f, d0, d1, d2, d00, d11, d22, d01, d02, d12 over (p0, p1, p2)
+ATM_NF = 38
+SAMPLE_BLOCK = 1 << 20                # points per device pass
+
 
 class GeoacParams(C.Structure):
     _fields_ = [

@@ -71,6 +71,7 @@ def lib():
         L.geoac_eigenray_direct.argtypes = [C.c_void_p, C.POINTER(abi.GeoacEigOpts), C.c_int, _dp, _dp, _dp, C.POINTER(C.c_int64)]
         L.geoac_get_variant.argtypes = [C.c_void_p]
         L.geoac_source_state.argtypes = [C.c_void_p, _dp]
+        L.geoac_sample_atmosphere.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp]
         L.geoac_set_knob.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
         L.geoac_last_schedule.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
         L.geoac_last_launch_ms.argtypes = [C.c_void_p, _dp]
@@ -92,6 +93,7 @@ EXPORTED_SYMBOLS = [
     "geoac_set_atmosphere_3d", "geoac_get_params", "geoac_set_params", "geoac_trace", "geoac_trace_paths", "geoac_trace_device",
     "geoac_reserve", "geoac_last_trace_stats", "geoac_last_trace_counters", "geoac_selftest_math", "geoac_load_met_1d", "geoac_load_met_grid", "geoac_eq_count", "geoac_measure_fp64_peak",
     "geoac_get_grid_tables", "geoac_default_eig_opts", "geoac_eigenray_search", "geoac_eigenray_direct", "geoac_get_variant", "geoac_source_state",
+    "geoac_sample_atmosphere",
     "geoac_set_knob", "geoac_last_schedule", "geoac_last_launch_ms", "geoac_trace_paths_compact", "geoac_get_costs",
     "geoac_host_alloc", "geoac_host_free",
     "geoac_create_multi", "geoac_multi_set_atmosphere_1d", "geoac_multi_set_atmosphere_3d", "geoac_multi_set_params", "geoac_trace_multi",
@@ -258,6 +260,17 @@ class Tracer:
         """c, u, v, rho at the source point as the kernels sample them."""
         out = np.zeros(4)
         self._check(lib().geoac_source_state(self._h, _p(out)), "geoac_source_state")
+        return out
+
+    def sample_atmosphere(self, p0, p1, p2):
+        """The atmosphere as the kernels evaluate it at n points in the variant's coordinates ((x, y, z) [km], or Global
+        (r [km from the Earth's centre], lat [rad], lon [rad])): array [ATM_NF, n] (rows: abi.ATM_*)."""
+        pts = [np.ascontiguousarray(a, dtype=np.float64) for a in (p0, p1, p2)]
+        if any(a.ndim != 1 or a.shape != pts[0].shape for a in pts):
+            raise GeoAcError("sample_atmosphere: p0, p1, p2 must be 1-D arrays of one length")
+        n = len(pts[0])
+        out = np.empty((abi.ATM_NF, n))
+        self._check(lib().geoac_sample_atmosphere(self._h, n, *[_p(a) for a in pts], _p(out)), "geoac_sample_atmosphere")
         return out
 
     def grid_tables(self, n0, n1, nz):

@@ -22,6 +22,7 @@
 #include "eq_global.cuh"
 #include "eq_rngdep.cuh"
 #include "trace_kernel.cuh"
+#include "atmo_sample.cuh"
 #include "host_tables.hpp"
 
 using namespace geoac;
@@ -131,6 +132,8 @@ struct geoac_ctx {
     // pinned host staging of geoac_trace_multi (this context's share of the batch: angles in, records out)
     Buf<double, true> pin_theta, pin_phi, pin_rec;
     Buf<int32_t, true> pin_status, pin_nsteps;
+    // staging of geoac_sample_atmosphere: the three coordinates in, GEOAC_ATM_NF rows out, one pass of points at a time
+    Buf<double> d_smp_in, d_smp_out;
 };
 
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
@@ -1017,6 +1020,60 @@ extern "C" int geoac_source_state(geoac_ctx* ctx, double* out4) {
     CK(cudaMemcpyAsync(&L, ctx->d_consts.p, sizeof L, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     out4[0] = L.c_src; out4[1] = L.u_src; out4[2] = L.v_src; out4[3] = L.rho_src;
+    return GEOAC_OK;
+}
+
+// ---- the atmosphere at arbitrary points (atmo_sample.cuh): one thread per point, coordinates and rows SoA ----
+enum { SMP_1D = 0, SMP_1D_GLOBAL = 1, SMP_GRID = 2, SMP_GRID_GLOBAL = 3 };
+template <int KIND>
+__global__ void __launch_bounds__(128) sample_atmosphere_kernel(const LaunchConsts* __restrict__ Lc, const Table1D T, const Grid3D g, int64_t n,
+                                                                const double* __restrict__ p, double* __restrict__ out) {
+    const LaunchConsts& L = *Lc;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const double p0 = p[i], p1 = p[n + i], p2 = p[2 * n + i];
+        if constexpr (KIND == SMP_1D) sample_point_1d<false>(L, T, p0, p2, out + i, n);
+        else if constexpr (KIND == SMP_1D_GLOBAL) sample_point_1d<true>(L, T, p0, p2, out + i, n);
+        else if constexpr (KIND == SMP_GRID) sample_point_grid<false>(L, g, p0, p1, p2, out + i, n);
+        else sample_point_grid<true>(L, g, p0, p1, p2, out + i, n);
+    }
+}
+
+extern "C" int geoac_sample_atmosphere(geoac_ctx* ctx, int64_t n, const double* p0, const double* p1, const double* p2, double* out) {
+    if (!ctx) return GEOAC_ERR_BAD_ARG;
+    if (n < 0) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_sample_atmosphere: n < 0");
+    if (n > 0 && (!p0 || !p1 || !p2 || !out)) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_sample_atmosphere: null buffer");
+    for (int64_t i = 0; i < n; i++)
+        if (!std::isfinite(p0[i]) || !std::isfinite(p1[i]) || !std::isfinite(p2[i]))
+            return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_sample_atmosphere: coordinates of point " + std::to_string(i) + " are not finite");
+    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");
+    if (n == 0) return GEOAC_OK;
+    cudaSetDevice(ctx->device);
+    if (int rc = refresh_consts(ctx)) return rc;                       // L.sb and the absorption parameters; no trace state is touched
+    const int64_t B = std::min<int64_t>(n, GEOAC_SAMPLE_BLOCK);
+    CK(ctx->d_smp_in.grow(sizeof(double) * 3 * B));
+    CK(ctx->d_smp_out.grow(sizeof(double) * GEOAC_ATM_NF * B));
+    const cudaStream_t st = ctx->stream;
+    Table1D T{}; T.base = ctx->d_table.p; T.n = ctx->n; T.xmin = ctx->xmin; T.xmax = ctx->xmax; T.jump_scale = 0.0; T.sbpoly = nullptr;
+    const int kind = ctx->is_grid ? (ctx->variant == GEOAC_GLOBAL_RNGDEP ? SMP_GRID_GLOBAL : SMP_GRID)
+                                  : (ctx->variant == GEOAC_GLOBAL ? SMP_1D_GLOBAL : SMP_1D);
+    for (int64_t s0 = 0; s0 < n; s0 += B) {
+        const int64_t m = std::min(B, n - s0);
+        double *in = ctx->d_smp_in.p, *res = ctx->d_smp_out.p;
+        CK(cudaMemcpyAsync(in, p0 + s0, sizeof(double) * m, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(in + m, p1 + s0, sizeof(double) * m, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(in + 2 * m, p2 + s0, sizeof(double) * m, cudaMemcpyHostToDevice, st));
+        const int grid = (int)std::min<int64_t>((m + 127) / 128, (int64_t)ctx->sm_count * 16);
+        switch (kind) {
+            case SMP_1D:          sample_atmosphere_kernel<SMP_1D><<<grid, 128, 0, st>>>(ctx->d_consts.p, T, ctx->grid, m, in, res); break;
+            case SMP_1D_GLOBAL:   sample_atmosphere_kernel<SMP_1D_GLOBAL><<<grid, 128, 0, st>>>(ctx->d_consts.p, T, ctx->grid, m, in, res); break;
+            case SMP_GRID:        sample_atmosphere_kernel<SMP_GRID><<<grid, 128, 0, st>>>(ctx->d_consts.p, T, ctx->grid, m, in, res); break;
+            default:              sample_atmosphere_kernel<SMP_GRID_GLOBAL><<<grid, 128, 0, st>>>(ctx->d_consts.p, T, ctx->grid, m, in, res); break;
+        }
+        CK(cudaGetLastError());
+        for (int f = 0; f < GEOAC_ATM_NF; f++)
+            CK(cudaMemcpyAsync(out + (int64_t)f * n + s0, res + (int64_t)f * m, sizeof(double) * m, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
     return GEOAC_OK;
 }
 

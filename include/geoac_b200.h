@@ -70,6 +70,26 @@ enum {
     GEOAC_CAUSTIC_NF   = 6
 };
 
+/* ---- atmosphere sample fields (geoac_sample_atmosphere): out[field * n + i] ---- */
+enum {
+    GEOAC_ATM_C     = 0,       /* c() [km/s] = sqrt(gamR T)                                                               */
+    GEOAC_ATM_U     = 1,       /* u() [km/s]                                                                              */
+    GEOAC_ATM_V     = 2,       /* v() [km/s]                                                                              */
+    GEOAC_ATM_RHO   = 3,       /* rho() [g/cm^3]                                                                          */
+    GEOAC_ATM_DC    = 4,       /* c_diff / u_diff / v_diff along the vertical coordinate (z Cartesian, r Global)          */
+    GEOAC_ATM_DU    = 5,
+    GEOAC_ATM_DV    = 6,
+    GEOAC_ATM_ALPHA = 7,       /* SuthBass_Alpha [dB/km] (x tweak_abs), full model                                       */
+    GEOAC_ATM_T     = 8,       /* 8..17: T and its derivatives over (p0, p1, p2): f, d0, d1, d2, d00, d11, d22, d01, d02, d12,
+                                  as the right-hand side sees them (Eval_Spline_AllOrder2 on the grids, slips of SURVEY
+                                  App. A-8 / A-9 included; the vertical spline's f, f', f'' for stratified atmospheres)   */
+    GEOAC_ATM_UF    = 18,      /* 18..27: u, the same 10 entries                                                         */
+    GEOAC_ATM_VF    = 28,      /* 28..37: v, the same 10 entries                                                         */
+    GEOAC_ATM_NF    = 38
+};
+/* points per device pass of geoac_sample_atmosphere (bounds its device memory at 41 doubles per point of a pass) */
+enum { GEOAC_SAMPLE_BLOCK = 1 << 20 };
+
 /* per-slot status */
 enum {
     GEOAC_ST_NONE    = 0,      /* ray ended before this bounce                                     */
@@ -282,6 +302,20 @@ int geoac_eigenray_direct(geoac_ctx* ctx, const geoac_eig_opts* opts, int n, con
 /* Variant the context was created for; c, u, v, rho at the source point (device-sampled), 4 doubles. */
 int geoac_get_variant(const geoac_ctx* ctx);
 int geoac_source_state(geoac_ctx* ctx, double* out4);
+
+/* Atmosphere as the kernels evaluate it, at n points given in the variant's own coordinates (the reference's Atmo_State.h
+ * argument order): 2D / 3D / 3D.RngDep (x, y, z) [km]; Global / Global.RngDep (r [km from the Earth's centre, i.e.
+ * r_earth + altitude], lat [rad], lon [rad]).  Stratified atmospheres use only the vertical coordinate.  Coordinates outside
+ * the table / grid are clamped exactly as every reference look-up clamps them.  out: GEOAC_ATM_NF * n doubles, SoA,
+ * out[f * n + i].  Absorption uses the context's params (freq, tweak_abs, z_grnd).  Synchronous, on ctx's stream; the same
+ * concurrency contract as the trace calls.  Does not change anything a later trace reads or reports.
+ * Replaces, as callers see them, c/u/v/rho, c_diff/u_diff/v_diff along the vertical, SuthBass_Alpha and Eval_Spline_AllOrder2
+ * (Code/Atmo/Atmo_State.h:11-36).  Every point is evaluated as the reference would with cold cursors (accel = 0): a point
+ * exactly on knot m falls in interval m-1 in the lower half of an axis and in interval m in the upper half.
+ * Errors: GEOAC_ERR_BAD_ARG (NULL context, n < 0, a NULL pointer with n > 0, a non-finite coordinate -- the message names
+ * the first such index), GEOAC_ERR_NO_ATMO; n == 0 writes nothing.  Points go through the device in passes of
+ * GEOAC_SAMPLE_BLOCK. */
+int geoac_sample_atmosphere(geoac_ctx* ctx, int64_t n, const double* p0, const double* p1, const double* p2, double* out);
 
 /* Number of state equations for (variant, calc_amp): GeoAc_SetEqCnt, Code/GeoAc/GeoAc.Interface.cpp:21-41. */
 int geoac_eq_count(int variant, int calc_amp);
