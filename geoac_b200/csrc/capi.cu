@@ -40,7 +40,7 @@ struct Knobs {
     int host_tables = 0;    // build the node tables on the host
     int long_alpha = 100;   // a packet is LONG if its cost exceeds long_alpha % of the average work of a lane
     int long_sm_pct = 90;   // at most this share of the SMs is given to the long-region launch (its CTAs help with the main region once theirs is drained)
-    int exclusive = 1;      // long-region launch keeps its SMs to itself (0: one launch, long packets first)
+    int exclusive = 1;      // long-region launch keeps its SMs to itself (0: one launch, which claims the main region first)
     int dilate = 400;       // range-dependent sets: the ordering cost of a ray is the maximum over its inclination neighbours within this many
                             // millidegrees (0 = off): the edge of a long ray family is scheduled as long
     int quarter = 1;        // the longest long-region packets are claimed as quarter packets while the exclusive SMs have warps to spare
@@ -124,9 +124,11 @@ struct geoac_ctx {
     Buf<int32_t> d_status, d_nsteps;
     cudaStream_t stream = nullptr, stream_long = nullptr;      // stream_long: the concurrent long-region launch of the range-dependent sets
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_fork = nullptr, ev_join = nullptr, ev_m0 = nullptr, ev_m1 = nullptr, ev_l0 = nullptr, ev_l1 = nullptr;
+    cudaEvent_t ev_d0 = nullptr, ev_d1 = nullptr;                // the work of the last geoac_trace_device on the caller's stream
     bool timed_launches = false;
     int last_long_packets = 0, last_long_ctas = 0, last_quarter_packets = 0;
     int64_t last_steps = 0; double last_ms = 0.0;
+    bool ms_pending = false;                                    // last_ms is still to be read from ev_d0 / ev_d1
     bool consts_dirty = true;
     bool src_set = false;
     // pinned host staging of geoac_trace_multi (this context's share of the batch: angles in, records out)
@@ -185,6 +187,7 @@ extern "C" geoac_ctx* geoac_create(int variant, int device, int* status) {
            && cudaEventCreate(&ctx->ev0) == cudaSuccess && cudaEventCreate(&ctx->ev1) == cudaSuccess
            && cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming) == cudaSuccess
            && cudaEventCreate(&ctx->ev_m0) == cudaSuccess && cudaEventCreate(&ctx->ev_m1) == cudaSuccess && cudaEventCreate(&ctx->ev_l0) == cudaSuccess && cudaEventCreate(&ctx->ev_l1) == cudaSuccess
+           && cudaEventCreate(&ctx->ev_d0) == cudaSuccess && cudaEventCreate(&ctx->ev_d1) == cudaSuccess
            && ctx->d_consts.grow(sizeof(LaunchConsts)) == cudaSuccess
            && ctx->d_counters.grow(8 * sizeof(unsigned long long)) == cudaSuccess;
     if (!ok) { std::string m = cudaGetErrorString(cudaGetLastError()); delete ctx; return bail(GEOAC_ERR_CUDA, "context allocation failed: " + m); }
@@ -201,6 +204,8 @@ extern "C" void geoac_destroy(geoac_ctx* ctx) {
     if (ctx->ev_m1) cudaEventDestroy(ctx->ev_m1);
     if (ctx->ev_l0) cudaEventDestroy(ctx->ev_l0);
     if (ctx->ev_l1) cudaEventDestroy(ctx->ev_l1);
+    if (ctx->ev_d0) cudaEventDestroy(ctx->ev_d0);
+    if (ctx->ev_d1) cudaEventDestroy(ctx->ev_d1);
     if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
     if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
     if (ctx->stream_long) cudaStreamDestroy(ctx->stream_long);
@@ -594,8 +599,9 @@ static int build_claim_order(geoac_ctx* ctx, TraceArgs& a, long long lanes, int 
     return GEOAC_OK;
 }
 
-// Step 2: CTAs of the exclusive long-region launch (0 = none: the main launch drains the long region first).  Sets
-// a.n_quarter_packets.  The capture kernels always run as one launch.
+// Step 2: CTAs of the exclusive long-region launch (0 = none: one launch, whose warps claim the main region first, then the
+// long region, then the quarter packets -- trace_kernel.cuh).  Sets a.n_quarter_packets.  The capture kernels always run as
+// one launch.
 static int size_long_region(const geoac_ctx* ctx, TraceArgs& a, int64_t n_quarter, int block, bool paths) {
     if (a.n_long_packets == 0 || !ctx->knobs.exclusive || paths) return 0;
     const int64_t max_ctas = std::max<int64_t>(1, (int64_t)ctx->sm_count * ctx->knobs.long_sm_pct / 100);
@@ -729,8 +735,11 @@ static int enqueue_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
 
 extern "C" int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, const double* d_phi,
                                   double* d_rec, int32_t* d_status, int32_t* d_n_steps, void* cuda_stream) {
-    if (!ctx || n_rays < 0) return GEOAC_ERR_BAD_ARG;
+    if (!ctx) return GEOAC_ERR_BAD_ARG;
+    if (n_rays < 0) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_device: n_rays < 0");
     if (n_rays == 0) return GEOAC_OK;
+    if (!d_theta || !d_phi || !d_rec || !d_status || !d_n_steps) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_device: null buffer");
+    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");
     cudaSetDevice(ctx->device);
     if (int rc = refresh_consts(ctx)) return rc;
     const cudaStream_t st = (cudaStream_t)cuda_stream;
@@ -740,7 +749,12 @@ extern "C" int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* 
     }
     TraceArgs a{};
     a.theta = d_theta; a.phi = d_phi; a.n_rays = n_rays; a.rec = d_rec; a.status = d_status; a.n_steps = d_n_steps;
-    return enqueue_trace(ctx, a, st);
+    ctx->last_ms = std::numeric_limits<double>::quiet_NaN(); ctx->ms_pending = false;
+    CK(cudaEventRecord(ctx->ev_d0, st));
+    if (int rc = enqueue_trace(ctx, a, st)) return rc;
+    CK(cudaEventRecord(ctx->ev_d1, st));
+    ctx->ms_pending = true;                                 // read by geoac_last_trace_stats once the stream has got there
+    return GEOAC_OK;
 }
 
 // device staging of the host-buffer entry point (angles in, records out), grown on demand and kept across calls
@@ -860,7 +874,7 @@ static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const
     CK(cudaMemcpyAsync(cnt, ctx->d_counters.p, sizeof cnt, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     float ms = 0.f; cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    ctx->last_ms = ms; ctx->last_steps = (int64_t)cnt[1];
+    ctx->last_ms = ms; ctx->ms_pending = false; ctx->last_steps = (int64_t)cnt[1];
     return GEOAC_OK;
 }
 
@@ -1083,6 +1097,11 @@ extern "C" int geoac_last_trace_stats(geoac_ctx* ctx, int64_t* total_steps, doub
     unsigned long long cnt[2] = { 0, 0 };
     CK(cudaMemcpy(cnt, ctx->d_counters.p, sizeof cnt, cudaMemcpyDeviceToHost));   // also valid after geoac_trace_device + sync
     ctx->last_steps = (int64_t)cnt[1];
+    if (ctx->ms_pending) {                                  // geoac_trace_device: NaN until its work on the caller's stream has completed
+        float ms = 0.f;
+        if (cudaEventElapsedTime(&ms, ctx->ev_d0, ctx->ev_d1) == cudaSuccess) { ctx->last_ms = ms; ctx->ms_pending = false; }
+        else cudaGetLastError();
+    }
     if (total_steps) *total_steps = ctx->last_steps;
     if (kernel_ms) *kernel_ms = ctx->last_ms;
     return GEOAC_OK;

@@ -130,7 +130,8 @@ typedef struct geoac_ctx geoac_ctx;
  * y_{k-1} history) that every trace reuses, so AT MOST ONE trace may be in flight per context, on ONE stream at a time:
  * calls on one context are serialised by the caller (the reference itself is single-threaded and non-reentrant,
  * Code/GeoAc/GeoAc.Parameters.h globals), and after geoac_trace_device the caller must synchronise the stream it passed
- * before the next call on that context (any entry point, geoac_set_params included).  Different contexts are
+ * before the next call on that context (any entry point, geoac_set_params included) other than another
+ * geoac_trace_device on the same stream.  Different contexts are
  * independent and may be driven from different host threads -- one context per device is how a front end uses
  * several GPUs (geoac_trace_multi below does exactly that). */
 geoac_ctx* geoac_create(int variant, int device, int* status);
@@ -166,7 +167,13 @@ int geoac_trace(geoac_ctx* ctx, int64_t n_rays, const double* theta, const doubl
                 double* rec, int32_t* status, int32_t* n_steps);
 
 /* Same, but every pointer is a DEVICE pointer on ctx's device and the work is enqueued on `cuda_stream`
- * (a cudaStream_t passed as void*, NULL = default stream); returns without synchronising. */
+ * (a cudaStream_t passed as void*, NULL = default stream); returns without synchronising.  The call zeroes every record
+ * slot before the trace, so the outputs need no initialisation.  Parameter and atmosphere changes made before the call are
+ * ordered into `cuda_stream` by the call itself.  Calls that follow one another on the SAME stream need no synchronisation
+ * between them (each one's work, the concurrent long-region launch of the range-dependent sets included, is complete
+ * before the next one's starts); any other call on the context waits for a synchronisation of that stream (geoac_create).
+ * Errors, returned before anything is enqueued: GEOAC_ERR_BAD_ARG (NULL context, n_rays < 0, a NULL pointer with
+ * n_rays > 0), GEOAC_ERR_NO_ATMO; n_rays == 0 enqueues nothing and is GEOAC_OK whatever the pointers. */
 int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, const double* d_phi,
                        double* d_rec, int32_t* d_status, int32_t* d_n_steps, void* cuda_stream);
 
@@ -231,7 +238,10 @@ void  geoac_host_free(void* p);
  * `bounces`) ahead of time, so that the first trace call does not pay for it.  geoac_trace() grows it on demand anyway. */
 int geoac_reserve(geoac_ctx* ctx, int64_t n_rays);
 
-/* Total RK4 steps of the last trace on this ctx (sum of n_steps), and milliseconds the kernel(s) took (CUDA events). */
+/* Total RK4 steps of the last trace on this ctx (sum of n_steps), and its duration in milliseconds (CUDA events).  After
+ * the host-buffer calls the duration covers the work between the angle upload and the record download.  After
+ * geoac_trace_device it covers the call's work on the caller's stream (zeroing, claim order, trace launches, join); both
+ * values are valid once that stream has been synchronised, and kernel_ms is NaN while the work has not completed. */
 int geoac_last_trace_stats(geoac_ctx* ctx, int64_t* total_steps, double* kernel_ms);
 
 /* Host helper mirroring Load_G2S (Code/Atmo/G2S_Spline1D.cpp:109-142): read a .met profile ("zTuvdp" or "zuvwTdp"),

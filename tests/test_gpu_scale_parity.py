@@ -6,7 +6,10 @@ the reference, tests/test_oracle_golden.py) on
   * config 4: 64 seeded rays on the FULL 200 x 200 x 300 node grid,
   * config 5: 64 seeded rays on the FULL 181 x 361 x 300 global grid (step limit lowered so ducted rays end on LIMIT),
 
-with the near-threshold listing (geoac_b200/nearthreshold.py) applied: discrete outputs bit-exact except on slots the
+with the near-threshold listing (geoac_b200/nearthreshold.py) applied; the same angles traced through geoac_trace_device (torch
+buffers, the default stream) with the claim order forced on must give bitwise the records held to the oracle, which carries the
+verdict over to the scheduled path the benchmark times -- the stratified sort and whole-warp refill, and for configs 4 and 5
+the long region, its exclusive launch and the quarter claims.  The parity bar is discrete outputs bit-exact except on slots the
 listing flags; ray position, eikonal, travel time, attenuation, turning height, inclination, back azimuth, celerity to
 1e-9 on every arrival; amplitude / Jacobian / auxiliary states to 1e-9 except where a 1e-10 rad change of the launch angle
 moves them by more than that (listed with |D|).  The oracle runs one process per host core (fork: the children share the
@@ -20,6 +23,7 @@ import pytest
 import geoac_b200 as g
 from geoac_b200 import abi, nearthreshold as nt
 from tests import util
+from tests.test_gpu_device_path import assert_bitwise, trace_device
 
 sys.path.insert(0, util.ROOT)
 import bench            # noqa: E402  (workload definitions only)
@@ -37,6 +41,19 @@ def _report(capsys, label, problems, listed, stats, n_disc, lines, n_arr):
             print("    flagged:", ln)
 
 
+def _scheduled_device_trace_equals(workload, p, th, ph, got):
+    tr, _ = bench.setup_tracer(workload, 0)
+    tr.params = p
+    tr.set_knob("lpt", 2)
+    dev = trace_device(tr, th, ph)
+    assert_bitwise(dev, got, f"{workload}: geoac_trace_device, claim order forced on")
+    assert tr.last_kernel_launches() > 1
+    if util.is_rngdep(bench.WORKLOADS[workload][0]):
+        s = tr.last_schedule()
+        assert s["long_packets"] > 0 and s["long_ctas"] > 0 and s["quarter_packets"] > 0, s
+    tr.close()
+
+
 def _run(workload, th_deg, ph_deg, th, ph, oracle, capsys, label, chunk, ray_limit=None):
     variant = bench.WORKLOADS[workload][0]
     tr, p = bench.setup_tracer(workload, 0)
@@ -45,6 +62,7 @@ def _run(workload, th_deg, ph_deg, th, ph, oracle, capsys, label, chunk, ray_lim
         tr.params = p
     p = tr.params
     got = tr.trace(th, ph)
+    _scheduled_device_trace_equals(workload, p, th, ph, got)
     cond = nt.conditioning(tr.trace, th, ph, got, variant, p.calc_amp)
     tainted, reasons = nt.margin_flags(got, variant, p)
     # oracle on the same inputs (atmosphere built once, before the fork)
