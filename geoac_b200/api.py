@@ -51,6 +51,7 @@ def lib():
         _lp = C.POINTER(C.c_int64)
         L.geoac_trace_paths_compact.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _ip, _ip, C.c_int, C.c_int64, C.c_int64, _dp, _lp,
                                                 C.c_int64, C.c_int64, _dp, _lp]
+        L.geoac_trace_sources.argtypes = [C.c_void_p, C.c_int, _dp, C.c_int64, _ip, _dp, _dp, _dp, _ip, _ip]
         L.geoac_trace_device.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.geoac_reserve.argtypes = [C.c_void_p, C.c_int64]
         L.geoac_host_alloc.restype = C.c_void_p
@@ -91,6 +92,7 @@ def lib():
 EXPORTED_SYMBOLS = [
     "geoac_create", "geoac_destroy", "geoac_last_error", "geoac_default_params", "geoac_set_atmosphere_1d",
     "geoac_set_atmosphere_3d", "geoac_get_params", "geoac_set_params", "geoac_trace", "geoac_trace_paths", "geoac_trace_device",
+    "geoac_trace_sources",
     "geoac_reserve", "geoac_last_trace_stats", "geoac_last_trace_counters", "geoac_selftest_math", "geoac_load_met_1d", "geoac_load_met_grid", "geoac_eq_count", "geoac_measure_fp64_peak",
     "geoac_get_grid_tables", "geoac_default_eig_opts", "geoac_eigenray_search", "geoac_eigenray_direct", "geoac_get_variant", "geoac_source_state",
     "geoac_sample_atmosphere",
@@ -289,14 +291,14 @@ class Tracer:
     def params(self, p):
         self._check(lib().geoac_set_params(self._h, C.byref(p)), "geoac_set_params")
 
-    def trace(self, theta, phi, out=None):
-        """Host buffers in, host buffers out (H2D + kernels + D2H inside). Returns dict(rec, status, n_steps)."""
+    def _rays_and_records(self, what, theta, phi, out):
+        """The angles as contiguous float64 arrays and the record buffers of a trace of them (`out`, checked, or new ones)."""
         theta = np.ascontiguousarray(theta, dtype=np.float64)
         phi = np.ascontiguousarray(phi, dtype=np.float64)
         n = len(theta)
         n_rec = self.params.bounces + 1
         if phi.shape != theta.shape or theta.ndim != 1:
-            raise GeoAcError("trace: theta and phi must be 1-D arrays of one length")
+            raise GeoAcError(f"{what}: theta and phi must be 1-D arrays of one length")
         if out is None:
             out = {"rec": np.empty((abi.NFIELDS, n, n_rec)), "status": np.empty((n, n_rec), dtype=np.int32),
                    "n_steps": np.empty((n, n_rec), dtype=np.int32)}
@@ -304,9 +306,31 @@ class Tracer:
             for k, dt, size in (("rec", np.float64, abi.NFIELDS * n * n_rec), ("status", np.int32, n * n_rec), ("n_steps", np.int32, n * n_rec)):
                 a = out[k]
                 if not (isinstance(a, np.ndarray) and a.dtype == dt and a.flags["C_CONTIGUOUS"] and a.flags["WRITEABLE"] and a.size == size):
-                    raise GeoAcError(f"trace: out['{k}'] must be a writeable C-contiguous {np.dtype(dt).name} array of {size} elements")
-        self._check(lib().geoac_trace(self._h, n, _p(theta), _p(phi), _p(out["rec"]), out["status"].ctypes.data_as(_ip),
+                    raise GeoAcError(f"{what}: out['{k}'] must be a writeable C-contiguous {np.dtype(dt).name} array of {size} elements")
+        return theta, phi, out
+
+    def trace(self, theta, phi, out=None):
+        """Host buffers in, host buffers out (H2D + kernels + D2H inside). Returns dict(rec, status, n_steps)."""
+        theta, phi, out = self._rays_and_records("trace", theta, phi, out)
+        self._check(lib().geoac_trace(self._h, len(theta), _p(theta), _p(phi), _p(out["rec"]), out["status"].ctypes.data_as(_ip),
                                       out["n_steps"].ctypes.data_as(_ip)), "geoac_trace")
+        return out
+
+    def trace_sources(self, src, src_id, theta, phi, out=None):
+        """trace() for rays from many sources in one call: ray r starts from src[src_id[r]].  src: [n_src, 3] in the
+        convention of params.src; src_id: int32 [n].  Ray r's records equal those of trace() with params.src = src[src_id[r]]
+        (include/geoac_b200.h: geoac_trace_sources).  Lay the batch out source by source."""
+        theta, phi, out = self._rays_and_records("trace_sources", theta, phi, out)
+        src = np.ascontiguousarray(src, dtype=np.float64)
+        if src.ndim != 2 or src.shape[1] != 3:
+            raise GeoAcError("trace_sources: src must be an array of shape [n_src, 3]")
+        src_id = np.asarray(src_id)
+        if src_id.dtype != np.int32 or src_id.shape != theta.shape:
+            raise GeoAcError("trace_sources: src_id must be an int32 array with one entry per ray")
+        src_id = np.ascontiguousarray(src_id)
+        self._check(lib().geoac_trace_sources(self._h, len(src), _p(src), len(theta), src_id.ctypes.data_as(_ip), _p(theta), _p(phi),
+                                              _p(out["rec"]), out["status"].ctypes.data_as(_ip), out["n_steps"].ctypes.data_as(_ip)),
+                    "geoac_trace_sources")
         return out
 
     def trace_paths(self, theta, phi, stride=25, cap=2400, caustic_cap=0):

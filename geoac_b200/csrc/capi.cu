@@ -136,6 +136,8 @@ struct geoac_ctx {
     Buf<int32_t, true> pin_status, pin_nsteps;
     // staging of geoac_sample_atmosphere: the three coordinates in, GEOAC_ATM_NF rows out, one pass of points at a time
     Buf<double> d_smp_in, d_smp_out;
+    // staging of geoac_trace_sources: the sources, each ray's source and the invariants of each source
+    Buf<double> d_src; Buf<int32_t> d_src_id; Buf<LaunchConsts> d_src_consts;
 };
 
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
@@ -455,13 +457,23 @@ extern "C" int geoac_get_grid_tables(geoac_ctx* ctx, int64_t cap_tuv, double* tu
 }
 
 // ---- per-launch invariants, computed on the device with the same spline routines the kernel uses ----
-__global__ void setup_consts_kernel(LaunchConsts* out, const LaunchConsts in, const double* table, int n,
+// The source a ray starts from: s as geoac_params.src gives it, with z_src = max(z_grnd, z_src) (altitude for Global).
+__host__ __device__ static void set_source(LaunchConsts& L, const double* s, int variant) {
+    for (int i = 0; i < 3; i++) L.src[i] = s[i];
+    const int k = (variant == GEOAC_2D || variant == GEOAC_3D || variant == GEOAC_3D_RNGDEP) ? 2 : 0;
+    L.src[k] = (L.z_grnd < s[k]) ? s[k] : L.z_grnd;
+}
+
+// One thread per source: out[i] = the invariants of `in` launched from src[i] (src == nullptr: from in.src, n_src = 1).
+__global__ void setup_consts_kernel(LaunchConsts* out, const LaunchConsts in, const double* src, int n_src, const double* table, int n,
                                     double xmin, double xmax, int variant) {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_src) return;
     Table1D T; T.base = table; T.n = n; T.xmin = xmin; T.xmax = xmax; T.jump_scale = 0.0;
     LaunchConsts L = in;
+    if (src) set_source(L, src + 3 * (size_t)i, variant);
     fill_launch_consts_1d(L, T, variant);
-    *out = L;
+    out[i] = L;
 }
 
 // per-interval absorption polynomials (core.cuh: sbpoly_build_interval), one thread per interval, after the invariants
@@ -474,35 +486,44 @@ __global__ void build_sbpoly_kernel(const LaunchConsts* Lc, const double* table,
     for (int i = 0; i < SBP_STRIDE; i++) out[(size_t)k * SBP_STRIDE + i] = o[i];
 }
 
-__global__ void setup_consts_grid_kernel(LaunchConsts* out, const LaunchConsts in, const Grid3D g, int variant) {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+__global__ void setup_consts_grid_kernel(LaunchConsts* out, const LaunchConsts in, const double* src, int n_src, const Grid3D g, int variant) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_src) return;
     LaunchConsts L = in;
+    if (src) set_source(L, src + 3 * (size_t)i, variant);
     fill_launch_consts_3d(L, g, variant);
-    *out = L;
+    out[i] = L;
 }
 
-static int refresh_consts(geoac_ctx* ctx) {
-    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");      // the set-up kernel samples the tables
-    if (!ctx->consts_dirty) return GEOAC_OK;
+// The invariants of the context's parameters launched from `src` (device, n_src rows of 3 doubles; nullptr: params.src),
+// one LaunchConsts per source into `out` on ctx->stream.
+static int setup_consts(geoac_ctx* ctx, LaunchConsts* out, const double* src, int n_src) {
     const geoac_params& p = ctx->prm;
     LaunchConsts L; std::memset(&L, 0, sizeof L);
     L.ds_min = p.ds_min; L.ds_max = p.ds_max; L.vert_limit = p.vert_limit; L.range_limit = p.range_limit;
     L.z_grnd = p.z_grnd; L.tweak_abs = p.tweak_abs; L.freq = p.freq;
     for (int i = 0; i < 2; i++) { L.box_min[i] = p.box_min[i]; L.box_max[i] = p.box_max[i]; }
-    for (int i = 0; i < 3; i++) L.src[i] = p.src[i];
-    if (ctx->variant == GEOAC_2D || ctx->variant == GEOAC_3D || ctx->variant == GEOAC_3D_RNGDEP) L.src[2] = std::max(p.z_grnd, p.src[2]);   // z_src = max(z_grnd, z_src)
-    else L.src[0] = std::max(p.z_grnd, p.src[0]);
+    set_source(L, p.src, ctx->variant);
     L.bounces = p.bounces; L.calc_amp = p.calc_amp;
     L.seg_mode = (ctx->variant == GEOAC_2D) ? 1 : (p.accum_per_segment ? 1 : 0);                          // App. A-2
     L.step_limit = (int)(p.ray_limit * (int)(1.0 / (p.ds_min * 10)));                                     // Solver.cpp:14
     L.per_bounce_zmax = (ctx->variant == GEOAC_3D_RNGDEP || ctx->variant == GEOAC_GLOBAL_RNGDEP);         // App. A-3
-    if (ctx->is_grid) setup_consts_grid_kernel<<<1, 32, 0, ctx->stream>>>(ctx->d_consts.p, L, ctx->grid, ctx->variant);
-    else {
-        setup_consts_kernel<<<1, 32, 0, ctx->stream>>>(ctx->d_consts.p, L, ctx->d_table.p, ctx->n, ctx->xmin, ctx->xmax, ctx->variant);
+    const int blocks = (int)(((int64_t)n_src + 31) / 32);
+    if (ctx->is_grid) setup_consts_grid_kernel<<<blocks, 32, 0, ctx->stream>>>(out, L, src, n_src, ctx->grid, ctx->variant);
+    else setup_consts_kernel<<<blocks, 32, 0, ctx->stream>>>(out, L, src, n_src, ctx->d_table.p, ctx->n, ctx->xmin, ctx->xmax, ctx->variant);
+    CK(cudaGetLastError());
+    return GEOAC_OK;
+}
+
+static int refresh_consts(geoac_ctx* ctx) {
+    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");      // the set-up kernel samples the tables
+    if (!ctx->consts_dirty) return GEOAC_OK;
+    if (int rc = setup_consts(ctx, ctx->d_consts.p, nullptr, 1)) return rc;
+    if (!ctx->is_grid) {
         build_sbpoly_kernel<<<(ctx->n - 1 + 63) / 64, 64, 0, ctx->stream>>>(ctx->d_consts.p, ctx->d_table.p, ctx->n, ctx->xmin, ctx->xmax,
                                                                             ctx->variant == GEOAC_GLOBAL, ctx->d_sbpoly.p);
+        CK(cudaGetLastError());
     }
-    CK(cudaGetLastError());
     ctx->consts_dirty = false;
     return GEOAC_OK;
 }
@@ -510,15 +531,15 @@ static int refresh_consts(geoac_ctx* ctx) {
 // ---- kernel launch ----
 // cost scout: predicted RK4 step counts of the rays into ctx->d_cost, their maximum and sum.  Persistent, the table in shared
 // memory when it fits.
-template <class SEQ>
-static int launch_cost_scout(geoac_ctx* ctx, const TraceArgs& a, int max_optin, cudaStream_t st, uint32_t* cmax, unsigned long long* cost_sum) {
+template <class SEQ, bool MSRC>
+static int launch_cost_scout(geoac_ctx* ctx, const KernelArgs<MSRC>& a, int max_optin, cudaStream_t st, uint32_t* cmax, unsigned long long* cost_sum) {
     constexpr bool kGrid = PacketMode<SEQ>::value;
     constexpr int kScoutBlock = ScoutBlock<SEQ>::value;
     const size_t s_tab = kGrid ? 0 : 16 + (size_t)TAB_NARR * ctx->n * sizeof(double);
     const bool s_in = !kGrid && s_tab <= (size_t)max_optin;
     const void* sfn;
-    if constexpr (kGrid) sfn = (const void*)scout_kernel<SEQ, false>;
-    else sfn = s_in ? (const void*)scout_kernel<SEQ, true> : (const void*)scout_kernel<SEQ, false>;
+    if constexpr (kGrid) sfn = scout_kernel_fn<SEQ, false, MSRC>();
+    else sfn = s_in ? scout_kernel_fn<SEQ, true, MSRC>() : scout_kernel_fn<SEQ, false, MSRC>();
     const size_t s_smem = s_in ? s_tab : 16;
     CK(cudaFuncSetAttribute(sfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s_smem));
     int s_per_sm = 1;
@@ -535,8 +556,8 @@ static int launch_cost_scout(geoac_ctx* ctx, const TraceArgs& a, int max_optin, 
 // Step 1: the longest-predicted-ray-first claim order (trace_kernel.cuh): cost scout, (range-dependent sets) cost dilation, sort.
 // Sets a.order, a.n_claims, a.packet_refill and a.n_long_packets; n_quarter = long packets long enough for quarter claims.
 // `lanes` = lanes of the main launch (the average work of a lane is the scout's cost sum over them).
-template <class EQ>
-static int build_claim_order(geoac_ctx* ctx, TraceArgs& a, long long lanes, int max_optin, cudaStream_t st, int64_t& n_quarter) {
+template <class EQ, bool MSRC>
+static int build_claim_order(geoac_ctx* ctx, KernelArgs<MSRC>& a, long long lanes, int max_optin, cudaStream_t st, int64_t& n_quarter) {
     constexpr bool kGrid = PacketMode<EQ>::value;
     constexpr int group = kGrid ? 32 : 1;                     // range-dependent sets: packets of 32 consecutive rays
     const int64_t n = a.n_rays, n_entries = ((n + group - 1) / group) * group;
@@ -548,7 +569,7 @@ static int build_claim_order(geoac_ctx* ctx, TraceArgs& a, long long lanes, int 
     uint32_t* cmax = ctx->d_hist.p + kCostBuckets;
     uint32_t* n_long = cmax + 1;                              // n_long[1]: quarter packets
     unsigned long long* cost_sum = reinterpret_cast<unsigned long long*>(cmax + 4);
-    if (int rc = launch_cost_scout<typename EQ::Scout>(ctx, a, max_optin, st, cmax, cost_sum)) return rc;
+    if (int rc = launch_cost_scout<typename EQ::Scout, MSRC>(ctx, a, max_optin, st, cmax, cost_sum)) return rc;
     if (kGrid) {
         const uint32_t* cost = ctx->d_cost.p;
         if (ctx->knobs.dilate > 0) {
@@ -619,12 +640,12 @@ static int size_long_region(const geoac_ctx* ctx, TraceArgs& a, int64_t n_quarte
 // -- packets that would outlast the pass on a loaded SM -- goes to CTAs that keep their SM to themselves (their
 // shared-memory request leaves no room for a main CTA), launched first on a high-priority stream; the main launch fills the
 // other SMs, and its surplus CTAs start as SMs free up.  Each side drains its own region first and then helps with the other.
-template <class EQ, int BLOCK>
-static int enqueue_launches(geoac_ctx* ctx, const void* fn, size_t smem, int max_optin, int grid, int grid_long, TraceArgs a, cudaStream_t st) {
+template <class EQ, int BLOCK, class A>
+static int enqueue_launches(geoac_ctx* ctx, const void* fn, size_t smem, int max_optin, int grid, int grid_long, A a, cudaStream_t st) {
     if (grid_long > 0) {
         const size_t smem_long = std::min((size_t)max_optin, std::max(smem, (size_t)max_optin - smem + 4096));
         CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_long));
-        TraceArgs al = a;
+        A al = a;
         al.prefer_long = 1;
         if (NeedsPrev<EQ>::value) {                          // y_{k-1} scratch of both launches, the long one's after the main one's
             const size_t main_doubles = (size_t)EQ::NEQ * grid * BLOCK;
@@ -655,8 +676,8 @@ static int enqueue_launches(geoac_ctx* ctx, const void* fn, size_t smem, int max
     return GEOAC_OK;
 }
 
-template <class EQ, int BLOCK, bool PATHS>
-static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
+template <class EQ, int BLOCK, bool PATHS, bool MSRC>
+static int launch_trace(geoac_ctx* ctx, KernelArgs<MSRC> a, cudaStream_t st) {
     constexpr bool kGrid = PacketMode<EQ>::value;
     const size_t lane_doubles = ((size_t)LaneLayout<EQ>::STRIDE * BLOCK + 1) & ~(size_t)1;
     const size_t fixed = ((sizeof(LaunchConsts) + 15) / 16) * 16 + 16 + lane_doubles * sizeof(double);
@@ -668,8 +689,8 @@ static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
     const size_t smem = in_smem ? fixed + tab_bytes : fixed;
     // the range-dependent node tables, and a profile too large for shared memory, are read through L1 / L2
     const void* fn;
-    if constexpr (kGrid) fn = (const void*)trace_kernel<EQ, BLOCK, false, PATHS>;
-    else fn = in_smem ? (const void*)trace_kernel<EQ, BLOCK, true, PATHS> : (const void*)trace_kernel<EQ, BLOCK, false, PATHS>;
+    if constexpr (kGrid) fn = trace_kernel_fn<EQ, BLOCK, false, PATHS, MSRC>();
+    else fn = in_smem ? trace_kernel_fn<EQ, BLOCK, true, PATHS, MSRC>() : trace_kernel_fn<EQ, BLOCK, false, PATHS, MSRC>();
     CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 1;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, BLOCK, smem));
@@ -689,7 +710,7 @@ static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
     const int lpt_mode = ctx->knobs.lpt;
     if ((lpt_mode == 2 || (lpt_mode == 1 && a.n_rays > (int64_t)grid * BLOCK)) && a.n_rays < ((int64_t)1 << 32)) {
         int64_t n_quarter = 0;
-        if (int rc = build_claim_order<EQ>(ctx, a, (long long)grid * BLOCK, max_optin, st, n_quarter)) return rc;
+        if (int rc = build_claim_order<EQ, MSRC>(ctx, a, (long long)grid * BLOCK, max_optin, st, n_quarter)) return rc;
         grid_long = size_long_region(ctx, a, n_quarter, BLOCK, PATHS);
     }
     ctx->last_long_packets = (int)a.n_long_packets;
@@ -697,28 +718,31 @@ static int launch_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
     return enqueue_launches<EQ, BLOCK>(ctx, fn, smem, max_optin, grid, grid_long, a, st);
 }
 
-// variant -> (equation set, lanes per CTA); PATHS: the raypath / caustic capture kernels (same lanes per SM as the plain ones)
-template <bool PATHS>
-static int dispatch_trace(geoac_ctx* ctx, const TraceArgs& a, cudaStream_t st) {
+// variant -> (equation set, lanes per CTA); PATHS: the raypath / caustic capture kernels (same lanes per SM as the plain ones);
+// MSRC: the many-source record kernels (a.src_consts, a.src_id)
+template <bool PATHS, bool MSRC = false>
+static int dispatch_trace(geoac_ctx* ctx, const KernelArgs<MSRC>& a, cudaStream_t st) {
     const bool amp = ctx->prm.calc_amp != 0;
     switch (ctx->variant) {
-        case GEOAC_2D:     return amp ? launch_trace<Eq2D<true>, 512, PATHS>(ctx, a, st) : launch_trace<Eq2D<false>, 512, PATHS>(ctx, a, st);
+        case GEOAC_2D:     return amp ? launch_trace<Eq2D<true>, 512, PATHS, MSRC>(ctx, a, st) : launch_trace<Eq2D<false>, 512, PATHS, MSRC>(ctx, a, st);
         // Eq3D<true>: 384 lanes = 3 warps per scheduler at <= 168 registers, no spills (420 ms per config-2 pass vs 491 (256) /
         // 494 (512) in round 1).  Nothing in between exists: the register file is four 16 K-register banks, one per scheduler, so
         // 13 or 14 warps put 4 on some scheduler and cap every lane at 128 registers -- the 512-lane case, which spills (measured
         // on B200: 416 / 448 lanes at 152 / 144 registers compile without spills but do not fit on an SM).
-        case GEOAC_3D:     return amp ? launch_trace<Eq3D<true>, 384, PATHS>(ctx, a, st) : launch_trace<Eq3D<false>, 512, PATHS>(ctx, a, st);
-        case GEOAC_GLOBAL: return amp ? launch_trace<EqGlobal<true>, 384, PATHS>(ctx, a, st) : launch_trace<EqGlobal<false>, 512, PATHS>(ctx, a, st);
-        case GEOAC_3D_RNGDEP:     return amp ? launch_trace<Eq3DRD<true>, 128, PATHS>(ctx, a, st)     : launch_trace<Eq3DRD<false>, 128, PATHS>(ctx, a, st);
-        case GEOAC_GLOBAL_RNGDEP: return amp ? launch_trace<EqGlobalRD<true>, 128, PATHS>(ctx, a, st) : launch_trace<EqGlobalRD<false>, 128, PATHS>(ctx, a, st);
+        case GEOAC_3D:     return amp ? launch_trace<Eq3D<true>, 384, PATHS, MSRC>(ctx, a, st) : launch_trace<Eq3D<false>, 512, PATHS, MSRC>(ctx, a, st);
+        case GEOAC_GLOBAL: return amp ? launch_trace<EqGlobal<true>, 384, PATHS, MSRC>(ctx, a, st) : launch_trace<EqGlobal<false>, 512, PATHS, MSRC>(ctx, a, st);
+        case GEOAC_3D_RNGDEP:     return amp ? launch_trace<Eq3DRD<true>, 128, PATHS, MSRC>(ctx, a, st)     : launch_trace<Eq3DRD<false>, 128, PATHS, MSRC>(ctx, a, st);
+        case GEOAC_GLOBAL_RNGDEP: return amp ? launch_trace<EqGlobalRD<true>, 128, PATHS, MSRC>(ctx, a, st) : launch_trace<EqGlobalRD<false>, 128, PATHS, MSRC>(ctx, a, st);
     }
     return fail(ctx, GEOAC_ERR_BAD_ARG, "variant not implemented");
 }
 
 // One trace on `st`: zeroes the records and counters, fills in the context's part of `a` and launches.  The caller sets the
-// rays (theta, phi, n_rays) and their outputs (rec, status, n_steps), and the capture fields (zero: no capture).  The launch
-// invariants must be current (refresh_consts) and ordered before `st`.
-static int enqueue_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
+// rays (theta, phi, n_rays) and their outputs (rec, status, n_steps), the capture fields (zero: no capture) and, for rays
+// from several sources (A = TraceArgsMS, no capture), src_consts and src_id.  The launch invariants must be current
+// (refresh_consts) and ordered before `st`.
+template <class A>
+static int enqueue_trace(geoac_ctx* ctx, A a, cudaStream_t st) {
     const int n_rec = ctx->prm.bounces + 1;
     const int64_t n_slots = a.n_rays * n_rec;
     CK(cudaMemsetAsync(ctx->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
@@ -730,7 +754,8 @@ static int enqueue_trace(geoac_ctx* ctx, TraceArgs a, cudaStream_t st) {
     a.sbpoly = (ctx->is_grid || !ctx->knobs.sbpoly) ? nullptr : ctx->d_sbpoly.p;   // knob sbpoly = 0: the full absorption model at every step (A/B measurements, tests)
     a.consts = ctx->d_consts.p; a.n_rec = n_rec;
     a.counter = ctx->d_counters.p; a.total_steps = ctx->d_counters.p + 1; a.warp_trips = ctx->d_counters.p + 2;
-    return (a.path_stride > 0 || a.caus_cap > 0) ? dispatch_trace<true>(ctx, a, st) : dispatch_trace<false>(ctx, a, st);
+    if constexpr (std::is_same<A, TraceArgsMS>::value) return dispatch_trace<false, true>(ctx, a, st);
+    else return (a.path_stride > 0 || a.caus_cap > 0) ? dispatch_trace<true>(ctx, a, st) : dispatch_trace<false>(ctx, a, st);
 }
 
 extern "C" int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, const double* d_phi,
@@ -796,11 +821,15 @@ __global__ void compact_rows_kernel(const double* dense, const int32_t* rows, co
 // total_cap of them; ray i's run from offs[i] to offs[i + 1].
 enum class Capture { none, dense, compact };
 struct CaptureOut { int64_t cap = 0; double* data = nullptr; int32_t* rows = nullptr; int64_t* offs = nullptr; int64_t total_cap = 0; };
+// Rays from several sources (geoac_trace_sources, already validated): ray r starts from src[id[r]], n rows of 3 doubles.
+// id == nullptr: every ray starts from params.src.
+struct Sources { int n = 0; const double* src = nullptr; const int32_t* id = nullptr; };
 
-// The host-buffer trace (geoac_trace, geoac_trace_paths, geoac_trace_paths_compact, each context of geoac_trace_multi):
-// angles in, one trace on ctx->stream, records out, plus the raypath rows (every path_stride steps) and caustic events asked for.
+// The host-buffer trace (geoac_trace, geoac_trace_paths, geoac_trace_paths_compact, geoac_trace_sources, each context of
+// geoac_trace_multi): angles in, one trace on ctx->stream, records out, plus the raypath rows (every path_stride steps) and
+// caustic events asked for.  With `srcs`, the rays start from their own sources (no capture).
 static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps,
-                      Capture mode = Capture::none, int path_stride = 0, CaptureOut path = {}, CaptureOut caus = {}) {
+                      Capture mode = Capture::none, int path_stride = 0, CaptureOut path = {}, CaptureOut caus = {}, Sources srcs = {}) {
     if (!ctx || n_rays < 0 || (n_rays > 0 && (!theta || !phi || !rec || !status || !n_steps))) return GEOAC_ERR_BAD_ARG;
     const bool compact = mode == Capture::compact;
     auto has_rows = [&](const CaptureOut& c) { return compact ? c.offs != nullptr : c.rows != nullptr; };
@@ -832,15 +861,25 @@ static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const
         if (!compact) CK(cudaMemsetAsync(s.data.p, 0, bytes, st));       // the caller receives every slot; compaction copies only rows produced
         CK(cudaMemsetAsync(s.rows.p, 0, sizeof(int32_t) * n_rays, st));
     }
-    TraceArgs a{};
+    TraceArgsMS a{};                                                     // the source fields are used with `srcs` only
     a.theta = ctx->d_theta.p; a.phi = ctx->d_phi.p; a.n_rays = n_rays; a.rec = ctx->d_rec.p; a.status = ctx->d_status.p; a.n_steps = ctx->d_nsteps.p;
     if (path_stride > 0) { a.path = ctx->d_path.p; a.path_rows = ctx->d_path_rows.p; a.path_stride = path_stride; a.path_cap = path.cap; }
     if (caus.cap > 0) { a.caus = ctx->d_caus.p; a.caus_rows = ctx->d_caus_rows.p; a.caus_cap = caus.cap; }
+    if (srcs.id) {
+        CK(ctx->d_src.grow(sizeof(double) * 3 * srcs.n)); CK(ctx->d_src_consts.grow(sizeof(LaunchConsts) * srcs.n));
+        CK(ctx->d_src_id.grow(sizeof(int32_t) * n_rays));
+        a.src_consts = ctx->d_src_consts.p; a.src_id = ctx->d_src_id.p;
+    }
     CK(cudaMemcpyAsync(ctx->d_theta.p, theta, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(ctx->d_phi.p, phi, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
+    if (srcs.id) {
+        CK(cudaMemcpyAsync(ctx->d_src.p, srcs.src, sizeof(double) * 3 * srcs.n, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(ctx->d_src_id.p, srcs.id, sizeof(int32_t) * n_rays, cudaMemcpyHostToDevice, st));
+    }
     if (int rc = refresh_consts(ctx)) return rc;                         // before ev0: the timed window holds the trace alone
+    if (srcs.id) { if (int rc = setup_consts(ctx, ctx->d_src_consts.p, ctx->d_src.p, srcs.n)) return rc; }
     CK(cudaEventRecord(ctx->ev0, st));
-    if (int rc = enqueue_trace(ctx, a, st)) return rc;
+    if (int rc = srcs.id ? enqueue_trace(ctx, a, st) : enqueue_trace(ctx, static_cast<const TraceArgs&>(a), st)) return rc;
     CK(cudaEventRecord(ctx->ev1, st));
     CK(cudaMemcpyAsync(rec, ctx->d_rec.p, sizeof(double) * GEOAC_NFIELDS * n_slots, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(status, ctx->d_status.p, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
@@ -881,6 +920,23 @@ static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const
 extern "C" int geoac_trace(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,
                            double* rec, int32_t* status, int32_t* n_steps) {
     return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps);
+}
+
+extern "C" int geoac_trace_sources(geoac_ctx* ctx, int n_src, const double* src, int64_t n_rays, const int32_t* src_id,
+                                   const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps) {
+    if (!ctx) return GEOAC_ERR_BAD_ARG;
+    if (n_rays < 0) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: n_rays < 0");
+    if (n_rays == 0) return GEOAC_OK;
+    if (n_src < 1 || !src || !src_id || !theta || !phi || !rec || !status || !n_steps)
+        return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: need n_src >= 1 and non-null buffers");
+    for (int s = 0; s < n_src; s++)
+        if (!std::isfinite(src[3 * (size_t)s]) || !std::isfinite(src[3 * (size_t)s + 1]) || !std::isfinite(src[3 * (size_t)s + 2]))
+            return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: coordinates of source " + std::to_string(s) + " are not finite");
+    for (int64_t r = 0; r < n_rays; r++)
+        if (src_id[r] < 0 || src_id[r] >= n_src)
+            return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: src_id of ray " + std::to_string(r) + " is " + std::to_string(src_id[r])
+                                                + ", outside [0, " + std::to_string(n_src) + ")");
+    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, Capture::none, 0, {}, {}, { n_src, src, src_id });
 }
 
 extern "C" int geoac_trace_paths(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,

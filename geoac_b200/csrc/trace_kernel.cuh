@@ -57,6 +57,13 @@ struct TraceArgs {
     double* caus; int32_t* caus_rows; int64_t caus_cap;                    // caustic events (PATHS kernels), else unused
     double* prev;                     // y_{k-1} scratch: [NEQ][grid * block] doubles (variants with a quadratic intercept)
 };
+// Arguments of the many-source kernels (MSRC): ray r is launched from source src_id[r], whose invariants are
+// src_consts[src_id[r]].  A type of their own, so that the single-source kernels keep their parameters as they are.
+struct TraceArgsMS : TraceArgs {
+    const LaunchConsts* src_consts;
+    const int32_t* src_id;
+};
+template <bool MSRC> using KernelArgs = std::conditional_t<MSRC, TraceArgsMS, TraceArgs>;
 
 // Per-launch invariants of the stratified variants (source / ground / reference-level atmosphere samples and the
 // Sutherland-Bass reference state), evaluated once with the same spline routines the rays use.
@@ -328,8 +335,19 @@ template <class EQ> struct LaneLayout {
     static constexpr int STRIDE = (WORK + EXTRA) | 1;
 };
 
-template <class EQ, int BLOCK, bool TABLE_IN_SMEM, bool PATHS = false>
-__global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__ TraceArgs a) {
+// The invariants a ray is traced with: the launch's (L) or, in the many-source kernels, those of the ray's own source s, read
+// from global memory through L1 (a warp whose rays share a source reads one address).  Rays keep the caller's order among
+// equal claim keys, so a batch laid out source by source gives warps of mostly one source.
+template <bool MSRC>
+__device__ __forceinline__ const LaunchConsts& ray_consts(const LaunchConsts& L, const KernelArgs<MSRC>& a, int s) {
+    if constexpr (MSRC) return a.src_consts[s];
+    else return L;
+}
+
+// ARGS: TraceArgs, or TraceArgsMS for the many-source kernels (MSRC)
+template <class EQ, int BLOCK, bool TABLE_IN_SMEM, bool PATHS = false, class ARGS = TraceArgs>
+__global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__ ARGS a) {
+    constexpr bool MSRC = std::is_same<ARGS, TraceArgsMS>::value;
     constexpr int NEQ = EQ::NEQ;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // layout: [LaunchConsts][mbarrier][lane records: BLOCK x STRIDE doubles][table]
@@ -338,8 +356,10 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
     double* lanes = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(bar) + 16);
     double* tab_s = lanes + ((LaneLayout<EQ>::STRIDE * BLOCK + 1) & ~1);          // keep the table 16-byte aligned
 
-    for (int i = threadIdx.x; i < (int)(sizeof(LaunchConsts) / 8); i += BLOCK)
-        reinterpret_cast<double*>(Ls)[i] = reinterpret_cast<const double*>(a.consts)[i];
+    if constexpr (!MSRC) {                      // the many-source kernels read each ray's invariants from a.src_consts instead
+        for (int i = threadIdx.x; i < (int)(sizeof(LaunchConsts) / 8); i += BLOCK)
+            reinterpret_cast<double*>(Ls)[i] = reinterpret_cast<const double*>(a.consts)[i];
+    }
     typename EQ::Atmo T;
     double* const work = lanes + (size_t)threadIdx.x * LaneLayout<EQ>::STRIDE + LaneLayout<EQ>::WORK;
     if constexpr (std::is_same<typename EQ::Atmo, Grid3D>::value) {
@@ -363,6 +383,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
     o.caus = a.caus; o.caus_rows = a.caus_rows; o.caus_cap = a.caus_cap;
     LaneD<EQ>& ld = *reinterpret_cast<LaneD<EQ>*>(lanes + (size_t)threadIdx.x * LaneLayout<EQ>::STRIDE);
     LaneI<EQ> li;
+    int rsrc = 0;                      // MSRC: source of the lane's ray
     // y_{k-1} history (quadratic intercept only): [eq][global thread] in an L2-resident global scratch, written once per step
     const int64_t pstride = (int64_t)gridDim.x * BLOCK;
     double* prev = a.prev + ((int64_t)blockIdx.x * BLOCK + threadIdx.x);
@@ -409,7 +430,10 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
                 else if ((int)lane < width) {
                     const int64_t idx = (int64_t)base + lane;
                     const int64_t r = a.order ? (int64_t)a.order[idx] : idx;
-                    if (r < a.n_rays) { lane_start<EQ>(ld, li, L, T, r, a.theta[r], a.phi[r]); have_ray = true; }
+                    if (r < a.n_rays) {
+                        if constexpr (MSRC) rsrc = a.src_id[r];
+                        lane_start<EQ>(ld, li, ray_consts<MSRC>(L, a, rsrc), T, r, a.theta[r], a.phi[r]); have_ray = true;
+                    }
                 }
             }
         } else {
@@ -426,7 +450,10 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
                     const int64_t idx = (int64_t)base + rank;
                     if (idx < a.n_claims) {
                         const int64_t r = a.order ? (int64_t)a.order[idx] : idx;
-                        if (r < a.n_rays) { lane_start<EQ>(ld, li, L, T, r, a.theta[r], a.phi[r]); have_ray = true; }
+                        if (r < a.n_rays) {
+                            if constexpr (MSRC) rsrc = a.src_id[r];
+                            lane_start<EQ>(ld, li, ray_consts<MSRC>(L, a, rsrc), T, r, a.theta[r], a.phi[r]); have_ray = true;
+                        }
                     }
                     else exhausted = true;
                 }
@@ -453,6 +480,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
             gi.ray = __shfl_sync(0xffffffffu, (long long)li.ray, owner);
             gi.path_n = __shfl_sync(0xffffffffu, li.path_n, owner); gi.caus_n = __shfl_sync(0xffffffffu, li.caus_n, owner);
             gi.caus_b = PATHS ? __shfl_sync(0xffffffffu, li.caus_b, owner) : 0;
+            const int gsrc = MSRC ? __shfl_sync(0xffffffffu, rsrc, owner) : 0;     // a ray keeps its source: nothing to hand back
             const int othread = (int)(threadIdx.x & ~31u) + owner;
             double* const rec = lanes + (size_t)othread * LaneLayout<EQ>::STRIDE;
             double* const gwork = rec + LaneLayout<EQ>::WORK;
@@ -460,7 +488,8 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
             Tg.scratch = gwork + 2 * NEQ;
             if (coop) { Tg.role = (int)lane & 3; Tg.nrole = 4; Tg.glane0 = (int)lane & ~3; Tg.gmask = 0xFu << ((int)lane & ~3); }
             bool alive = false;
-            if (run) alive = lane_advance<EQ, PATHS>(*reinterpret_cast<LaneD<EQ>*>(rec), gi, L, Tg, a.prev + ((int64_t)blockIdx.x * BLOCK + othread), pstride, o, gwork);
+            if (run) alive = lane_advance<EQ, PATHS>(*reinterpret_cast<LaneD<EQ>*>(rec), gi, ray_consts<MSRC>(L, a, gsrc), Tg,
+                                                       a.prev + ((int64_t)blockIdx.x * BLOCK + othread), pstride, o, gwork);
             // hand the integer state back to the lane that owns the ray (itself in serial mode)
             const int src = (coop && have_ray) ? 4 * __popc(act & ((1u << lane) - 1u)) : (int)lane;
             const int bka = __shfl_sync(0xffffffffu, gi.cur.ka, src), bkb = __shfl_sync(0xffffffffu, gi.cur.kb, src);
@@ -476,7 +505,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
             }
         } else {
             if (have_ray) {
-                have_ray = lane_advance<EQ, PATHS>(ld, li, L, T, prev, pstride, o, work);
+                have_ray = lane_advance<EQ, PATHS>(ld, li, ray_consts<MSRC>(L, a, rsrc), T, prev, pstride, o, work);
                 my_steps++;
             }
         }
@@ -502,9 +531,11 @@ template <class EQ> struct ScoutBlock { static constexpr int value = std::is_sam
 // Persistent like the trace kernel: lanes are refilled from a counter as their rays end (a warp of rays with different
 // lifetimes never idles), the 1-D table sits in shared memory; the ray state (<= 6 equations, no auxiliary set) fits
 // in registers.
-template <class EQ, bool TABLE_IN_SMEM>
-__global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const __grid_constant__ TraceArgs a, uint32_t* cost, uint32_t* cost_max,
+// ARGS = TraceArgsMS (MSRC): each ray is predicted with its own source's invariants (ray_consts).
+template <class EQ, bool TABLE_IN_SMEM, class ARGS = TraceArgs>
+__global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const __grid_constant__ ARGS a, uint32_t* cost, uint32_t* cost_max,
                                                                unsigned long long* cost_sum, unsigned long long* counter, int coarse) {
+    constexpr bool MSRC = std::is_same<ARGS, TraceArgsMS>::value;
     constexpr int NEQ = EQ::NEQ;
     constexpr bool kGrid = std::is_same<typename EQ::Atmo, Grid3D>::value;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -525,6 +556,7 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
     double y[NEQ], ym1[NEQ];
     typename EQ::RayC rc; typename EQ::Cursor cur = typename EQ::Cursor{};
     uint32_t est = 0, seg = 0, worst = 0; int bounce = 0; int64_t ray = 0;
+    int rsrc = 0;
     unsigned long long total = 0;
     bool have_ray = false, exhausted = false;
     while (true) {
@@ -539,7 +571,8 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
                 ray = (int64_t)(base + __popc(wmask & ((1u << lane) - 1u)));
                 if (ray < a.n_rays) {
                     cur = typename EQ::Cursor{};
-                    EQ::init(L, T, a.theta[ray], a.phi[ray], rc, y, cur);
+                    if constexpr (MSRC) rsrc = a.src_id[ray];
+                    EQ::init(ray_consts<MSRC>(L, a, rsrc), T, a.theta[ray], a.phi[ray], rc, y, cur);
 #pragma unroll
                     for (int i = 0; i < NEQ; i++) ym1[i] = y[i];
                     est = 0; seg = 0; bounce = 0; have_ray = true;
@@ -548,24 +581,25 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
         }
         if (!__any_sync(0xffffffffu, have_ray)) break;
         if (!have_ray) continue;
+        const LaunchConsts& Lr = ray_consts<MSRC>(L, a, rsrc);
         double acc[NEQ], p[NEQ], f[NEQ];
-        const double ds = (double)coarse * EQ::step_size(L, y);
+        const double ds = (double)coarse * EQ::step_size(Lr, y);
 #pragma unroll
         for (int i = 0; i < NEQ; i++) { acc[i] = y[i]; p[i] = y[i]; }
 #pragma unroll 1
         for (int s = 0; s < 4; s++) {
-            const double sc = EQ::rhs(L, T, rc, p, f, cur);
+            const double sc = EQ::rhs(Lr, T, rc, p, f, cur);
             const double dsa = ds * ((s == 2) ? 1.0 : 0.5) * sc, dsb = ds * ((s == 0 || s == 3) ? (1.0 / 6.0) : (1.0 / 3.0)) * sc;
 #pragma unroll
             for (int i = 0; i < NEQ; i++) { acc[i] = fma(f[i], dsb, acc[i]); p[i] = fma(f[i], dsa, y[i]); }
         }
         est += (uint32_t)coarse; seg += (uint32_t)coarse;
-        bool done = EQ::left_region(L, rc, acc) || seg >= cap;
-        if (!done && EQ::below_ground(L, acc)) {
+        bool done = EQ::left_region(Lr, rc, acc) || seg >= cap;
+        if (!done && EQ::below_ground(Lr, acc)) {
             if (bounce >= L.bounces) done = true;
             else {
                 double y0[NEQ];
-                EQ::reflect(L, T, rc, ym1, y, acc, y0, cur);
+                EQ::reflect(Lr, T, rc, ym1, y, acc, y0, cur);
 #pragma unroll
                 for (int i = 0; i < NEQ; i++) { acc[i] = y0[i]; y[i] = y0[i]; }      // restart: y = ym1 = reflected state
                 bounce++; seg = 0;
@@ -585,6 +619,7 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
     if (lane == 0 && worst) { atomicMax(cost_max, worst); atomicAdd(cost_sum, total); }
 }
 
+#ifndef GEOAC_TRACE_KERNELS_ONLY          // the claim-order kernels below have one home: capi.cu
 // The cost scout is accurate in bulk (config 5: correlation 0.988 with the true step counts, median ratio 0.999) but a ray at the edge
 // of a ducted family can go either way: measured, a ray predicted at 21 k steps took 389 k, its packet sat at the back of the
 // claim order and one rank in eight ran 27 s instead of 22.5 s.  Such rays are neighbours in inclination of rays that ARE predicted
@@ -742,6 +777,24 @@ __global__ void stable_scatter_kernel(const uint8_t* key, const uint32_t* src, i
         }
         __syncwarp();
     }
+}
+
+#endif  // GEOAC_TRACE_KERNELS_ONLY
+
+// The many-source kernels (ARGS = TraceArgsMS) are instantiated in trace_sources.cu, a translation unit of their own: the out-of-line
+// absorption path (core.cuh: suthbass_alpha_cold) is one function per unit, compiled for the shared-memory invariants of the
+// single-source kernels; a caller passing global-memory invariants in the same unit would turn its shared loads generic.
+template <class EQ, int BLOCK, bool TABLE_IN_SMEM> const void* msrc_trace_kernel();
+template <class EQ, bool TABLE_IN_SMEM> const void* msrc_scout_kernel();
+template <class EQ, int BLOCK, bool TABLE_IN_SMEM, bool PATHS, bool MSRC>
+const void* trace_kernel_fn() {
+    if constexpr (MSRC) return msrc_trace_kernel<EQ, BLOCK, TABLE_IN_SMEM>();
+    else return (const void*)trace_kernel<EQ, BLOCK, TABLE_IN_SMEM, PATHS>;
+}
+template <class EQ, bool TABLE_IN_SMEM, bool MSRC>
+const void* scout_kernel_fn() {
+    if constexpr (MSRC) return msrc_scout_kernel<EQ, TABLE_IN_SMEM>();
+    else return (const void*)scout_kernel<EQ, TABLE_IN_SMEM>;
 }
 
 #endif  // __CUDACC__

@@ -177,6 +177,23 @@ int geoac_trace(geoac_ctx* ctx, int64_t n_rays, const double* theta, const doubl
 int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, const double* d_phi,
                        double* d_rec, int32_t* d_status, int32_t* d_n_steps, void* cuda_stream);
 
+/* geoac_trace() for rays from many sources in one call: ray r is launched at (theta[r], phi[r]) from source src_id[r].
+ *   src    : n_src rows of 3 doubles in the convention of geoac_params.src -- (x, y, z) [km] in Cartesian (2D uses z only),
+ *            (altitude [km], lat [rad], lon [rad]) for Global -- each clamped to the ground as params.src is;
+ *   src_id : n_rays int32 in [0, n_src);
+ *   rec, status, n_steps : laid out exactly as geoac_trace's.
+ * The record, status and step count of ray r are bit for bit what geoac_trace returns for (theta[r], phi[r]) on this context
+ * with params.src set to src[src_id[r]], whatever the other rays of the batch, their sources and their order.  The
+ * context's parameters are not changed; geoac_last_trace_stats, geoac_last_trace_counters, geoac_last_schedule and
+ * geoac_get_costs report the call like any trace.  Lay the batch out source by source, each source's rays in the mains'
+ * loop order: the claim order keeps the caller's order among rays of equal predicted cost, so warps then hold rays of
+ * mostly one source (one cached read of its invariants) and neighbouring paths.  Same concurrency contract as geoac_trace.
+ * Errors, returned before any device work: GEOAC_ERR_BAD_ARG (NULL context, n_rays < 0; with n_rays > 0: n_src < 1, a NULL
+ * pointer, a non-finite source coordinate, a src_id outside [0, n_src) -- the message names the source or the first such
+ * ray), GEOAC_ERR_NO_ATMO; n_rays == 0 reads and writes nothing and is GEOAC_OK. */
+int geoac_trace_sources(geoac_ctx* ctx, int n_src, const double* src, int64_t n_rays, const int32_t* src_id,
+                        const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps);
+
 /* geoac_trace() plus the raypath rows of the mains' WriteRays=True mode (Code/GeoAc3D_main.cpp:249-262 and siblings; the
  * same call serves `-interactive`, which plots one ray): every `path_stride` steps (the mains use 25) one row of
  * GEOAC_PATH_NF doubles { state[0], state[1], state[2], amplitude (linear, 0 with calc_amp = 0), absorption sum, travel-time
