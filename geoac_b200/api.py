@@ -52,6 +52,8 @@ def lib():
         L.geoac_trace_paths_compact.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _ip, _ip, C.c_int, C.c_int64, C.c_int64, _dp, _lp,
                                                 C.c_int64, C.c_int64, _dp, _lp]
         L.geoac_trace_sources.argtypes = [C.c_void_p, C.c_int, _dp, C.c_int64, _ip, _dp, _dp, _dp, _ip, _ip]
+        L.geoac_set_ensemble_1d.argtypes = [C.c_void_p, C.c_int, _lp, _dp, _dp, _dp, _dp, _dp]
+        L.geoac_trace_ensemble.argtypes = [C.c_void_p, C.c_int64, _ip, _dp, _dp, _dp, _ip, _ip]
         L.geoac_trace_device.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.geoac_reserve.argtypes = [C.c_void_p, C.c_int64]
         L.geoac_host_alloc.restype = C.c_void_p
@@ -92,7 +94,7 @@ def lib():
 EXPORTED_SYMBOLS = [
     "geoac_create", "geoac_destroy", "geoac_last_error", "geoac_default_params", "geoac_set_atmosphere_1d",
     "geoac_set_atmosphere_3d", "geoac_get_params", "geoac_set_params", "geoac_trace", "geoac_trace_paths", "geoac_trace_device",
-    "geoac_trace_sources",
+    "geoac_trace_sources", "geoac_set_ensemble_1d", "geoac_trace_ensemble",
     "geoac_reserve", "geoac_last_trace_stats", "geoac_last_trace_counters", "geoac_selftest_math", "geoac_load_met_1d", "geoac_load_met_grid", "geoac_eq_count", "geoac_measure_fp64_peak",
     "geoac_get_grid_tables", "geoac_default_eig_opts", "geoac_eigenray_search", "geoac_eigenray_direct", "geoac_get_variant", "geoac_source_state",
     "geoac_sample_atmosphere",
@@ -215,6 +217,18 @@ class Tracer:
             raise GeoAcError("set_atmosphere_1d: z, T, u, v, rho must be 1-D arrays of one length")
         self._check(lib().geoac_set_atmosphere_1d(self._h, len(arrs[0]), *[_p(a) for a in arrs]), "geoac_set_atmosphere_1d")
 
+    def set_ensemble_1d(self, members):
+        """An ensemble of stratified profiles, next to the context's own atmosphere: members is a list of (z, T, u, v, rho), each
+        in the form set_atmosphere_1d takes (include/geoac_b200.h: geoac_set_ensemble_1d)."""
+        members = [[np.ascontiguousarray(a, dtype=np.float64) for a in m] for m in members]
+        if not members or any(len(m) != 5 or any(a.ndim != 1 or a.shape != m[0].shape for a in m) for m in members):
+            raise GeoAcError("set_ensemble_1d: members must be a non-empty list of (z, T, u, v, rho), 1-D arrays of one length each")
+        offs = np.zeros(len(members) + 1, dtype=np.int64)
+        offs[1:] = np.cumsum([len(m[0]) for m in members])
+        cols = [np.ascontiguousarray(np.concatenate([m[k] for m in members])) for k in range(5)]
+        self._check(lib().geoac_set_ensemble_1d(self._h, len(members), offs.ctypes.data_as(C.POINTER(C.c_int64)), *[_p(a) for a in cols]),
+                    "geoac_set_ensemble_1d")
+
     def set_atmosphere_3d(self, ax0, ax1, axz, T, u, v, rho):
         arrs = [np.ascontiguousarray(a, dtype=np.float64) for a in (ax0, ax1, axz, T, u, v, rho)]
         nodes = len(arrs[0]) * len(arrs[1]) * len(arrs[2])
@@ -331,6 +345,20 @@ class Tracer:
         self._check(lib().geoac_trace_sources(self._h, len(src), _p(src), len(theta), src_id.ctypes.data_as(_ip), _p(theta), _p(phi),
                                               _p(out["rec"]), out["status"].ctypes.data_as(_ip), out["n_steps"].ctypes.data_as(_ip)),
                     "geoac_trace_sources")
+        return out
+
+    def trace_ensemble(self, atm_id, theta, phi, out=None):
+        """trace() for rays through many atmospheres in one call: ray r runs through member atm_id[r] (int32 [n]) of the
+        ensemble of set_ensemble_1d.  Ray r's records equal those of trace() on a context with that member's profile and
+        these parameters (include/geoac_b200.h: geoac_trace_ensemble).  Lay the batch out member by member."""
+        theta, phi, out = self._rays_and_records("trace_ensemble", theta, phi, out)
+        atm_id = np.asarray(atm_id)
+        if atm_id.dtype != np.int32 or atm_id.shape != theta.shape:
+            raise GeoAcError("trace_ensemble: atm_id must be an int32 array with one entry per ray")
+        atm_id = np.ascontiguousarray(atm_id)
+        self._check(lib().geoac_trace_ensemble(self._h, len(theta), atm_id.ctypes.data_as(_ip), _p(theta), _p(phi), _p(out["rec"]),
+                                               out["status"].ctypes.data_as(_ip), out["n_steps"].ctypes.data_as(_ip)),
+                    "geoac_trace_ensemble")
         return out
 
     def trace_paths(self, theta, phi, stride=25, cap=2400, caustic_cap=0):

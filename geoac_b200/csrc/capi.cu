@@ -138,6 +138,17 @@ struct geoac_ctx {
     Buf<double> d_smp_in, d_smp_out;
     // staging of geoac_trace_sources: the sources, each ray's source and the invariants of each source
     Buf<double> d_src; Buf<int32_t> d_src_id; Buf<LaunchConsts> d_src_consts;
+    // the ensemble of geoac_set_ensemble_1d (ens_n members, 0 = none): the members' tables one after the other, their
+    // absorption polynomials (member m's from interval ens_iv_off[m] on), 3 ens_n descriptors (Table1D: [0, n) with the
+    // polynomials, [n, 2n) without, [2n, 3n) for the cost scout), and one LaunchConsts per member, rebuilt when ens_dirty
+    int ens_n = 0;
+    int64_t ens_n_iv = 0;
+    Buf<double> d_ens_table, d_ens_sbpoly;
+    Buf<int64_t> d_ens_iv_off;
+    Buf<Table1D> d_ens_tab;
+    Buf<LaunchConsts> d_ens_consts;
+    bool ens_dirty = true;
+    Buf<int32_t> d_atm_id;                         // staging of geoac_trace_ensemble: each ray's member
 };
 
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
@@ -221,7 +232,7 @@ extern "C" int geoac_get_params(const geoac_ctx* ctx, geoac_params* p) { if (!ct
 extern "C" int geoac_set_params(geoac_ctx* ctx, const geoac_params* p) {
     if (!ctx || !p) return GEOAC_ERR_BAD_ARG;
     if (p->bounces < 0 || p->ds_min <= 0.0 || p->ray_limit <= 0.0) return fail(ctx, GEOAC_ERR_BAD_ARG, "bad params");
-    ctx->prm = *p; ctx->consts_dirty = true; ctx->src_set = true; return GEOAC_OK;
+    ctx->prm = *p; ctx->consts_dirty = true; ctx->ens_dirty = true; ctx->src_set = true; return GEOAC_OK;
 }
 
 extern "C" int geoac_set_knob(geoac_ctx* ctx, const char* name, int value) {
@@ -254,19 +265,11 @@ static void natural_slopes(const std::vector<double>& x, const double* f, double
     for (int i = n - 2; i > -1; i--) s[i] = dp[i] - cp[i] * s[i + 1];
 }
 
-extern "C" int geoac_set_atmosphere_1d(geoac_ctx* ctx, int n, const double* z, const double* T,
-                                       const double* u, const double* v, const double* rho) {
-    if (!ctx) return GEOAC_ERR_BAD_ARG;
-    if (ctx->variant != GEOAC_2D && ctx->variant != GEOAC_3D && ctx->variant != GEOAC_GLOBAL)
-        return fail(ctx, GEOAC_ERR_BAD_ARG, "variant needs geoac_set_atmosphere_3d");
-    if (n < 3 || !z || !T || !u || !v || !rho) return fail(ctx, GEOAC_ERR_BAD_ARG, "need >= 3 levels and non-null arrays");
-    for (int i = 1; i < n; i++) if (!(z[i] > z[i - 1])) return fail(ctx, GEOAC_ERR_BAD_ARG, "altitudes must be strictly increasing");
-    cudaSetDevice(ctx->device);
-    const bool glob = ctx->variant == GEOAC_GLOBAL;
+// The table of one profile (n >= 3 levels of z, T, u, v, rho, altitudes strictly increasing) into tb, TAB_NARR * n doubles: one
+// record per level (core.cuh), x = z (+ r_earth for Global), 1/h, and each field with its natural-spline knot slope.
+static void build_table_1d(bool glob, int n, const double* z, const double* T, const double* u, const double* v, const double* rho, double* tb) {
     std::vector<double> x(n), col(n), slo(n);
     for (int i = 0; i < n; i++) { x[i] = z[i]; if (glob) x[i] += kREarth; }   // r_vals[nr] += r_earth
-    ctx->h_table.assign((size_t)TAB_NARR * n, 0.0);                           // one record per level (core.cuh)
-    double* tb = ctx->h_table.data();
     for (int i = 0; i < n; i++) {
         tb[(size_t)i * TAB_NARR + TAB_X] = x[i];
         tb[(size_t)i * TAB_NARR + TAB_INVH] = (i + 1 < n) ? 1.0 / (x[i + 1] - x[i]) : 0.0;
@@ -278,6 +281,28 @@ extern "C" int geoac_set_atmosphere_1d(geoac_ctx* ctx, int n, const double* z, c
         natural_slopes(x, col.data(), slo.data());
         for (int i = 0; i < n; i++) { tb[(size_t)i * TAB_NARR + slots[f]] = col[i]; tb[(size_t)i * TAB_NARR + slots[f] + 1] = slo[i]; }
     }
+}
+
+// GeoAc_SetPropRegion (G2S_Spline1D.cpp:22-28 / G2S_GlobalSpline1D.cpp:22-30) for a profile whose top is xmax (table coordinates)
+static void set_prop_region_1d(geoac_ctx* ctx, double xmax) {
+    const bool glob = ctx->variant == GEOAC_GLOBAL;
+    ctx->prm.vert_limit = xmax;
+    ctx->prm.range_limit = glob ? 1500.0 : 10000.0;
+    if (glob) { ctx->prm.box_min[0] = -kPi / 2.0; ctx->prm.box_max[0] = kPi / 2.0; ctx->prm.box_min[1] = -kPi; ctx->prm.box_max[1] = kPi; }
+    ctx->consts_dirty = true; ctx->ens_dirty = true;
+}
+
+extern "C" int geoac_set_atmosphere_1d(geoac_ctx* ctx, int n, const double* z, const double* T,
+                                       const double* u, const double* v, const double* rho) {
+    if (!ctx) return GEOAC_ERR_BAD_ARG;
+    if (ctx->variant != GEOAC_2D && ctx->variant != GEOAC_3D && ctx->variant != GEOAC_GLOBAL)
+        return fail(ctx, GEOAC_ERR_BAD_ARG, "variant needs geoac_set_atmosphere_3d");
+    if (n < 3 || !z || !T || !u || !v || !rho) return fail(ctx, GEOAC_ERR_BAD_ARG, "need >= 3 levels and non-null arrays");
+    for (int i = 1; i < n; i++) if (!(z[i] > z[i - 1])) return fail(ctx, GEOAC_ERR_BAD_ARG, "altitudes must be strictly increasing");
+    cudaSetDevice(ctx->device);
+    ctx->h_table.assign((size_t)TAB_NARR * n, 0.0);
+    double* tb = ctx->h_table.data();
+    build_table_1d(ctx->variant == GEOAC_GLOBAL, n, z, T, u, v, rho, tb);
     // build into fresh buffers and swap them in only after every step succeeded: a failed call leaves the previous
     // atmosphere (or "none") fully intact instead of dangling pointers
     Buf<double> nt, ns;
@@ -287,12 +312,72 @@ extern "C" int geoac_set_atmosphere_1d(geoac_ctx* ctx, int n, const double* z, c
         return fail(ctx, GEOAC_ERR_CUDA, std::string("geoac_set_atmosphere_1d: ") + cudaGetErrorString(cudaGetLastError()));
     cudaStreamSynchronize(ctx->stream);                                          // no launch may still read the old tables
     ctx->d_table = std::move(nt); ctx->d_sbpoly = std::move(ns);
-    ctx->n = n; ctx->xmin = x[0]; ctx->xmax = x[n - 1];
-    // GeoAc_SetPropRegion: G2S_Spline1D.cpp:22-28 / G2S_GlobalSpline1D.cpp:22-30
-    ctx->prm.vert_limit = ctx->xmax;
-    ctx->prm.range_limit = glob ? 1500.0 : 10000.0;
-    if (glob) { ctx->prm.box_min[0] = -kPi / 2.0; ctx->prm.box_max[0] = kPi / 2.0; ctx->prm.box_min[1] = -kPi; ctx->prm.box_max[1] = kPi; }
-    ctx->have_atmo = true; ctx->consts_dirty = true;
+    ctx->n = n; ctx->xmin = tb[TAB_X]; ctx->xmax = tb[(size_t)(n - 1) * TAB_NARR + TAB_X];
+    set_prop_region_1d(ctx, ctx->xmax);
+    ctx->have_atmo = true;
+    return GEOAC_OK;
+}
+
+extern "C" int geoac_set_ensemble_1d(geoac_ctx* ctx, int n_atm, const int64_t* level_offset,
+                                     const double* z, const double* T, const double* u, const double* v, const double* rho) {
+    if (!ctx) return GEOAC_ERR_BAD_ARG;
+    if (ctx->variant != GEOAC_2D && ctx->variant != GEOAC_3D && ctx->variant != GEOAC_GLOBAL)
+        return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_set_ensemble_1d: for the stratified variants (2D, 3D, Global) only");
+    if (n_atm < 1 || !level_offset || !z || !T || !u || !v || !rho)
+        return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_set_ensemble_1d: need n_atm >= 1 and non-null arrays");
+    if (level_offset[0] != 0) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_set_ensemble_1d: level_offset[0] must be 0");
+    for (int m = 0; m < n_atm; m++) {
+        const int64_t l0 = level_offset[m], n = level_offset[m + 1] - l0;
+        const std::string who = "geoac_set_ensemble_1d: member " + std::to_string(m);
+        if (n < 0) return fail(ctx, GEOAC_ERR_BAD_ARG, who + ": level_offset is not non-decreasing");
+        if (n < 3) return fail(ctx, GEOAC_ERR_BAD_ARG, who + ": need >= 3 levels");
+        if (n > std::numeric_limits<int>::max()) return fail(ctx, GEOAC_ERR_BAD_ARG, who + ": too many levels");
+        for (int64_t i = l0 + 1; i < l0 + n; i++)
+            if (!(z[i] > z[i - 1])) return fail(ctx, GEOAC_ERR_BAD_ARG, who + ": altitudes must be strictly increasing");
+    }
+    cudaSetDevice(ctx->device);
+    const bool glob = ctx->variant == GEOAC_GLOBAL;
+    const int64_t n_lvl = level_offset[n_atm], n_iv = n_lvl - n_atm;
+    // the members' tables back to back: TAB_NARR doubles (80 bytes) per level and SBP_STRIDE doubles (192 bytes) per interval,
+    // so every member's table and polynomial block starts 16-byte aligned (ld_pair reads double2)
+    static_assert((TAB_NARR * sizeof(double)) % 16 == 0 && (SBP_STRIDE * sizeof(double)) % 16 == 0, "member blocks must stay 16-byte aligned");
+    std::vector<double> tb((size_t)TAB_NARR * n_lvl);
+    std::vector<int64_t> iv_off(n_atm + 1);
+    double top = std::numeric_limits<double>::infinity();
+    for (int m = 0; m < n_atm; m++) {
+        const int64_t l0 = level_offset[m];
+        const int n = (int)(level_offset[m + 1] - l0);
+        build_table_1d(glob, n, z + l0, T + l0, u + l0, v + l0, rho + l0, tb.data() + (size_t)TAB_NARR * l0);
+        iv_off[m] = l0 - m;
+        top = std::min(top, tb[(size_t)TAB_NARR * (l0 + n - 1) + TAB_X]);
+    }
+    iv_off[n_atm] = n_iv;
+    // build into fresh buffers and swap them in only after every step succeeded: a failed call leaves the previous ensemble intact
+    Buf<double> nt, ns; Buf<int64_t> no; Buf<Table1D> nd; Buf<LaunchConsts> nc;
+    const cudaError_t e = [&] {
+        cudaError_t r;
+        if ((r = nt.grow(sizeof(double) * tb.size())) || (r = ns.grow(sizeof(double) * SBP_STRIDE * n_iv)) || (r = no.grow(sizeof(int64_t) * (n_atm + 1)))
+            || (r = nd.grow(sizeof(Table1D) * 3 * n_atm)) || (r = nc.grow(sizeof(LaunchConsts) * n_atm))) return r;
+        std::vector<Table1D> d(3 * (size_t)n_atm);
+        for (int m = 0; m < n_atm; m++) {
+            const int64_t l0 = level_offset[m];
+            const int n = (int)(level_offset[m + 1] - l0);
+            Table1D t; t.base = nt.p + (size_t)TAB_NARR * l0; t.n = n; t.jump_scale = 0.0; t.sbpoly = nullptr;
+            t.xmin = tb[(size_t)TAB_NARR * l0 + TAB_X]; t.xmax = tb[(size_t)TAB_NARR * (l0 + n - 1) + TAB_X];
+            d[n_atm + m] = t;                                                      // the set-up kernels' and knob sbpoly = 0
+            d[m] = t; d[m].sbpoly = ns.p + (size_t)SBP_STRIDE * iv_off[m];
+            d[2 * n_atm + m] = t; d[2 * n_atm + m].jump_scale = (double)(n - 1) / (t.xmax - t.xmin);   // as scout_kernel sets it
+        }
+        if ((r = cudaMemcpy(nt.p, tb.data(), sizeof(double) * tb.size(), cudaMemcpyHostToDevice))
+            || (r = cudaMemcpy(no.p, iv_off.data(), sizeof(int64_t) * (n_atm + 1), cudaMemcpyHostToDevice))) return r;
+        return cudaMemcpy(nd.p, d.data(), sizeof(Table1D) * d.size(), cudaMemcpyHostToDevice);
+    }();
+    if (e != cudaSuccess) return fail(ctx, GEOAC_ERR_CUDA, std::string("geoac_set_ensemble_1d: ") + cudaGetErrorString(e));
+    cudaStreamSynchronize(ctx->stream);                                          // no launch may still read the old ensemble
+    ctx->d_ens_table = std::move(nt); ctx->d_ens_sbpoly = std::move(ns); ctx->d_ens_iv_off = std::move(no);
+    ctx->d_ens_tab = std::move(nd); ctx->d_ens_consts = std::move(nc);
+    ctx->ens_n = n_atm; ctx->ens_n_iv = n_iv;
+    set_prop_region_1d(ctx, top);                                                // the lowest top among the members
     return GEOAC_OK;
 }
 
@@ -495,9 +580,8 @@ __global__ void setup_consts_grid_kernel(LaunchConsts* out, const LaunchConsts i
     out[i] = L;
 }
 
-// The invariants of the context's parameters launched from `src` (device, n_src rows of 3 doubles; nullptr: params.src),
-// one LaunchConsts per source into `out` on ctx->stream.
-static int setup_consts(geoac_ctx* ctx, LaunchConsts* out, const double* src, int n_src) {
+// The part of the invariants that the parameters give (the source from params.src); the set-up kernels add the atmosphere's.
+static LaunchConsts param_consts(const geoac_ctx* ctx) {
     const geoac_params& p = ctx->prm;
     LaunchConsts L; std::memset(&L, 0, sizeof L);
     L.ds_min = p.ds_min; L.ds_max = p.ds_max; L.vert_limit = p.vert_limit; L.range_limit = p.range_limit;
@@ -508,6 +592,13 @@ static int setup_consts(geoac_ctx* ctx, LaunchConsts* out, const double* src, in
     L.seg_mode = (ctx->variant == GEOAC_2D) ? 1 : (p.accum_per_segment ? 1 : 0);                          // App. A-2
     L.step_limit = (int)(p.ray_limit * (int)(1.0 / (p.ds_min * 10)));                                     // Solver.cpp:14
     L.per_bounce_zmax = (ctx->variant == GEOAC_3D_RNGDEP || ctx->variant == GEOAC_GLOBAL_RNGDEP);         // App. A-3
+    return L;
+}
+
+// The invariants of the context's parameters launched from `src` (device, n_src rows of 3 doubles; nullptr: params.src),
+// one LaunchConsts per source into `out` on ctx->stream.
+static int setup_consts(geoac_ctx* ctx, LaunchConsts* out, const double* src, int n_src) {
+    const LaunchConsts L = param_consts(ctx);
     const int blocks = (int)(((int64_t)n_src + 31) / 32);
     if (ctx->is_grid) setup_consts_grid_kernel<<<blocks, 32, 0, ctx->stream>>>(out, L, src, n_src, ctx->grid, ctx->variant);
     else setup_consts_kernel<<<blocks, 32, 0, ctx->stream>>>(out, L, src, n_src, ctx->d_table.p, ctx->n, ctx->xmin, ctx->xmax, ctx->variant);
@@ -528,18 +619,29 @@ static int refresh_consts(geoac_ctx* ctx) {
     return GEOAC_OK;
 }
 
+// The ensemble's counterpart of refresh_consts: every member's invariants and absorption polynomials (trace_ensemble.cu),
+// rebuilt when the parameters or the ensemble changed.
+static int refresh_ensemble(geoac_ctx* ctx) {
+    if (!ctx->ens_n) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an ensemble first (geoac_set_ensemble_1d)");
+    if (!ctx->ens_dirty) return GEOAC_OK;
+    CK(ens_setup(ctx->d_ens_consts.p, param_consts(ctx), ctx->d_ens_tab.p + ctx->ens_n, ctx->ens_n, ctx->d_ens_iv_off.p, ctx->ens_n_iv,
+                 ctx->variant, ctx->d_ens_sbpoly.p, ctx->stream));
+    ctx->ens_dirty = false;
+    return GEOAC_OK;
+}
+
 // ---- kernel launch ----
 // cost scout: predicted RK4 step counts of the rays into ctx->d_cost, their maximum and sum.  Persistent, the table in shared
 // memory when it fits.
-template <class SEQ, bool MSRC>
-static int launch_cost_scout(geoac_ctx* ctx, const KernelArgs<MSRC>& a, int max_optin, cudaStream_t st, uint32_t* cmax, unsigned long long* cost_sum) {
+template <class SEQ, class A>
+static int launch_cost_scout(geoac_ctx* ctx, const A& a, int max_optin, cudaStream_t st, uint32_t* cmax, unsigned long long* cost_sum) {
     constexpr bool kGrid = PacketMode<SEQ>::value;
     constexpr int kScoutBlock = ScoutBlock<SEQ>::value;
     const size_t s_tab = kGrid ? 0 : 16 + (size_t)TAB_NARR * ctx->n * sizeof(double);
-    const bool s_in = !kGrid && s_tab <= (size_t)max_optin;
+    const bool s_in = !kGrid && !IsEns<A>::value && s_tab <= (size_t)max_optin;     // the ensemble scout reads its tables from global memory
     const void* sfn;
-    if constexpr (kGrid) sfn = scout_kernel_fn<SEQ, false, MSRC>();
-    else sfn = s_in ? scout_kernel_fn<SEQ, true, MSRC>() : scout_kernel_fn<SEQ, false, MSRC>();
+    if constexpr (kGrid) sfn = scout_kernel_fn<SEQ, false, A>();
+    else sfn = s_in ? scout_kernel_fn<SEQ, true, A>() : scout_kernel_fn<SEQ, false, A>();
     const size_t s_smem = s_in ? s_tab : 16;
     CK(cudaFuncSetAttribute(sfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s_smem));
     int s_per_sm = 1;
@@ -556,8 +658,8 @@ static int launch_cost_scout(geoac_ctx* ctx, const KernelArgs<MSRC>& a, int max_
 // Step 1: the longest-predicted-ray-first claim order (trace_kernel.cuh): cost scout, (range-dependent sets) cost dilation, sort.
 // Sets a.order, a.n_claims, a.packet_refill and a.n_long_packets; n_quarter = long packets long enough for quarter claims.
 // `lanes` = lanes of the main launch (the average work of a lane is the scout's cost sum over them).
-template <class EQ, bool MSRC>
-static int build_claim_order(geoac_ctx* ctx, KernelArgs<MSRC>& a, long long lanes, int max_optin, cudaStream_t st, int64_t& n_quarter) {
+template <class EQ, class A>
+static int build_claim_order(geoac_ctx* ctx, A& a, long long lanes, int max_optin, cudaStream_t st, int64_t& n_quarter) {
     constexpr bool kGrid = PacketMode<EQ>::value;
     constexpr int group = kGrid ? 32 : 1;                     // range-dependent sets: packets of 32 consecutive rays
     const int64_t n = a.n_rays, n_entries = ((n + group - 1) / group) * group;
@@ -569,7 +671,7 @@ static int build_claim_order(geoac_ctx* ctx, KernelArgs<MSRC>& a, long long lane
     uint32_t* cmax = ctx->d_hist.p + kCostBuckets;
     uint32_t* n_long = cmax + 1;                              // n_long[1]: quarter packets
     unsigned long long* cost_sum = reinterpret_cast<unsigned long long*>(cmax + 4);
-    if (int rc = launch_cost_scout<typename EQ::Scout, MSRC>(ctx, a, max_optin, st, cmax, cost_sum)) return rc;
+    if (int rc = launch_cost_scout<typename EQ::Scout>(ctx, a, max_optin, st, cmax, cost_sum)) return rc;
     if (kGrid) {
         const uint32_t* cost = ctx->d_cost.p;
         if (ctx->knobs.dilate > 0) {
@@ -676,8 +778,8 @@ static int enqueue_launches(geoac_ctx* ctx, const void* fn, size_t smem, int max
     return GEOAC_OK;
 }
 
-template <class EQ, int BLOCK, bool PATHS, bool MSRC>
-static int launch_trace(geoac_ctx* ctx, KernelArgs<MSRC> a, cudaStream_t st) {
+template <class EQ, int BLOCK, bool PATHS, class A>
+static int launch_trace(geoac_ctx* ctx, A a, cudaStream_t st) {
     constexpr bool kGrid = PacketMode<EQ>::value;
     const size_t lane_doubles = ((size_t)LaneLayout<EQ>::STRIDE * BLOCK + 1) & ~(size_t)1;
     const size_t fixed = ((sizeof(LaunchConsts) + 15) / 16) * 16 + 16 + lane_doubles * sizeof(double);
@@ -685,12 +787,12 @@ static int launch_trace(geoac_ctx* ctx, KernelArgs<MSRC> a, cudaStream_t st) {
     int max_optin = 0;
     CK(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
     if (fixed > (size_t)max_optin) return fail(ctx, GEOAC_ERR_CUDA, "lane records do not fit in shared memory");
-    const bool in_smem = !kGrid && fixed + tab_bytes <= (size_t)max_optin;
+    const bool in_smem = !kGrid && !IsEns<A>::value && fixed + tab_bytes <= (size_t)max_optin;
     const size_t smem = in_smem ? fixed + tab_bytes : fixed;
-    // the range-dependent node tables, and a profile too large for shared memory, are read through L1 / L2
+    // the range-dependent node tables, a profile too large for shared memory and the ensemble's tables are read through L1 / L2
     const void* fn;
-    if constexpr (kGrid) fn = trace_kernel_fn<EQ, BLOCK, false, PATHS, MSRC>();
-    else fn = in_smem ? trace_kernel_fn<EQ, BLOCK, true, PATHS, MSRC>() : trace_kernel_fn<EQ, BLOCK, false, PATHS, MSRC>();
+    if constexpr (kGrid) fn = trace_kernel_fn<EQ, BLOCK, false, PATHS, A>();
+    else fn = in_smem ? trace_kernel_fn<EQ, BLOCK, true, PATHS, A>() : trace_kernel_fn<EQ, BLOCK, false, PATHS, A>();
     CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 1;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, BLOCK, smem));
@@ -710,7 +812,7 @@ static int launch_trace(geoac_ctx* ctx, KernelArgs<MSRC> a, cudaStream_t st) {
     const int lpt_mode = ctx->knobs.lpt;
     if ((lpt_mode == 2 || (lpt_mode == 1 && a.n_rays > (int64_t)grid * BLOCK)) && a.n_rays < ((int64_t)1 << 32)) {
         int64_t n_quarter = 0;
-        if (int rc = build_claim_order<EQ, MSRC>(ctx, a, (long long)grid * BLOCK, max_optin, st, n_quarter)) return rc;
+        if (int rc = build_claim_order<EQ>(ctx, a, (long long)grid * BLOCK, max_optin, st, n_quarter)) return rc;
         grid_long = size_long_region(ctx, a, n_quarter, BLOCK, PATHS);
     }
     ctx->last_long_packets = (int)a.n_long_packets;
@@ -719,28 +821,34 @@ static int launch_trace(geoac_ctx* ctx, KernelArgs<MSRC> a, cudaStream_t st) {
 }
 
 // variant -> (equation set, lanes per CTA); PATHS: the raypath / caustic capture kernels (same lanes per SM as the plain ones);
-// MSRC: the many-source record kernels (a.src_consts, a.src_id)
-template <bool PATHS, bool MSRC = false>
-static int dispatch_trace(geoac_ctx* ctx, const KernelArgs<MSRC>& a, cudaStream_t st) {
+// A = TraceArgsMS: the many-source record kernels (a.src_consts, a.src_id); A = TraceArgsEns: the ensemble record kernels
+// (stratified sets only)
+template <bool PATHS, class A>
+static int dispatch_trace(geoac_ctx* ctx, const A& a, cudaStream_t st) {
     const bool amp = ctx->prm.calc_amp != 0;
     switch (ctx->variant) {
-        case GEOAC_2D:     return amp ? launch_trace<Eq2D<true>, 512, PATHS, MSRC>(ctx, a, st) : launch_trace<Eq2D<false>, 512, PATHS, MSRC>(ctx, a, st);
+        case GEOAC_2D:     return amp ? launch_trace<Eq2D<true>, 512, PATHS>(ctx, a, st) : launch_trace<Eq2D<false>, 512, PATHS>(ctx, a, st);
         // Eq3D<true>: 384 lanes = 3 warps per scheduler at <= 168 registers, no spills (420 ms per config-2 pass vs 491 (256) /
         // 494 (512) in round 1).  Nothing in between exists: the register file is four 16 K-register banks, one per scheduler, so
         // 13 or 14 warps put 4 on some scheduler and cap every lane at 128 registers -- the 512-lane case, which spills (measured
         // on B200: 416 / 448 lanes at 152 / 144 registers compile without spills but do not fit on an SM).
-        case GEOAC_3D:     return amp ? launch_trace<Eq3D<true>, 384, PATHS, MSRC>(ctx, a, st) : launch_trace<Eq3D<false>, 512, PATHS, MSRC>(ctx, a, st);
-        case GEOAC_GLOBAL: return amp ? launch_trace<EqGlobal<true>, 384, PATHS, MSRC>(ctx, a, st) : launch_trace<EqGlobal<false>, 512, PATHS, MSRC>(ctx, a, st);
-        case GEOAC_3D_RNGDEP:     return amp ? launch_trace<Eq3DRD<true>, 128, PATHS, MSRC>(ctx, a, st)     : launch_trace<Eq3DRD<false>, 128, PATHS, MSRC>(ctx, a, st);
-        case GEOAC_GLOBAL_RNGDEP: return amp ? launch_trace<EqGlobalRD<true>, 128, PATHS, MSRC>(ctx, a, st) : launch_trace<EqGlobalRD<false>, 128, PATHS, MSRC>(ctx, a, st);
+        case GEOAC_3D:     return amp ? launch_trace<Eq3D<true>, 384, PATHS>(ctx, a, st) : launch_trace<Eq3D<false>, 512, PATHS>(ctx, a, st);
+        case GEOAC_GLOBAL: return amp ? launch_trace<EqGlobal<true>, 384, PATHS>(ctx, a, st) : launch_trace<EqGlobal<false>, 512, PATHS>(ctx, a, st);
+    }
+    if constexpr (!IsEns<A>::value) {
+        switch (ctx->variant) {
+            case GEOAC_3D_RNGDEP:     return amp ? launch_trace<Eq3DRD<true>, 128, PATHS>(ctx, a, st)     : launch_trace<Eq3DRD<false>, 128, PATHS>(ctx, a, st);
+            case GEOAC_GLOBAL_RNGDEP: return amp ? launch_trace<EqGlobalRD<true>, 128, PATHS>(ctx, a, st) : launch_trace<EqGlobalRD<false>, 128, PATHS>(ctx, a, st);
+        }
     }
     return fail(ctx, GEOAC_ERR_BAD_ARG, "variant not implemented");
 }
 
 // One trace on `st`: zeroes the records and counters, fills in the context's part of `a` and launches.  The caller sets the
-// rays (theta, phi, n_rays) and their outputs (rec, status, n_steps), the capture fields (zero: no capture) and, for rays
-// from several sources (A = TraceArgsMS, no capture), src_consts and src_id.  The launch invariants must be current
-// (refresh_consts) and ordered before `st`.
+// rays (theta, phi, n_rays) and their outputs (rec, status, n_steps), the capture fields (zero: no capture), for rays from
+// several sources (A = TraceArgsMS, no capture) src_consts and src_id, and for rays through the ensemble's members
+// (A = TraceArgsEns, no capture) atm_id.  The launch invariants must be current (refresh_consts; refresh_ensemble for
+// TraceArgsEns) and ordered before `st`.
 template <class A>
 static int enqueue_trace(geoac_ctx* ctx, A a, cudaStream_t st) {
     const int n_rec = ctx->prm.bounces + 1;
@@ -754,7 +862,13 @@ static int enqueue_trace(geoac_ctx* ctx, A a, cudaStream_t st) {
     a.sbpoly = (ctx->is_grid || !ctx->knobs.sbpoly) ? nullptr : ctx->d_sbpoly.p;   // knob sbpoly = 0: the full absorption model at every step (A/B measurements, tests)
     a.consts = ctx->d_consts.p; a.n_rec = n_rec;
     a.counter = ctx->d_counters.p; a.total_steps = ctx->d_counters.p + 1; a.warp_trips = ctx->d_counters.p + 2;
-    if constexpr (std::is_same<A, TraceArgsMS>::value) return dispatch_trace<false, true>(ctx, a, st);
+    if constexpr (IsEns<A>::value) {
+        // the members' invariants and tables; the descriptors without polynomials for knob sbpoly = 0.  The scout reads only
+        // parameters from a.consts, the same in every member.
+        a.atm_consts = ctx->d_ens_consts.p; a.consts = a.atm_consts;
+        a.atm_tab = ctx->d_ens_tab.p + (ctx->knobs.sbpoly ? 0 : ctx->ens_n); a.atm_tab_scout = ctx->d_ens_tab.p + 2 * ctx->ens_n;
+    }
+    if constexpr (!std::is_same<A, TraceArgs>::value) return dispatch_trace<false>(ctx, a, st);
     else return (a.path_stride > 0 || a.caus_cap > 0) ? dispatch_trace<true>(ctx, a, st) : dispatch_trace<false>(ctx, a, st);
 }
 
@@ -824,12 +938,17 @@ struct CaptureOut { int64_t cap = 0; double* data = nullptr; int32_t* rows = nul
 // Rays from several sources (geoac_trace_sources, already validated): ray r starts from src[id[r]], n rows of 3 doubles.
 // id == nullptr: every ray starts from params.src.
 struct Sources { int n = 0; const double* src = nullptr; const int32_t* id = nullptr; };
+// Rays through the members of the context's ensemble (geoac_trace_ensemble, already validated): ray r through member id[r].
+// id == nullptr: every ray through the context's atmosphere.
+struct Members { const int32_t* id = nullptr; };
 
-// The host-buffer trace (geoac_trace, geoac_trace_paths, geoac_trace_paths_compact, geoac_trace_sources, each context of
-// geoac_trace_multi): angles in, one trace on ctx->stream, records out, plus the raypath rows (every path_stride steps) and
-// caustic events asked for.  With `srcs`, the rays start from their own sources (no capture).
+// The host-buffer trace (geoac_trace, geoac_trace_paths, geoac_trace_paths_compact, geoac_trace_sources, geoac_trace_ensemble,
+// each context of geoac_trace_multi): angles in, one trace on ctx->stream, records out, plus the raypath rows (every
+// path_stride steps) and caustic events asked for.  With `srcs`, the rays start from their own sources; with `mems`, they run
+// through their own members of the ensemble (either: no capture).
 static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps,
-                      Capture mode = Capture::none, int path_stride = 0, CaptureOut path = {}, CaptureOut caus = {}, Sources srcs = {}) {
+                      Capture mode = Capture::none, int path_stride = 0, CaptureOut path = {}, CaptureOut caus = {}, Sources srcs = {},
+                      Members mems = {}) {
     if (!ctx || n_rays < 0 || (n_rays > 0 && (!theta || !phi || !rec || !status || !n_steps))) return GEOAC_ERR_BAD_ARG;
     const bool compact = mode == Capture::compact;
     auto has_rows = [&](const CaptureOut& c) { return compact ? c.offs != nullptr : c.rows != nullptr; };
@@ -845,7 +964,7 @@ static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const
     if (compact && path_stride > 0) path.offs[0] = 0;
     if (compact && caus.cap > 0) caus.offs[0] = 0;
     if (n_rays == 0) return GEOAC_OK;
-    if (!ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, "set an atmosphere first");
+    if (mems.id ? !ctx->ens_n : !ctx->have_atmo) return fail(ctx, GEOAC_ERR_NO_ATMO, mems.id ? "set an ensemble first (geoac_set_ensemble_1d)" : "set an atmosphere first");
     cudaSetDevice(ctx->device);
     const int64_t n_slots = n_rays * (ctx->prm.bounces + 1);
     if (int rc = reserve_staging(ctx, n_rays)) return rc;
@@ -861,25 +980,37 @@ static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const
         if (!compact) CK(cudaMemsetAsync(s.data.p, 0, bytes, st));       // the caller receives every slot; compaction copies only rows produced
         CK(cudaMemsetAsync(s.rows.p, 0, sizeof(int32_t) * n_rays, st));
     }
-    TraceArgsMS a{};                                                     // the source fields are used with `srcs` only
+    TraceArgs a{};
     a.theta = ctx->d_theta.p; a.phi = ctx->d_phi.p; a.n_rays = n_rays; a.rec = ctx->d_rec.p; a.status = ctx->d_status.p; a.n_steps = ctx->d_nsteps.p;
     if (path_stride > 0) { a.path = ctx->d_path.p; a.path_rows = ctx->d_path_rows.p; a.path_stride = path_stride; a.path_cap = path.cap; }
     if (caus.cap > 0) { a.caus = ctx->d_caus.p; a.caus_rows = ctx->d_caus_rows.p; a.caus_cap = caus.cap; }
     if (srcs.id) {
         CK(ctx->d_src.grow(sizeof(double) * 3 * srcs.n)); CK(ctx->d_src_consts.grow(sizeof(LaunchConsts) * srcs.n));
         CK(ctx->d_src_id.grow(sizeof(int32_t) * n_rays));
-        a.src_consts = ctx->d_src_consts.p; a.src_id = ctx->d_src_id.p;
     }
+    if (mems.id) CK(ctx->d_atm_id.grow(sizeof(int32_t) * n_rays));
     CK(cudaMemcpyAsync(ctx->d_theta.p, theta, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(ctx->d_phi.p, phi, sizeof(double) * n_rays, cudaMemcpyHostToDevice, st));
     if (srcs.id) {
         CK(cudaMemcpyAsync(ctx->d_src.p, srcs.src, sizeof(double) * 3 * srcs.n, cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(ctx->d_src_id.p, srcs.id, sizeof(int32_t) * n_rays, cudaMemcpyHostToDevice, st));
     }
-    if (int rc = refresh_consts(ctx)) return rc;                         // before ev0: the timed window holds the trace alone
+    if (mems.id) CK(cudaMemcpyAsync(ctx->d_atm_id.p, mems.id, sizeof(int32_t) * n_rays, cudaMemcpyHostToDevice, st));
+    // before ev0: the timed window holds the trace alone
+    if (int rc = mems.id ? refresh_ensemble(ctx) : refresh_consts(ctx)) return rc;
     if (srcs.id) { if (int rc = setup_consts(ctx, ctx->d_src_consts.p, ctx->d_src.p, srcs.n)) return rc; }
     CK(cudaEventRecord(ctx->ev0, st));
-    if (int rc = srcs.id ? enqueue_trace(ctx, a, st) : enqueue_trace(ctx, static_cast<const TraceArgs&>(a), st)) return rc;
+    int rc = GEOAC_OK;
+    if (srcs.id) {
+        TraceArgsMS m{}; static_cast<TraceArgs&>(m) = a;
+        m.src_consts = ctx->d_src_consts.p; m.src_id = ctx->d_src_id.p;
+        rc = enqueue_trace(ctx, m, st);
+    } else if (mems.id) {
+        TraceArgsEns e{}; static_cast<TraceArgs&>(e) = a;
+        e.atm_id = ctx->d_atm_id.p;
+        rc = enqueue_trace(ctx, e, st);
+    } else rc = enqueue_trace(ctx, a, st);
+    if (rc) return rc;
     CK(cudaEventRecord(ctx->ev1, st));
     CK(cudaMemcpyAsync(rec, ctx->d_rec.p, sizeof(double) * GEOAC_NFIELDS * n_slots, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(status, ctx->d_status.p, sizeof(int32_t) * n_slots, cudaMemcpyDeviceToHost, st));
@@ -937,6 +1068,20 @@ extern "C" int geoac_trace_sources(geoac_ctx* ctx, int n_src, const double* src,
             return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: src_id of ray " + std::to_string(r) + " is " + std::to_string(src_id[r])
                                                 + ", outside [0, " + std::to_string(n_src) + ")");
     return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, Capture::none, 0, {}, {}, { n_src, src, src_id });
+}
+
+extern "C" int geoac_trace_ensemble(geoac_ctx* ctx, int64_t n_rays, const int32_t* atm_id, const double* theta, const double* phi,
+                                    double* rec, int32_t* status, int32_t* n_steps) {
+    if (!ctx) return GEOAC_ERR_BAD_ARG;
+    if (n_rays < 0) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_ensemble: n_rays < 0");
+    if (n_rays == 0) return GEOAC_OK;
+    if (!atm_id || !theta || !phi || !rec || !status || !n_steps) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_ensemble: need non-null buffers");
+    if (!ctx->ens_n) return fail(ctx, GEOAC_ERR_NO_ATMO, "geoac_trace_ensemble: set an ensemble first (geoac_set_ensemble_1d)");
+    for (int64_t r = 0; r < n_rays; r++)
+        if (atm_id[r] < 0 || atm_id[r] >= ctx->ens_n)
+            return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_ensemble: atm_id of ray " + std::to_string(r) + " is " + std::to_string(atm_id[r])
+                                                + ", outside [0, " + std::to_string(ctx->ens_n) + ")");
+    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, Capture::none, 0, {}, {}, {}, { atm_id });
 }
 
 extern "C" int geoac_trace_paths(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi,

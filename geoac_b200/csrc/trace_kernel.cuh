@@ -63,7 +63,18 @@ struct TraceArgsMS : TraceArgs {
     const LaunchConsts* src_consts;
     const int32_t* src_id;
 };
-template <bool MSRC> using KernelArgs = std::conditional_t<MSRC, TraceArgsMS, TraceArgs>;
+// Arguments of the ensemble kernels (stratified sets): ray r is traced through member atm_id[r] of an ensemble of 1-D
+// profiles, with that member's invariants atm_consts[m] and table atm_tab[m] (base, n, xmin, xmax, sbpoly; jump_scale 0).
+// The cost scout reads atm_tab_scout[m] instead (the same table with jump_scale = (n-1)/(xmax-xmin), no sbpoly).  All of
+// them in global memory, read through L1.
+struct TraceArgsEns : TraceArgs {
+    const LaunchConsts* atm_consts;
+    const Table1D* atm_tab;
+    const Table1D* atm_tab_scout;
+    const int32_t* atm_id;
+};
+template <class ARGS> struct IsMSrc { static constexpr bool value = std::is_same<ARGS, TraceArgsMS>::value; };
+template <class ARGS> struct IsEns { static constexpr bool value = std::is_same<ARGS, TraceArgsEns>::value; };
 
 // Per-launch invariants of the stratified variants (source / ground / reference-level atmosphere samples and the
 // Sutherland-Bass reference state), evaluated once with the same spline routines the rays use.
@@ -335,19 +346,30 @@ template <class EQ> struct LaneLayout {
     static constexpr int STRIDE = (WORK + EXTRA) | 1;
 };
 
-// The invariants a ray is traced with: the launch's (L) or, in the many-source kernels, those of the ray's own source s, read
-// from global memory through L1 (a warp whose rays share a source reads one address).  Rays keep the caller's order among
-// equal claim keys, so a batch laid out source by source gives warps of mostly one source.
-template <bool MSRC>
-__device__ __forceinline__ const LaunchConsts& ray_consts(const LaunchConsts& L, const KernelArgs<MSRC>& a, int s) {
-    if constexpr (MSRC) return a.src_consts[s];
+// The invariants a ray is traced with: the launch's (L) or, in the many-source kernels, those of the ray's own source s (in
+// the ensemble kernels: of its member s), read from global memory through L1 (a warp whose rays share a source reads one
+// address).  Rays keep the caller's order among equal claim keys, so a batch laid out source by source (member by member)
+// gives warps of mostly one source (member).
+template <class ARGS>
+__device__ __forceinline__ const LaunchConsts& ray_consts(const LaunchConsts& L, const ARGS& a, int s) {
+    if constexpr (IsMSrc<ARGS>::value) return a.src_consts[s];
+    else if constexpr (IsEns<ARGS>::value) return a.atm_consts[s];
     else return L;
 }
+// The atmosphere a ray is traced through: the launch's (T) or, in the ensemble kernels, the table of its member s -- a
+// reference into global memory, not a register copy.
+template <class ARGS, class ATMO>
+__device__ __forceinline__ const ATMO& ray_atmo(const ATMO& T, const ARGS& a, int s) {
+    if constexpr (IsEns<ARGS>::value) return a.atm_tab[s];
+    else return T;
+}
 
-// ARGS: TraceArgs, or TraceArgsMS for the many-source kernels (MSRC)
+// ARGS: TraceArgs, TraceArgsMS for the many-source kernels (MSRC) or TraceArgsEns for the ensemble kernels (ENS, stratified
+// sets, TABLE_IN_SMEM = false)
 template <class EQ, int BLOCK, bool TABLE_IN_SMEM, bool PATHS = false, class ARGS = TraceArgs>
 __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__ ARGS a) {
-    constexpr bool MSRC = std::is_same<ARGS, TraceArgsMS>::value;
+    constexpr bool MSRC = IsMSrc<ARGS>::value, ENS = IsEns<ARGS>::value;
+    static_assert(!ENS || (!TABLE_IN_SMEM && !PacketMode<EQ>::value), "the ensemble kernels read 1-D tables from global memory");
     constexpr int NEQ = EQ::NEQ;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // layout: [LaunchConsts][mbarrier][lane records: BLOCK x STRIDE doubles][table]
@@ -356,7 +378,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
     double* lanes = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(bar) + 16);
     double* tab_s = lanes + ((LaneLayout<EQ>::STRIDE * BLOCK + 1) & ~1);          // keep the table 16-byte aligned
 
-    if constexpr (!MSRC) {                      // the many-source kernels read each ray's invariants from a.src_consts instead
+    if constexpr (!MSRC && !ENS) {              // the many-source / ensemble kernels read each ray's invariants from global memory instead
         for (int i = threadIdx.x; i < (int)(sizeof(LaunchConsts) / 8); i += BLOCK)
             reinterpret_cast<double*>(Ls)[i] = reinterpret_cast<const double*>(a.consts)[i];
     }
@@ -383,7 +405,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
     o.caus = a.caus; o.caus_rows = a.caus_rows; o.caus_cap = a.caus_cap;
     LaneD<EQ>& ld = *reinterpret_cast<LaneD<EQ>*>(lanes + (size_t)threadIdx.x * LaneLayout<EQ>::STRIDE);
     LaneI<EQ> li;
-    int rsrc = 0;                      // MSRC: source of the lane's ray
+    int rsrc = 0;                      // MSRC: source of the lane's ray; ENS: its member
     // y_{k-1} history (quadratic intercept only): [eq][global thread] in an L2-resident global scratch, written once per step
     const int64_t pstride = (int64_t)gridDim.x * BLOCK;
     double* prev = a.prev + ((int64_t)blockIdx.x * BLOCK + threadIdx.x);
@@ -432,7 +454,8 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
                     const int64_t r = a.order ? (int64_t)a.order[idx] : idx;
                     if (r < a.n_rays) {
                         if constexpr (MSRC) rsrc = a.src_id[r];
-                        lane_start<EQ>(ld, li, ray_consts<MSRC>(L, a, rsrc), T, r, a.theta[r], a.phi[r]); have_ray = true;
+                        if constexpr (ENS) rsrc = a.atm_id[r];
+                        lane_start<EQ>(ld, li, ray_consts(L, a, rsrc), ray_atmo(T, a, rsrc), r, a.theta[r], a.phi[r]); have_ray = true;
                     }
                 }
             }
@@ -452,7 +475,8 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
                         const int64_t r = a.order ? (int64_t)a.order[idx] : idx;
                         if (r < a.n_rays) {
                             if constexpr (MSRC) rsrc = a.src_id[r];
-                            lane_start<EQ>(ld, li, ray_consts<MSRC>(L, a, rsrc), T, r, a.theta[r], a.phi[r]); have_ray = true;
+                            if constexpr (ENS) rsrc = a.atm_id[r];
+                            lane_start<EQ>(ld, li, ray_consts(L, a, rsrc), ray_atmo(T, a, rsrc), r, a.theta[r], a.phi[r]); have_ray = true;
                         }
                     }
                     else exhausted = true;
@@ -480,7 +504,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
             gi.ray = __shfl_sync(0xffffffffu, (long long)li.ray, owner);
             gi.path_n = __shfl_sync(0xffffffffu, li.path_n, owner); gi.caus_n = __shfl_sync(0xffffffffu, li.caus_n, owner);
             gi.caus_b = PATHS ? __shfl_sync(0xffffffffu, li.caus_b, owner) : 0;
-            const int gsrc = MSRC ? __shfl_sync(0xffffffffu, rsrc, owner) : 0;     // a ray keeps its source: nothing to hand back
+            const int gsrc = (MSRC || ENS) ? __shfl_sync(0xffffffffu, rsrc, owner) : 0;     // a ray keeps its source: nothing to hand back
             const int othread = (int)(threadIdx.x & ~31u) + owner;
             double* const rec = lanes + (size_t)othread * LaneLayout<EQ>::STRIDE;
             double* const gwork = rec + LaneLayout<EQ>::WORK;
@@ -488,7 +512,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
             Tg.scratch = gwork + 2 * NEQ;
             if (coop) { Tg.role = (int)lane & 3; Tg.nrole = 4; Tg.glane0 = (int)lane & ~3; Tg.gmask = 0xFu << ((int)lane & ~3); }
             bool alive = false;
-            if (run) alive = lane_advance<EQ, PATHS>(*reinterpret_cast<LaneD<EQ>*>(rec), gi, ray_consts<MSRC>(L, a, gsrc), Tg,
+            if (run) alive = lane_advance<EQ, PATHS>(*reinterpret_cast<LaneD<EQ>*>(rec), gi, ray_consts(L, a, gsrc), Tg,
                                                        a.prev + ((int64_t)blockIdx.x * BLOCK + othread), pstride, o, gwork);
             // hand the integer state back to the lane that owns the ray (itself in serial mode)
             const int src = (coop && have_ray) ? 4 * __popc(act & ((1u << lane) - 1u)) : (int)lane;
@@ -505,7 +529,7 @@ __global__ void __launch_bounds__(BLOCK, 1) trace_kernel(const __grid_constant__
             }
         } else {
             if (have_ray) {
-                have_ray = lane_advance<EQ, PATHS>(ld, li, ray_consts<MSRC>(L, a, rsrc), T, prev, pstride, o, work);
+                have_ray = lane_advance<EQ, PATHS>(ld, li, ray_consts(L, a, rsrc), ray_atmo(T, a, rsrc), prev, pstride, o, work);
                 my_steps++;
             }
         }
@@ -528,14 +552,23 @@ constexpr int kCostBuckets = 256;
 // lanes per CTA of the scout: 512 (<= 128 registers) for the stratified sets, 256 for the range-dependent sampler
 template <class EQ> struct ScoutBlock { static constexpr int value = std::is_same<typename EQ::Atmo, Grid3D>::value ? 256 : 512; };
 
+// The atmosphere the scout predicts a ray in: the launch's (T) or, in the ensemble scout, the table of its member s.
+template <class ARGS, class ATMO>
+__device__ __forceinline__ const ATMO& scout_atmo(const ATMO& T, const ARGS& a, int s) {
+    if constexpr (IsEns<ARGS>::value) return a.atm_tab_scout[s];
+    else return T;
+}
+
 // Persistent like the trace kernel: lanes are refilled from a counter as their rays end (a warp of rays with different
 // lifetimes never idles), the 1-D table sits in shared memory; the ray state (<= 6 equations, no auxiliary set) fits
 // in registers.
-// ARGS = TraceArgsMS (MSRC): each ray is predicted with its own source's invariants (ray_consts).
+// ARGS = TraceArgsMS (MSRC): each ray is predicted with its own source's invariants (ray_consts).  ARGS = TraceArgsEns (ENS):
+// with its own member's invariants and table (atm_tab_scout); a.consts is then any member's (only the parameters are read).
 template <class EQ, bool TABLE_IN_SMEM, class ARGS = TraceArgs>
 __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const __grid_constant__ ARGS a, uint32_t* cost, uint32_t* cost_max,
                                                                unsigned long long* cost_sum, unsigned long long* counter, int coarse) {
-    constexpr bool MSRC = std::is_same<ARGS, TraceArgsMS>::value;
+    constexpr bool MSRC = IsMSrc<ARGS>::value, ENS = IsEns<ARGS>::value;
+    static_assert(!ENS || !TABLE_IN_SMEM, "the ensemble scout reads 1-D tables from global memory");
     constexpr int NEQ = EQ::NEQ;
     constexpr bool kGrid = std::is_same<typename EQ::Atmo, Grid3D>::value;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -572,7 +605,8 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
                 if (ray < a.n_rays) {
                     cur = typename EQ::Cursor{};
                     if constexpr (MSRC) rsrc = a.src_id[ray];
-                    EQ::init(ray_consts<MSRC>(L, a, rsrc), T, a.theta[ray], a.phi[ray], rc, y, cur);
+                    if constexpr (ENS) rsrc = a.atm_id[ray];
+                    EQ::init(ray_consts(L, a, rsrc), scout_atmo(T, a, rsrc), a.theta[ray], a.phi[ray], rc, y, cur);
 #pragma unroll
                     for (int i = 0; i < NEQ; i++) ym1[i] = y[i];
                     est = 0; seg = 0; bounce = 0; have_ray = true;
@@ -581,14 +615,15 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
         }
         if (!__any_sync(0xffffffffu, have_ray)) break;
         if (!have_ray) continue;
-        const LaunchConsts& Lr = ray_consts<MSRC>(L, a, rsrc);
+        const LaunchConsts& Lr = ray_consts(L, a, rsrc);
+        const typename EQ::Atmo& Tr = scout_atmo(T, a, rsrc);
         double acc[NEQ], p[NEQ], f[NEQ];
         const double ds = (double)coarse * EQ::step_size(Lr, y);
 #pragma unroll
         for (int i = 0; i < NEQ; i++) { acc[i] = y[i]; p[i] = y[i]; }
 #pragma unroll 1
         for (int s = 0; s < 4; s++) {
-            const double sc = EQ::rhs(Lr, T, rc, p, f, cur);
+            const double sc = EQ::rhs(Lr, Tr, rc, p, f, cur);
             const double dsa = ds * ((s == 2) ? 1.0 : 0.5) * sc, dsb = ds * ((s == 0 || s == 3) ? (1.0 / 6.0) : (1.0 / 3.0)) * sc;
 #pragma unroll
             for (int i = 0; i < NEQ; i++) { acc[i] = fma(f[i], dsb, acc[i]); p[i] = fma(f[i], dsa, y[i]); }
@@ -599,7 +634,7 @@ __global__ void __launch_bounds__(ScoutBlock<EQ>::value, 1) scout_kernel(const _
             if (bounce >= L.bounces) done = true;
             else {
                 double y0[NEQ];
-                EQ::reflect(Lr, T, rc, ym1, y, acc, y0, cur);
+                EQ::reflect(Lr, Tr, rc, ym1, y, acc, y0, cur);
 #pragma unroll
                 for (int i = 0; i < NEQ; i++) { acc[i] = y0[i]; y[i] = y0[i]; }      // restart: y = ym1 = reflected state
                 bounce++; seg = 0;
@@ -786,14 +821,28 @@ __global__ void stable_scatter_kernel(const uint8_t* key, const uint32_t* src, i
 // single-source kernels; a caller passing global-memory invariants in the same unit would turn its shared loads generic.
 template <class EQ, int BLOCK, bool TABLE_IN_SMEM> const void* msrc_trace_kernel();
 template <class EQ, bool TABLE_IN_SMEM> const void* msrc_scout_kernel();
-template <class EQ, int BLOCK, bool TABLE_IN_SMEM, bool PATHS, bool MSRC>
+// The ensemble kernels (ARGS = TraceArgsEns), and the set-up of the ensemble's invariants, live in trace_ensemble.cu for the
+// same reason.  They have one table placement (global memory): TABLE_IN_SMEM is ignored.
+template <class EQ, int BLOCK> const void* ens_trace_kernel();
+template <class EQ> const void* ens_scout_kernel();
+// On `st`: the invariants of every member, out[m] = `in` (the parameters, source clamped) filled in from table tab[m] (no
+// sbpoly), then the absorption polynomials of every interval of every member into poly (member m's intervals from
+// iv_off[m] on, n_iv in all).  One thread per member, then one per (member, interval).
+cudaError_t ens_setup(LaunchConsts* out, const LaunchConsts& in, const Table1D* tab, int n_atm, const int64_t* iv_off, int64_t n_iv,
+                      int variant, double* poly, cudaStream_t st);
+template <class EQ, int BLOCK, bool TABLE_IN_SMEM, bool PATHS, class ARGS>
 const void* trace_kernel_fn() {
-    if constexpr (MSRC) return msrc_trace_kernel<EQ, BLOCK, TABLE_IN_SMEM>();
+    if constexpr (IsMSrc<ARGS>::value) return msrc_trace_kernel<EQ, BLOCK, TABLE_IN_SMEM>();
+    else if constexpr (IsEns<ARGS>::value) {
+        static_assert(!PATHS, "the ensemble kernels have no raypath / caustic capture");
+        return ens_trace_kernel<EQ, BLOCK>();
+    }
     else return (const void*)trace_kernel<EQ, BLOCK, TABLE_IN_SMEM, PATHS>;
 }
-template <class EQ, bool TABLE_IN_SMEM, bool MSRC>
+template <class EQ, bool TABLE_IN_SMEM, class ARGS>
 const void* scout_kernel_fn() {
-    if constexpr (MSRC) return msrc_scout_kernel<EQ, TABLE_IN_SMEM>();
+    if constexpr (IsMSrc<ARGS>::value) return msrc_scout_kernel<EQ, TABLE_IN_SMEM>();
+    else if constexpr (IsEns<ARGS>::value) return ens_scout_kernel<EQ>();
     else return (const void*)scout_kernel<EQ, TABLE_IN_SMEM>;
 }
 

@@ -194,6 +194,35 @@ int geoac_trace_device(geoac_ctx* ctx, int64_t n_rays, const double* d_theta, co
 int geoac_trace_sources(geoac_ctx* ctx, int n_src, const double* src, int64_t n_rays, const int32_t* src_id,
                         const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps);
 
+/* An ensemble of n_atm stratified profiles (2D, 3D and Global variants), held by the context next to -- not instead of -- its
+ * own atmosphere.  Member m has levels level_offset[m] .. level_offset[m+1]-1 of z, T, u, v, rho, in the form
+ * geoac_set_atmosphere_1d takes; members may differ in level count and in altitudes.  Each member is checked as
+ * geoac_set_atmosphere_1d checks its profile (>= 3 levels, altitudes strictly increasing; the message names the member).
+ * Sets the propagation region as geoac_set_atmosphere_1d does (GeoAc_SetPropRegion), with vert_limit the lowest top among
+ * the members; geoac_set_params may override it afterwards.  A later call replaces the ensemble; a refused call leaves the
+ * previous one intact.  geoac_trace, geoac_sample_atmosphere and geoac_source_state never read the ensemble, and
+ * geoac_set_atmosphere_1d does not change it.
+ * Errors: GEOAC_ERR_BAD_ARG (NULL context, a range-dependent variant, n_atm < 1, a NULL pointer, level_offset not
+ * non-decreasing from 0, a member refused as above), GEOAC_ERR_CUDA. */
+int geoac_set_ensemble_1d(geoac_ctx* ctx, int n_atm, const int64_t* level_offset /* n_atm + 1 */,
+                          const double* z, const double* T, const double* u, const double* v, const double* rho);
+
+/* geoac_trace() for rays through many atmospheres in one call: ray r is traced at (theta[r], phi[r]) through member atm_id[r]
+ * (in [0, n_atm)) of the ensemble set by geoac_set_ensemble_1d; rec, status, n_steps are laid out exactly as geoac_trace's.
+ * The record, status and step count of ray r are bit for bit what geoac_trace returns for (theta[r], phi[r]) on a context
+ * of the same variant after geoac_set_atmosphere_1d with member atm_id[r]'s arrays, then geoac_set_params with this
+ * context's parameters as they are at this call -- whatever the other rays of the batch, their members and their order.
+ * The context's parameters, its own atmosphere and its invariants are not changed; geoac_last_trace_stats,
+ * geoac_last_trace_counters, geoac_last_schedule and geoac_get_costs report the call like any trace.  The members' tables
+ * are read from global memory (through L1).  Lay the batch out member by member, each member's rays in the mains' loop
+ * order: the claim order keeps the caller's order among rays of equal predicted cost, so warps then hold rays of mostly
+ * one member (their table reads hit one record) and neighbouring paths.  Same concurrency contract as geoac_trace.
+ * Errors, returned before any device work: GEOAC_ERR_BAD_ARG (NULL context, n_rays < 0; with n_rays > 0: a NULL pointer,
+ * an atm_id outside [0, n_atm) -- the message names the first such ray), GEOAC_ERR_NO_ATMO (no ensemble set); n_rays == 0
+ * reads and writes nothing and is GEOAC_OK. */
+int geoac_trace_ensemble(geoac_ctx* ctx, int64_t n_rays, const int32_t* atm_id, const double* theta, const double* phi,
+                         double* rec, int32_t* status, int32_t* n_steps);
+
 /* geoac_trace() plus the raypath rows of the mains' WriteRays=True mode (Code/GeoAc3D_main.cpp:249-262 and siblings; the
  * same call serves `-interactive`, which plots one ray): every `path_stride` steps (the mains use 25) one row of
  * GEOAC_PATH_NF doubles { state[0], state[1], state[2], amplitude (linear, 0 with calc_amp = 0), absorption sum, travel-time
