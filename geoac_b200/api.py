@@ -52,6 +52,8 @@ def lib():
         L.geoac_trace_paths_compact.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _ip, _ip, C.c_int, C.c_int64, C.c_int64, _dp, _lp,
                                                 C.c_int64, C.c_int64, _dp, _lp]
         L.geoac_trace_sources.argtypes = [C.c_void_p, C.c_int, _dp, C.c_int64, _ip, _dp, _dp, _dp, _ip, _ip]
+        L.geoac_trace_sources_paths_compact.argtypes = [C.c_void_p, C.c_int, _dp, C.c_int64, _ip, _dp, _dp, _dp, _ip, _ip,
+                                                        C.c_int, C.c_int64, C.c_int64, _dp, _lp, C.c_int64, C.c_int64, _dp, _lp]
         L.geoac_set_ensemble_1d.argtypes = [C.c_void_p, C.c_int, _lp, _dp, _dp, _dp, _dp, _dp]
         L.geoac_trace_ensemble.argtypes = [C.c_void_p, C.c_int64, _ip, _dp, _dp, _dp, _ip, _ip]
         L.geoac_trace_device.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -72,6 +74,9 @@ def lib():
         L.geoac_eigenray_search.argtypes = [C.c_void_p, C.POINTER(abi.GeoacEigOpts), C.c_int, _dp, C.c_int64, _dp,
                                             C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.geoac_eigenray_direct.argtypes = [C.c_void_p, C.POINTER(abi.GeoacEigOpts), C.c_int, _dp, _dp, _dp, C.POINTER(C.c_int64)]
+        L.geoac_eigenray_search_sources.argtypes = [C.c_void_p, C.POINTER(abi.GeoacEigOpts), C.c_int, _dp, C.c_int, _ip, _dp, C.c_int64, _dp,
+                                                    C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        L.geoac_last_eigenray_ms.argtypes = [C.c_void_p, _dp]
         L.geoac_get_variant.argtypes = [C.c_void_p]
         L.geoac_source_state.argtypes = [C.c_void_p, _dp]
         L.geoac_sample_atmosphere.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp]
@@ -94,7 +99,8 @@ def lib():
 EXPORTED_SYMBOLS = [
     "geoac_create", "geoac_destroy", "geoac_last_error", "geoac_default_params", "geoac_set_atmosphere_1d",
     "geoac_set_atmosphere_3d", "geoac_get_params", "geoac_set_params", "geoac_trace", "geoac_trace_paths", "geoac_trace_device",
-    "geoac_trace_sources", "geoac_set_ensemble_1d", "geoac_trace_ensemble",
+    "geoac_trace_sources", "geoac_set_ensemble_1d", "geoac_trace_ensemble", "geoac_trace_sources_paths_compact",
+    "geoac_eigenray_search_sources", "geoac_last_eigenray_ms",
     "geoac_reserve", "geoac_last_trace_stats", "geoac_last_trace_counters", "geoac_selftest_math", "geoac_load_met_1d", "geoac_load_met_grid", "geoac_eq_count", "geoac_measure_fp64_peak",
     "geoac_get_grid_tables", "geoac_default_eig_opts", "geoac_eigenray_search", "geoac_eigenray_direct", "geoac_get_variant", "geoac_source_state",
     "geoac_sample_atmosphere",
@@ -237,16 +243,21 @@ class Tracer:
         self._check(lib().geoac_set_atmosphere_3d(self._h, len(arrs[0]), len(arrs[1]), len(arrs[2]), *[_p(a) for a in arrs]),
                     "geoac_set_atmosphere_3d")
 
-    def eigenray_search(self, receivers, cap_rows=4096, **opts):
-        """GeoAc3D[.RngDep] -eig_search for one source (params.src) and many receivers [(x, y) km]: rows [n][EIG_NF] (one per
-        GeoAc_EstimateEigenray call of the reference, include/geoac_b200.h) and stats {rounds, rays, found}.
-        opts: theta_min, theta_max, bnc_min, bnc_max, iterations, azimuth_err_lim, d_theta_big, d_theta_small, tolerance."""
+    @staticmethod
+    def _eig_opts(opts):
         o = abi.GeoacEigOpts()
         lib().geoac_default_eig_opts(C.byref(o))
         for k, v in opts.items():
             if not hasattr(o, k):
                 raise TypeError(f"unknown eigenray option {k}")
             setattr(o, k, v)
+        return o
+
+    def eigenray_search(self, receivers, cap_rows=4096, **opts):
+        """GeoAc3D[.RngDep] -eig_search for one source (params.src) and many receivers [(x, y) km]: rows [n][EIG_NF] (one per
+        GeoAc_EstimateEigenray call of the reference, include/geoac_b200.h) and stats {rounds, rays, found}.
+        opts: theta_min, theta_max, bnc_min, bnc_max, iterations, azimuth_err_lim, d_theta_big, d_theta_small, tolerance."""
+        o = self._eig_opts(opts)
         rc = np.ascontiguousarray(receivers, dtype=np.float64).reshape(-1, 2)
         rows = np.zeros((cap_rows, abi.EIG_NF))
         n = C.c_int64(0)
@@ -258,12 +269,7 @@ class Tracer:
     def eigenray_direct(self, receivers, estimates, **opts):
         """-eig_direct: LM search from caller-supplied estimates [(theta_est, phi_est (deg from the x axis), bounces)], one per
         receiver entry; rows as eigenray_search."""
-        o = abi.GeoacEigOpts()
-        lib().geoac_default_eig_opts(C.byref(o))
-        for k, v in opts.items():
-            if not hasattr(o, k):
-                raise TypeError(f"unknown eigenray option {k}")
-            setattr(o, k, v)
+        o = self._eig_opts(opts)
         rc = np.ascontiguousarray(receivers, dtype=np.float64).reshape(-1, 2)
         est = np.ascontiguousarray(estimates, dtype=np.float64).reshape(-1, 3)
         assert len(rc) == len(est)
@@ -271,6 +277,42 @@ class Tracer:
         stats = (C.c_int64 * 3)()
         self._check(lib().geoac_eigenray_direct(self._h, C.byref(o), len(rc), _p(rc), _p(est), _p(rows), stats), "geoac_eigenray_direct")
         return rows, {"rounds": stats[0], "rays": stats[1], "found": stats[2]}
+
+    def eigenray_search_sources(self, src, src_id, receivers, cap_rows=None, **opts):
+        """eigenray_search() from many sources in one call: search i runs from src[src_id[i]] to receivers[i].  src: [n_src, 3],
+        Cartesian (x, y, z) [km], Global (altitude [km], lat [deg], lon [deg]); src_id: int32 [n]; receivers: [n, 2] as for
+        eigenray_search.  Rows as eigenray_search's with column 0 the search index; search i's rows equal those of
+        eigenray_search([receivers[i]]) from its source (include/geoac_b200.h: geoac_eigenray_search_sources).
+        cap_rows: row capacity (default: an estimate; grown and retried once if the library reports it too small)."""
+        o = self._eig_opts(opts)
+        src = np.ascontiguousarray(src, dtype=np.float64)
+        if src.ndim != 2 or src.shape[1] != 3:
+            raise GeoAcError("eigenray_search_sources: src must be an array of shape [n_src, 3]")
+        rc = np.ascontiguousarray(receivers, dtype=np.float64).reshape(-1, 2)
+        src_id = np.asarray(src_id)
+        if src_id.dtype != np.int32 or src_id.shape != (len(rc),):
+            raise GeoAcError("eigenray_search_sources: src_id must be an int32 array with one entry per receiver")
+        src_id = np.ascontiguousarray(src_id)
+        if cap_rows is None:
+            cap_rows = max(1, len(rc) * (o.bnc_max - o.bnc_min + 1) * 8)
+        n = C.c_int64(0)
+        stats = (C.c_int64 * 3)()
+        for attempt in range(2):
+            rows = np.zeros((max(cap_rows, 1), abi.EIG_NF))
+            st = lib().geoac_eigenray_search_sources(self._h, C.byref(o), len(src), _p(src), len(rc), src_id.ctypes.data_as(_ip), _p(rc),
+                                                     cap_rows, _p(rows), C.byref(n), stats)
+            if st == abi.GEOAC_ERR_TOO_LARGE and attempt == 0 and n.value > cap_rows:
+                cap_rows = int(n.value)
+                continue
+            self._check(st, "geoac_eigenray_search_sources")
+            break
+        return rows[:n.value].copy(), {"rounds": stats[0], "rays": stats[1], "found": stats[2]}
+
+    def last_eigenray_ms(self):
+        """Where the time of the last eigenray search went [ms]: host replay of the searches, kernel time of its traces, the call."""
+        ms = np.zeros(3)
+        self._check(lib().geoac_last_eigenray_ms(self._h, _p(ms)), "geoac_last_eigenray_ms")
+        return {"replay_ms": float(ms[0]), "kernel_ms": float(ms[1]), "call_ms": float(ms[2])}
 
     def source_state(self):
         """c, u, v, rho at the source point as the kernels sample them."""
@@ -387,21 +429,44 @@ class Tracer:
         n = len(theta)
         n_rec = self.params.bounces + 1
         out = {"rec": np.empty((abi.NFIELDS, n, n_rec)), "status": np.empty((n, n_rec), dtype=np.int32), "n_steps": np.empty((n, n_rec), dtype=np.int32)}
+        return self._paths_compact(lambda *cap_args: lib().geoac_trace_paths_compact(
+            self._h, n, _p(theta), _p(phi), _p(out["rec"]), out["status"].ctypes.data_as(_ip), out["n_steps"].ctypes.data_as(_ip), *cap_args),
+            "geoac_trace_paths_compact", n, out, stride, cap, caustic_cap, total_rows, total_events)
+
+    def _paths_compact(self, call, what, n, out, stride, cap, caustic_cap, total_rows, total_events):
+        """The capture buffers of a compacted-rows call (call(*capture arguments) -> status), grown and retried once when the
+        library reports them too small; adds them to `out`."""
         total_rows = total_rows if total_rows is not None else max(1, n * min(cap, 1024)) if stride > 0 else 1
         total_events = total_events if total_events is not None else max(1, n * min(max(caustic_cap, 1), 8))
         for attempt in range(2):
             path = np.zeros((max(total_rows, 1), abi.PATH_NF)); poff = np.zeros(n + 1, dtype=np.int64)
             caus = np.zeros((max(total_events, 1), abi.CAUSTIC_NF)); coff = np.zeros(n + 1, dtype=np.int64)
-            rc = lib().geoac_trace_paths_compact(self._h, n, _p(theta), _p(phi), _p(out["rec"]), out["status"].ctypes.data_as(_ip), out["n_steps"].ctypes.data_as(_ip),
-                                                 stride, cap, total_rows, _p(path), poff.ctypes.data_as(C.POINTER(C.c_int64)),
-                                                 caustic_cap, total_events, _p(caus), coff.ctypes.data_as(C.POINTER(C.c_int64)))
+            rc = call(stride, cap, total_rows, _p(path), poff.ctypes.data_as(C.POINTER(C.c_int64)),
+                      caustic_cap, total_events, _p(caus), coff.ctypes.data_as(C.POINTER(C.c_int64)))
             if rc == abi.GEOAC_ERR_TOO_LARGE and attempt == 0:
                 total_rows, total_events = max(total_rows, int(poff[-1])), max(total_events, int(coff[-1]))
                 continue
-            self._check(rc, "geoac_trace_paths_compact")
+            self._check(rc, what)
             break
         out.update(path=path[: poff[-1]], path_offset=poff, caustic=caus[: coff[-1]], caustic_offset=coff)
         return out
+
+    def trace_sources_paths_compact(self, src, src_id, theta, phi, stride=25, cap=2400, caustic_cap=0, total_rows=None, total_events=None):
+        """trace_paths_compact() for rays from many sources in one call: ray r starts from src[src_id[r]] (src, src_id as for
+        trace_sources).  Ray r's records and rows equal those of trace_paths_compact() with params.src = src[src_id[r]]
+        (include/geoac_b200.h: geoac_trace_sources_paths_compact)."""
+        theta, phi, out = self._rays_and_records("trace_sources_paths_compact", theta, phi, None)
+        src = np.ascontiguousarray(src, dtype=np.float64)
+        if src.ndim != 2 or src.shape[1] != 3:
+            raise GeoAcError("trace_sources_paths_compact: src must be an array of shape [n_src, 3]")
+        src_id = np.asarray(src_id)
+        if src_id.dtype != np.int32 or src_id.shape != theta.shape:
+            raise GeoAcError("trace_sources_paths_compact: src_id must be an int32 array with one entry per ray")
+        src_id = np.ascontiguousarray(src_id)
+        return self._paths_compact(lambda *cap_args: lib().geoac_trace_sources_paths_compact(
+            self._h, len(src), _p(src), len(theta), src_id.ctypes.data_as(_ip), _p(theta), _p(phi), _p(out["rec"]),
+            out["status"].ctypes.data_as(_ip), out["n_steps"].ctypes.data_as(_ip), *cap_args),
+            "geoac_trace_sources_paths_compact", len(theta), out, stride, cap, caustic_cap, total_rows, total_events)
 
     def reserve(self, n_rays):
         """Pre-allocate the device staging of trace() for batches of up to n_rays rays."""

@@ -149,12 +149,22 @@ struct geoac_ctx {
     Buf<LaunchConsts> d_ens_consts;
     bool ens_dirty = true;
     Buf<int32_t> d_atm_id;                         // staging of geoac_trace_ensemble: each ray's member
+    // the last eigenray search (eigenray.cu): host ms replaying its chains, summed kernel ms of its traces, ms of the call
+    double eig_ms[3] = { std::numeric_limits<double>::quiet_NaN(), std::numeric_limits<double>::quiet_NaN(), std::numeric_limits<double>::quiet_NaN() };
 };
 
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
     ctx->err = std::string(#call) + ": " + cudaGetErrorString(e_); return GEOAC_ERR_CUDA; } } while (0)
 
 static int fail(geoac_ctx* ctx, int code, const std::string& msg) { if (ctx) ctx->err = msg; return code; }
+// for eigenray.cu, which sees the context only through the C ABI
+int geoac_fail_msg(geoac_ctx* ctx, int code, const std::string& msg) { return fail(ctx, code, msg); }
+void geoac_set_eigenray_ms(geoac_ctx* ctx, const double* ms3) { for (int i = 0; i < 3; i++) ctx->eig_ms[i] = ms3[i]; }
+extern "C" int geoac_last_eigenray_ms(const geoac_ctx* ctx, double* ms3) {
+    if (!ctx || !ms3) return GEOAC_ERR_BAD_ARG;
+    for (int i = 0; i < 3; i++) ms3[i] = ctx->eig_ms[i];
+    return GEOAC_OK;
+}
 
 extern "C" int geoac_eq_count(int variant, int calc_amp) {          // Code/GeoAc/GeoAc.Interface.cpp:21-41
     switch (variant) {
@@ -846,8 +856,8 @@ static int dispatch_trace(geoac_ctx* ctx, const A& a, cudaStream_t st) {
 
 // One trace on `st`: zeroes the records and counters, fills in the context's part of `a` and launches.  The caller sets the
 // rays (theta, phi, n_rays) and their outputs (rec, status, n_steps), the capture fields (zero: no capture), for rays from
-// several sources (A = TraceArgsMS, no capture) src_consts and src_id, and for rays through the ensemble's members
-// (A = TraceArgsEns, no capture) atm_id.  The launch invariants must be current (refresh_consts; refresh_ensemble for
+// several sources (A = TraceArgsMS) src_consts and src_id, and for rays through the ensemble's members (A = TraceArgsEns,
+// no capture) atm_id.  The launch invariants must be current (refresh_consts; refresh_ensemble for
 // TraceArgsEns) and ordered before `st`.
 template <class A>
 static int enqueue_trace(geoac_ctx* ctx, A a, cudaStream_t st) {
@@ -868,7 +878,7 @@ static int enqueue_trace(geoac_ctx* ctx, A a, cudaStream_t st) {
         a.atm_consts = ctx->d_ens_consts.p; a.consts = a.atm_consts;
         a.atm_tab = ctx->d_ens_tab.p + (ctx->knobs.sbpoly ? 0 : ctx->ens_n); a.atm_tab_scout = ctx->d_ens_tab.p + 2 * ctx->ens_n;
     }
-    if constexpr (!std::is_same<A, TraceArgs>::value) return dispatch_trace<false>(ctx, a, st);
+    if constexpr (IsEns<A>::value) return dispatch_trace<false>(ctx, a, st);
     else return (a.path_stride > 0 || a.caus_cap > 0) ? dispatch_trace<true>(ctx, a, st) : dispatch_trace<false>(ctx, a, st);
 }
 
@@ -935,17 +945,17 @@ __global__ void compact_rows_kernel(const double* dense, const int32_t* rows, co
 // total_cap of them; ray i's run from offs[i] to offs[i + 1].
 enum class Capture { none, dense, compact };
 struct CaptureOut { int64_t cap = 0; double* data = nullptr; int32_t* rows = nullptr; int64_t* offs = nullptr; int64_t total_cap = 0; };
-// Rays from several sources (geoac_trace_sources, already validated): ray r starts from src[id[r]], n rows of 3 doubles.
-// id == nullptr: every ray starts from params.src.
+// Rays from several sources (geoac_trace_sources, geoac_trace_sources_paths_compact; already validated): ray r starts from
+// src[id[r]], n rows of 3 doubles.  id == nullptr: every ray starts from params.src.
 struct Sources { int n = 0; const double* src = nullptr; const int32_t* id = nullptr; };
 // Rays through the members of the context's ensemble (geoac_trace_ensemble, already validated): ray r through member id[r].
 // id == nullptr: every ray through the context's atmosphere.
 struct Members { const int32_t* id = nullptr; };
 
-// The host-buffer trace (geoac_trace, geoac_trace_paths, geoac_trace_paths_compact, geoac_trace_sources, geoac_trace_ensemble,
-// each context of geoac_trace_multi): angles in, one trace on ctx->stream, records out, plus the raypath rows (every
+// The host-buffer trace (geoac_trace, geoac_trace_paths, geoac_trace_paths_compact, geoac_trace_sources,
+// geoac_trace_sources_paths_compact, geoac_trace_ensemble, each context of geoac_trace_multi): angles in, one trace on ctx->stream, records out, plus the raypath rows (every
 // path_stride steps) and caustic events asked for.  With `srcs`, the rays start from their own sources; with `mems`, they run
-// through their own members of the ensemble (either: no capture).
+// through their own members of the ensemble (no capture).
 static int trace_host(geoac_ctx* ctx, int64_t n_rays, const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps,
                       Capture mode = Capture::none, int path_stride = 0, CaptureOut path = {}, CaptureOut caus = {}, Sources srcs = {},
                       Members mems = {}) {
@@ -1053,6 +1063,19 @@ extern "C" int geoac_trace(geoac_ctx* ctx, int64_t n_rays, const double* theta, 
     return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps);
 }
 
+// The source arguments of the many-source calls (n_src >= 1, non-null): every coordinate finite, every src_id in
+// [0, n_src).  The message names the call and the first source or ray refused.
+static int check_sources(geoac_ctx* ctx, const char* what, int n_src, const double* src, int64_t n_rays, const int32_t* src_id) {
+    for (int s = 0; s < n_src; s++)
+        if (!std::isfinite(src[3 * (size_t)s]) || !std::isfinite(src[3 * (size_t)s + 1]) || !std::isfinite(src[3 * (size_t)s + 2]))
+            return fail(ctx, GEOAC_ERR_BAD_ARG, std::string(what) + ": coordinates of source " + std::to_string(s) + " are not finite");
+    for (int64_t r = 0; r < n_rays; r++)
+        if (src_id[r] < 0 || src_id[r] >= n_src)
+            return fail(ctx, GEOAC_ERR_BAD_ARG, std::string(what) + ": src_id of ray " + std::to_string(r) + " is " + std::to_string(src_id[r])
+                                                + ", outside [0, " + std::to_string(n_src) + ")");
+    return GEOAC_OK;
+}
+
 extern "C" int geoac_trace_sources(geoac_ctx* ctx, int n_src, const double* src, int64_t n_rays, const int32_t* src_id,
                                    const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps) {
     if (!ctx) return GEOAC_ERR_BAD_ARG;
@@ -1060,14 +1083,24 @@ extern "C" int geoac_trace_sources(geoac_ctx* ctx, int n_src, const double* src,
     if (n_rays == 0) return GEOAC_OK;
     if (n_src < 1 || !src || !src_id || !theta || !phi || !rec || !status || !n_steps)
         return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: need n_src >= 1 and non-null buffers");
-    for (int s = 0; s < n_src; s++)
-        if (!std::isfinite(src[3 * (size_t)s]) || !std::isfinite(src[3 * (size_t)s + 1]) || !std::isfinite(src[3 * (size_t)s + 2]))
-            return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: coordinates of source " + std::to_string(s) + " are not finite");
-    for (int64_t r = 0; r < n_rays; r++)
-        if (src_id[r] < 0 || src_id[r] >= n_src)
-            return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources: src_id of ray " + std::to_string(r) + " is " + std::to_string(src_id[r])
-                                                + ", outside [0, " + std::to_string(n_src) + ")");
+    if (int rc = check_sources(ctx, "geoac_trace_sources", n_src, src, n_rays, src_id)) return rc;
     return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, Capture::none, 0, {}, {}, { n_src, src, src_id });
+}
+
+extern "C" int geoac_trace_sources_paths_compact(geoac_ctx* ctx, int n_src, const double* src, int64_t n_rays, const int32_t* src_id,
+                                                 const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps,
+                                                 int path_stride, int64_t path_cap, int64_t path_total_cap, double* path, int64_t* path_offset,
+                                                 int64_t caustic_cap, int64_t caustic_total_cap, double* caustic, int64_t* caustic_offset) {
+    if (!ctx) return GEOAC_ERR_BAD_ARG;
+    if (n_rays < 0) return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources_paths_compact: n_rays < 0");
+    if (n_rays > 0) {
+        if (n_src < 1 || !src || !src_id || !theta || !phi || !rec || !status || !n_steps)
+            return fail(ctx, GEOAC_ERR_BAD_ARG, "geoac_trace_sources_paths_compact: need n_src >= 1 and non-null buffers");
+        if (int rc = check_sources(ctx, "geoac_trace_sources_paths_compact", n_src, src, n_rays, src_id)) return rc;
+    }
+    return trace_host(ctx, n_rays, theta, phi, rec, status, n_steps, Capture::compact, path_stride,
+                      { path_cap, path, nullptr, path_offset, path_total_cap }, { caustic_cap, caustic, nullptr, caustic_offset, caustic_total_cap },
+                      { n_src, src, src_id });
 }
 
 extern "C" int geoac_trace_ensemble(geoac_ctx* ctx, int64_t n_rays, const int32_t* atm_id, const double* theta, const double* phi,

@@ -821,6 +821,8 @@ __global__ void stable_scatter_kernel(const uint8_t* key, const uint32_t* src, i
 // single-source kernels; a caller passing global-memory invariants in the same unit would turn its shared loads generic.
 template <class EQ, int BLOCK, bool TABLE_IN_SMEM> const void* msrc_trace_kernel();
 template <class EQ, bool TABLE_IN_SMEM> const void* msrc_scout_kernel();
+// Their raypath / caustic capture counterparts (PATHS = true) live in trace_sources_paths.cu, a unit of their own as well.
+template <class EQ, int BLOCK, bool TABLE_IN_SMEM> const void* msrc_paths_trace_kernel();
 // The ensemble kernels (ARGS = TraceArgsEns), and the set-up of the ensemble's invariants, live in trace_ensemble.cu for the
 // same reason.  They have one table placement (global memory): TABLE_IN_SMEM is ignored.
 template <class EQ, int BLOCK> const void* ens_trace_kernel();
@@ -832,7 +834,10 @@ cudaError_t ens_setup(LaunchConsts* out, const LaunchConsts& in, const Table1D* 
                       int variant, double* poly, cudaStream_t st);
 template <class EQ, int BLOCK, bool TABLE_IN_SMEM, bool PATHS, class ARGS>
 const void* trace_kernel_fn() {
-    if constexpr (IsMSrc<ARGS>::value) return msrc_trace_kernel<EQ, BLOCK, TABLE_IN_SMEM>();
+    if constexpr (IsMSrc<ARGS>::value) {
+        if constexpr (PATHS) return msrc_paths_trace_kernel<EQ, BLOCK, TABLE_IN_SMEM>();
+        else return msrc_trace_kernel<EQ, BLOCK, TABLE_IN_SMEM>();
+    }
     else if constexpr (IsEns<ARGS>::value) {
         static_assert(!PATHS, "the ensemble kernels have no raypath / caustic capture");
         return ens_trace_kernel<EQ, BLOCK>();

@@ -251,6 +251,20 @@ int geoac_trace_paths_compact(geoac_ctx* ctx, int64_t n_rays, const double* thet
                               int path_stride, int64_t path_cap, int64_t path_total_cap, double* path, int64_t* path_offset,
                               int64_t caustic_cap, int64_t caustic_total_cap, double* caustic, int64_t* caustic_offset);
 
+/* geoac_trace_paths_compact for rays from many sources in one call: ray r is launched at (theta[r], phi[r]) from source
+ * src_id[r].  src, src_id as geoac_trace_sources takes them; the records, the capture arguments, the layout of the rows and
+ * offsets and the GEOAC_ERR_TOO_LARGE behaviour as geoac_trace_paths_compact's.  The record, status, step count, raypath
+ * rows and caustic rows of ray r are bit for bit what geoac_trace_paths_compact returns for (theta[r], phi[r]) on this
+ * context with params.src set to src[src_id[r]], whatever the other rays of the batch, their sources and their order.
+ * Serves the raypath files of eigenrays found from many sources (<title>_Eigenray-N.dat, geoac_eigenray_search_sources) and
+ * WriteRays=True / WriteCaustics=True runs of -prop over many sources.  The context's parameters are not changed.
+ * Errors, returned before any device work: those of geoac_trace_sources (with n_rays > 0) and of geoac_trace_paths_compact
+ * (capture arguments); n_rays == 0 sets the first offset of each capture asked for and is GEOAC_OK. */
+int geoac_trace_sources_paths_compact(geoac_ctx* ctx, int n_src, const double* src, int64_t n_rays, const int32_t* src_id,
+                                      const double* theta, const double* phi, double* rec, int32_t* status, int32_t* n_steps,
+                                      int path_stride, int64_t path_cap, int64_t path_total_cap, double* path, int64_t* path_offset,
+                                      int64_t caustic_cap, int64_t caustic_total_cap, double* caustic, int64_t* caustic_offset);
+
 /* ---- several devices behind one call (SURVEY 8b / 8e; the data-parallel axis is the launch-angle loop, Code/GeoAc3D_main.cpp:226-227) ----
  * A front end creates one context per device (geoac_create_multi, or geoac_create in a loop), gives every context the same
  * atmosphere and parameters (the geoac_multi_set_* helpers do that from one host thread per context) and traces with
@@ -340,8 +354,8 @@ enum { GEOAC_EIG_NF = 18 };
  * inside the reference).  rows: cap_rows * GEOAC_EIG_NF doubles; *n_rows = rows produced (GEOAC_ERR_TOO_LARGE
  * if more than cap_rows).  stats (may be NULL): [0] trace batches, [1] rays traced, [2] eigenrays found.  The raypath file
  * of an eigenray (<title>_Eigenray-N.dat) is geoac_trace_paths at (theta, phi) with accum_per_segment = 1, stride 25.
- * While it runs the call sets bounces / calc_amp / accum_per_segment (Global: the source) on the context and restores the
- * caller's parameters before it returns, on the error paths too. */
+ * While it runs the call sets bounces / calc_amp / accum_per_segment on the context and restores the caller's parameters
+ * before it returns, on the error paths too. */
 int geoac_eigenray_search(geoac_ctx* ctx, const geoac_eig_opts* opts, int n_rcvr, const double* rcvr_xy,
                           int64_t cap_rows, double* rows, int64_t* n_rows, int64_t* stats);
 
@@ -354,6 +368,34 @@ int geoac_eigenray_search(geoac_ctx* ctx, const geoac_eig_opts* opts, int n_rcvr
  * ones -eig_search uses, and finds the same eigenray within `tolerance` rather than the same digits. */
 int geoac_eigenray_direct(geoac_ctx* ctx, const geoac_eig_opts* opts, int n, const double* rcvr_xy, const double* estimates,
                           double* rows, int64_t* stats);
+
+/* -eig_search from many sources in one call: search i runs from source src_id[i] (in [0, n_src)) to receiver
+ * rcvr_xy[2i..2i+1]; receivers may repeat across sources, a source may have any number of searches.
+ *   src  : n_src rows of 3 doubles -- Cartesian variants (x, y, z) [km] as params.src; Global variants (altitude [km],
+ *          lat [deg], lon [deg]) in degrees like the eigenray interface's receivers (the rays start from lat*Pi/180,
+ *          lon*Pi/180).  params.src and opts->src_lat_deg / src_lon_deg are not read.  Each source is clamped to the ground
+ *          as the one-source search clamps params.src.
+ *   rows : as geoac_eigenray_search's, column 0 the search index i; in the order (i, bounce count, theta_start ascending).
+ *   stats (may be NULL): [0] trace batches, [1] rays traced, [2] eigenrays found, for the whole call.
+ * Search i's rows, column 0 aside, are bit for bit those of geoac_eigenray_search with the same opts and the one receiver
+ * rcvr_xy[i] on this context with params.src = src[src_id[i]] (Global: params.src[0], opts->src_lat_deg, src_lon_deg from
+ * that row), whatever the other searches of the call and their order.  The rounds of all searches are shared: each round
+ * traces the rays every incomplete search needs in one geoac_trace_sources batch per calc_amp setting.  The raypath file of
+ * an eigenray is geoac_trace_sources_paths_compact at its angles from its source (accum_per_segment = 1, stride 25).  The
+ * context's parameters are restored before the call returns, on the error paths too.
+ * Errors, returned before any device work: GEOAC_ERR_BAD_ARG (NULL context, opts or n_rows, n_rcvr < 0; with n_rcvr > 0:
+ * a NULL src / src_id / rcvr_xy, n_src < 1, a non-finite source coordinate, a src_id outside [0, n_src) -- the message
+ * names the source or the first such search; rows NULL with cap_rows > 0; the 2D variant; opts refused as by
+ * geoac_eigenray_search), GEOAC_ERR_NO_ATMO.  n_rcvr == 0: GEOAC_OK, *n_rows = 0, rows untouched.  More rows than cap_rows:
+ * GEOAC_ERR_TOO_LARGE with *n_rows set (the first cap_rows rows are written). */
+int geoac_eigenray_search_sources(geoac_ctx* ctx, const geoac_eig_opts* opts, int n_src, const double* src,
+                                  int n_rcvr, const int32_t* src_id, const double* rcvr_xy,
+                                  int64_t cap_rows, double* rows, int64_t* n_rows, int64_t* stats);
+
+/* Where the time of the last eigenray search on ctx (any of the three calls above) went, in ms: ms3[0] host time replaying
+ * the searches against the ray cache, ms3[1] kernel time of its traces (geoac_last_trace_stats summed), ms3[2] the whole
+ * call.  NaN before the first search. */
+int geoac_last_eigenray_ms(const geoac_ctx* ctx, double* ms3);
 
 /* Variant the context was created for; c, u, v, rho at the source point (device-sampled), 4 doubles. */
 int geoac_get_variant(const geoac_ctx* ctx);
